@@ -4,6 +4,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...        # the UNMODIFIED reference losses/bl.py on the host cores (oracle/_ref)
+    python bench.py ... --dump-outputs DIR      # also save loss.npy / density_grad.npy of the last timed step
 
 One "step" = one pass of the hot path (BL forward + backward) over one batch of 16 synthetic
 QNRF-shaped images per GPU (2048x1536 px, stride-8 grid 192x256, 500..12000 heads, CSR-packed).
@@ -54,7 +55,23 @@ def parse():
     ap.add_argument("--no-aux", action="store_true", help="skip the splat / Gram lines")
     ap.add_argument("--no-eager", action="store_true", help="skip the PyTorch-eager-on-GPU reference leg")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling legs at N > 1")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and density gradient of the last timed step (rank 0) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
+
+
+def dump_outputs(out_dir, arrays):
+    """Save float32 / float64 arrays as ``out_dir/<name>.npy``; the inputs are seeded, so two builds can be compared."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def workload(rank):
@@ -634,13 +651,17 @@ def run_gpu(args, emit=print):
     for _ in range(args.steps):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        step_resident()
+        loss = step_resident()
         e1.record()
         events.append((e0, e1))
         flush.zero_()  # L2 flush between timed steps, outside the per-step events
+        # the loss's autograd node holds the step's workspace: kept alive, the next step would allocate a second one
+        loss = loss.detach() if args.dump_outputs else None
     barrier()
     wall = time.perf_counter() - t_wall0
     total_ms = sum(a.elapsed_time(c) for a, c in events)
+    if args.dump_outputs and rank == 0:   # the legs below overwrite the gradient
+        dump_outputs(args.dump_outputs, {"loss": loss, "density_grad": dens_d.grad})
 
     # informational: the same steps with the opt-in exact-zero culling (bit-identical results, not graded)
     loss_mod.exact_cull = True

@@ -129,7 +129,10 @@ def test_device_code_is_the_build_the_gpu_suite_ran_on():
 def test_no_entry_point_crashes_on_null_or_degenerate_arguments():
     """Error behaviour of the ABI: integer codes, never a crash.  Every exported function is called (i) with null
     pointers and zeros, (ii) with valid host pointers and sizes 0 / -1 and (iii) 1500 times with random small, boundary
-    and absurd (2^31 - 1) sizes, in ONE child process (a crash then names the call it died in).  No GPU needed: argument checks come first, and without a device the CUDA calls fail with a code.
+    and absurd (2^31 - 1) sizes, in ONE child process (a crash then names the call it died in).  The child sees no
+    device, even where there is one: every launcher first hands its stream to the CUDA runtime (the device guard in
+    csrc/common.cuh) and only then checks its arguments, and the host pointers the child passes also stand in for stream
+    handles.  A runtime without a device rejects such a call with a code; one with a device would dereference them.
     (Found dgvcc_isw_workspace_bytes(0, 0, 0), dgvcc_lw_loss_forward(hw = 0) and overflowing shapes dividing by zero in
     the split-K plans; the ISW-family launchers now check isw_shape_ok first.)"""
     import subprocess
@@ -185,7 +188,8 @@ for it in range(1500):
     getattr(lib, name)(*vals)
 print("survived", flush=True)
 ''' % ROOT
-    p = subprocess.run([sys.executable, "-c", child], capture_output=True, text=True, timeout=300)
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    p = subprocess.run([sys.executable, "-c", child], capture_output=True, text=True, timeout=300, env=env)
     last = (p.stdout.strip().splitlines() or ["<nothing>"])[-1]
     assert p.returncode == 0 and last == "survived", f"child rc={p.returncode}, last line: {last}\n{p.stderr[-600:]}"
 
