@@ -2088,12 +2088,12 @@ struct Plan {
     int warp_ctas() const { return ceil_div((int)grid.y * (g.tiles - g.task_first), WARPS_PER_CTA); }
 };
 
-int make_plan(const void* a, const void* b, const void* ws, size_t ws_bytes, int batch, int hp, int wp,
-              int64_t total_rows, int total_chunks, float stride, float sigma, Plan* p,
-              const dgvcc_bl_shard* shard = nullptr) {
-    if (!a || !b || !ws) return DGVCC_ERR_ARG;
+// What every plan starts from (world > 0: the symmetric layout of the sharded paths); the callers add checks and grid.
+int plan_common(const void* a, const void* ws, size_t ws_bytes, int batch, int hp, int wp, int64_t total_rows,
+                int total_chunks, float stride, float sigma, int world, Plan* p) {
+    if (!a || !ws) return DGVCC_ERR_ARG;
     if (!(stride > 0.f) || !(sigma > 0.f)) return DGVCC_ERR_ARG;
-    int rc = layout(total_rows, total_chunks, batch, hp, wp, &p->L, shard ? shard->world : 0);
+    int rc = layout(total_rows, total_chunks, batch, hp, wp, &p->L, world);
     if (rc) return rc;
     if (ws_bytes < (size_t)p->L.total) return DGVCC_ERR_WORKSPACE;
     p->v = Variant{p->L.rows_per_thread, p->L.cols_per_thread};
@@ -2101,6 +2101,15 @@ int make_plan(const void* a, const void* b, const void* ws, size_t ws_bytes, int
     p->k = make_scale(sigma);
     p->pow2 = is_pow2(p->k.s);
     p->sh = no_shard();
+    return DGVCC_OK;
+}
+
+int make_plan(const void* a, const void* b, const void* ws, size_t ws_bytes, int batch, int hp, int wp,
+              int64_t total_rows, int total_chunks, float stride, float sigma, Plan* p,
+              const dgvcc_bl_shard* shard = nullptr) {
+    if (!b) return DGVCC_ERR_ARG;
+    int rc = plan_common(a, ws, ws_bytes, batch, hp, wp, total_rows, total_chunks, stride, sigma, shard ? shard->world : 0, p);
+    if (rc) return rc;
     int slots = total_chunks;
     if (shard) {
         if (shard->world < 1 || shard->rank < 0 || shard->rank >= shard->world || shard->chunk_lo < 0 ||
@@ -2317,8 +2326,7 @@ int shard_wait(const ShardCtx& c, int ph) {
     return (int)cudaGetLastError();
 }
 
-// The density copy (owner -> sweeping ranks) is needed only by bl_counts, four kernels into the step: it runs on a
-// side stream of the library (one per device, created on first use) between two events, so it costs the step nothing.
+// The library's side stream and its two events, one set per device: created on first use, handed out once all three exist.
 struct SideStream {
     cudaStream_t stream = nullptr;
     cudaEvent_t fork = nullptr, join = nullptr;
@@ -2328,13 +2336,31 @@ SideStream* side_stream() {
     int d = 0;
     if (cudaGetDevice(&d) != cudaSuccess || d < 0 || d >= 64) return nullptr;
     SideStream& s = side[d];
-    if (!s.stream) {
-        if (cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking) != cudaSuccess) return nullptr;
-        if (cudaEventCreateWithFlags(&s.fork, cudaEventDisableTiming) != cudaSuccess ||
-            cudaEventCreateWithFlags(&s.join, cudaEventDisableTiming) != cudaSuccess)
-            return nullptr;
-    }
-    return &s;
+    if (!s.stream && cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking) != cudaSuccess) s.stream = nullptr;
+    if (s.stream && !s.fork && cudaEventCreateWithFlags(&s.fork, cudaEventDisableTiming) != cudaSuccess) s.fork = nullptr;
+    if (s.fork && !s.join && cudaEventCreateWithFlags(&s.join, cudaEventDisableTiming) != cudaSuccess) s.join = nullptr;
+    return s.join ? &s : nullptr;
+}
+
+// Phase DENS.  The density copy (owner -> sweeping ranks) is needed only by bl_counts, four kernels into the step: it runs
+// on the side stream between two events, so it costs the step nothing; *side = nullptr: there is none, it ran on c.st.
+int push_density(const ShardCtx& c, const float* density_local, SideStream** side) {
+    SideStream* s = *side = c.sh->push_first[DGVCC_BL_PH_DENS + 1] > c.sh->push_first[DGVCC_BL_PH_DENS] ? side_stream() : nullptr;
+    if (!s) return shard_push(c, DGVCC_BL_PH_DENS, density_local);
+    DGVCC_RETURN_IF_CUDA(cudaEventRecord(s->fork, c.st));
+    DGVCC_RETURN_IF_CUDA(cudaStreamWaitEvent(s->stream, s->fork, 0));
+    ShardCtx cs = c;
+    cs.st = s->stream;
+    if (int rc = shard_push(cs, DGVCC_BL_PH_DENS, density_local)) return rc;
+    DGVCC_RETURN_IF_CUDA(cudaEventRecord(s->join, s->stream));
+    return DGVCC_OK;
+}
+
+// Phase OUT, after the GRAD wait: the finished gradients of this rank's own images, gathered into the caller's tensor.
+int gather_grad(const ShardCtx& c, float* grad_local) {
+    if (int rc = shard_wait(c, DGVCC_BL_PH_GRAD)) return rc;
+    if (c.sh->push_first[DGVCC_BL_PH_OUT + 1] > c.sh->push_first[DGVCC_BL_PH_OUT] && !grad_local) return DGVCC_ERR_ARG;
+    return shard_push(c, DGVCC_BL_PH_OUT, c.ws, grad_local ? (void*)grad_local : c.ws, DGVCC_BL_PH_GRAD);
 }
 
 bool shard_args_ok(const dgvcc_bl_shard* sh, const dgvcc_bl_push* slices, const void* aux, void* const* peers) {
@@ -2408,18 +2434,9 @@ extern "C" int dgvcc_bl_shard_forward(const float* pts_xy, const float* targets,
     const int M = hp * wp;
     const dim3 pix_grid(ceil_div(M, 256), n_img > 0 ? n_img : 1);
     mark(events, 0, st);
-    // density of the images this rank owns -> every rank that sweeps them (needed from bl_counts on): on the side stream
-    SideStream* side = shard->push_first[DGVCC_BL_PH_DENS + 1] > shard->push_first[DGVCC_BL_PH_DENS] ? side_stream() : nullptr;
-    if (side) {
-        DGVCC_RETURN_IF_CUDA(cudaEventRecord(side->fork, st));
-        DGVCC_RETURN_IF_CUDA(cudaStreamWaitEvent(side->stream, side->fork, 0));
-        ShardCtx cs = c;
-        cs.st = side->stream;
-        if ((rc = shard_push(cs, DGVCC_BL_PH_DENS, density_local))) return rc;
-        DGVCC_RETURN_IF_CUDA(cudaEventRecord(side->join, side->stream));
-    } else if ((rc = shard_push(c, DGVCC_BL_PH_DENS, density_local))) {
-        return rc;
-    }
+    // density of the images this rank owns -> every rank that sweeps them (needed from bl_counts on)
+    SideStream* side;
+    if ((rc = push_density(c, density_local, &side))) return rc;
     mark(events, 1, st);
     // per-pixel minima of the images this rank touches, from ALL their points (replicated on every rank): no exchange
     (void)multi_chunk;
@@ -2520,10 +2537,7 @@ extern "C" int dgvcc_bl_shard_backward(const float* pts_xy, const int32_t* meta,
         c.make(DGVCC_BL_PH_GRAD, c.owner_mask(), p.L.gfinal, 0, DGVCC_BL_PH_GPART, -1), n_img, 0, M, 0);
     DGVCC_RETURN_IF_CUDA(cudaGetLastError());
     mark(events, 2, st);
-    if ((rc = shard_wait(c, DGVCC_BL_PH_GRAD))) return rc;
-    // the finished gradients of this rank's own images, gathered into the caller's tensor
-    if (shard->push_first[DGVCC_BL_PH_OUT + 1] > shard->push_first[DGVCC_BL_PH_OUT] && !grad_local) return DGVCC_ERR_ARG;
-    rc = shard_push(c, DGVCC_BL_PH_OUT, workspace, grad_local ? (void*)grad_local : workspace, DGVCC_BL_PH_GRAD);
+    rc = gather_grad(c, grad_local);
     mark(events, 3, st);
     if (rc == DGVCC_OK && deferred_loss_out) {  // the loss of a forward that ran with defer_loss
         if ((rc = shard_wait(c, DGVCC_BL_PH_LOSS))) return rc;
@@ -2538,31 +2552,27 @@ extern "C" int dgvcc_bl_shard_backward(const float* pts_xy, const int32_t* meta,
 // ------------------------------------------------------------------- row-band sharding: launch sequences
 namespace {
 
+// Rows of pixel tiles (R grid rows each) [lo, hi) of rank q's band: as equal as they come, as BandPlan cuts them.
+void band_rows(int hp, int R, int world, int q, int* lo, int* hi) {
+    const int n_tr = ceil_div(hp, R);
+    *lo = (int)((long long)n_tr * q / world);
+    *hi = (int)((long long)n_tr * (q + 1) / world);
+}
+
 // Plan of a rank that sweeps the grid rows [band_lo, band_hi) of every image over all chunks.
 int make_band_plan(const void* a, const void* ws, size_t ws_bytes, int batch, int hp, int wp, int64_t total_rows,
                    int total_chunks, float stride, float sigma, const dgvcc_bl_shard* sh, Plan* p) {
-    if (!a || !ws || !sh) return DGVCC_ERR_ARG;
-    if (!(stride > 0.f) || !(sigma > 0.f)) return DGVCC_ERR_ARG;
-    if (sh->world < 1 || sh->world > 32 || sh->rank < 0 || sh->rank >= sh->world) return DGVCC_ERR_ARG;
-    int rc = layout(total_rows, total_chunks, batch, hp, wp, &p->L, sh->world);
-    if (rc) return rc;
-    if (ws_bytes < (size_t)p->L.total) return DGVCC_ERR_WORKSPACE;
-    p->v = Variant{p->L.rows_per_thread, p->L.cols_per_thread};
+    if (!sh || sh->world < 1 || sh->world > 32 || sh->rank < 0 || sh->rank >= sh->world) return DGVCC_ERR_ARG;
+    if (int rc = plan_common(a, ws, ws_bytes, batch, hp, wp, total_rows, total_chunks, stride, sigma, sh->world, p)) return rc;
     const int R = p->v.rows;
     if (sh->band_lo < 0 || sh->band_hi < sh->band_lo || sh->band_hi > hp || sh->band_lo % R != 0 ||
         (sh->band_hi % R != 0 && sh->band_hi != hp))
         return DGVCC_ERR_ARG;   // bands are whole rows of pixel tiles
-    {   // the bands follow from (hp, R, world) alone -- every rank must be able to derive every other rank's
-        const int n_tr = ceil_div(hp, R);
-        const int lo = (int)((long long)n_tr * sh->rank / sh->world), hi = (int)((long long)n_tr * (sh->rank + 1) / sh->world);
-        if (sh->band_lo != (lo * R < hp ? lo * R : hp) || sh->band_hi != (hi * R < hp ? hi * R : hp)) return DGVCC_ERR_ARG;
-    }
-    p->g = make_geom(hp, wp, p->v, stride);
+    int lo, hi;
+    band_rows(hp, R, sh->world, sh->rank, &lo, &hi);   // from (hp, R, world) alone: every rank can derive every other rank's
+    if (sh->band_lo != (lo * R < hp ? lo * R : hp) || sh->band_hi != (hi * R < hp ? hi * R : hp)) return DGVCC_ERR_ARG;
     p->g.task_first = (sh->band_lo / R) * p->g.col_blocks;
     p->g.tiles = ceil_div(sh->band_hi, R) * p->g.col_blocks;
-    p->k = make_scale(sigma);
-    p->pow2 = is_pow2(p->k.s);
-    p->sh = no_shard();
     p->grid = dim3(ceil_div(p->g.tiles - p->g.task_first, WARPS_PER_CTA), total_chunks);
     return DGVCC_OK;
 }
@@ -2587,15 +2597,8 @@ extern "C" int dgvcc_bl_band_forward(const float* pts_xy, const float* targets, 
     const bool sweeps = p.grid.x > 0 && p.grid.y > 0;
     mark(events, 0, st);
     // density rows of the images this rank owns -> the ranks whose bands they fall into (needed from bl_counts on)
-    SideStream* side = shard->push_first[DGVCC_BL_PH_DENS + 1] > shard->push_first[DGVCC_BL_PH_DENS] ? side_stream() : nullptr;
-    if (side) {
-        DGVCC_RETURN_IF_CUDA(cudaEventRecord(side->fork, st));
-        DGVCC_RETURN_IF_CUDA(cudaStreamWaitEvent(side->stream, side->fork, 0));
-        ShardCtx cs = c;
-        cs.st = side->stream;
-        if ((rc = shard_push(cs, DGVCC_BL_PH_DENS, density_local))) return rc;
-        DGVCC_RETURN_IF_CUDA(cudaEventRecord(side->join, side->stream));
-    }
+    SideStream* side;
+    if ((rc = push_density(c, density_local, &side))) return rc;
     mark(events, 1, st);
     float* min_img = at<float>(workspace, p.L.gpart);  // free until the backward pass
     if (sweeps) {
@@ -2628,12 +2631,10 @@ extern "C" int dgvcc_bl_band_forward(const float* pts_xy, const float* targets, 
     mark(events, 4, st);
     if ((rc = shard_wait(c, DGVCC_BL_PH_CNT))) return rc;
     // every rank adds all partial rows in (rank, CTA) order -- the order of the pixel tiles, as on one GPU
-    BandRows br;
-    const int R = p.v.rows;
-    for (int q = 0; q < 32; ++q) br.n[q] = 0;
+    BandRows br{};
     for (int q = 0; q < shard->world; ++q) {  // the bands of all ranks follow from (hp, R, world) alone
-        const int n_tr = ceil_div(hp, R);
-        const int lo = (int)((long long)n_tr * q / shard->world), hi = (int)((long long)n_tr * (q + 1) / shard->world);
+        int lo, hi;
+        band_rows(hp, p.v.rows, shard->world, q, &lo, &hi);
         br.n[q] = ceil_div((hi - lo) * p.g.col_blocks, WARPS_PER_CTA);
     }
     const unsigned row_blocks = (unsigned)((total_rows + 255) / 256);
@@ -2679,9 +2680,7 @@ extern "C" int dgvcc_bl_band_backward(const float* pts_xy, const int32_t* meta, 
     }
     DGVCC_RETURN_IF_CUDA(cudaGetLastError());
     mark(events, 1, st);
-    if ((rc = shard_wait(c, DGVCC_BL_PH_GRAD))) return rc;
-    if (shard->push_first[DGVCC_BL_PH_OUT + 1] > shard->push_first[DGVCC_BL_PH_OUT] && !grad_local) return DGVCC_ERR_ARG;
-    rc = shard_push(c, DGVCC_BL_PH_OUT, workspace, grad_local ? (void*)grad_local : workspace, DGVCC_BL_PH_GRAD);
+    rc = gather_grad(c, grad_local);
     mark(events, 2, st);
     return rc;
 }

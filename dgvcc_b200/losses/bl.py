@@ -143,6 +143,24 @@ def _align16(n):
     return (n + 15) // 16 * 16
 
 
+def _pack_into(view, meta, points, targets, total_points):
+    """The host buffer of a packed batch, ``[int32 table | align16 | points | align16 | targets]`` (what
+    dgvcc_bl_pack_host writes).  Returns (o_pts, o_tgt, total bytes) for ``meta`` and ``total_points``; with a uint8
+    array ``view`` of at least that size it also writes table, points and, unless ``targets`` is None, targets."""
+    n = max(total_points, 1)
+    o_pts = _align16(meta.nbytes)
+    o_tgt = o_pts + _align16(8 * n)
+    if view is not None:
+        view[:meta.nbytes].view(np.int32)[:] = meta
+        if total_points:
+            np.concatenate([_host_f32(p.cpu()).reshape(-1, 2) for p in points if p.numel()], axis=0,
+                           out=view[o_pts:o_pts + 8 * total_points].view(np.float32).reshape(-1, 2))
+            if targets is not None:
+                np.concatenate([_host_f32(t.cpu()).reshape(-1) for t in targets if t.numel()],
+                               out=view[o_tgt:o_tgt + 4 * total_points].view(np.float32))
+    return o_pts, o_tgt, o_tgt + _align16(4 * n)
+
+
 class PackedBatch:
     """A ragged batch already packed on the host (table + points + targets in ONE buffer), built by
     ``pack_batch`` -- e.g. inside a DataLoader ``collate_fn`` in place of bay_dataset.py:13-19's tuples -- so that
@@ -174,18 +192,9 @@ def pack_batch(points, targets, use_background=True, chunk=None):
             raise ValueError(f"target length {t.shape[0]} does not match its {n} points")
     meta, total_chunks, multi_chunk = build_meta(counts, rows, chunk or chunk_points())
     total_points = int(counts.sum())
-    n_pts = max(total_points, 1)
-    o_pts = _align16(meta.nbytes)
-    o_tgt = o_pts + _align16(8 * n_pts)
-    total = o_tgt + _align16(4 * n_pts)
+    o_pts, o_tgt, total = _pack_into(None, meta, points, targets, total_points)
     buf = torch.zeros((total,), dtype=torch.uint8)
-    view = buf.numpy()
-    view[:meta.nbytes].view(np.int32)[:] = meta
-    if total_points:
-        np.concatenate([_host_f32(p) for p in points if p.shape[0]], axis=0,
-                       out=view[o_pts:o_pts + 8 * total_points].view(np.float32).reshape(-1, 2))
-        np.concatenate([_host_f32(t) for t in targets if t.shape[0]],
-                       out=view[o_tgt:o_tgt + 4 * total_points].view(np.float32))
+    _pack_into(buf.numpy(), meta, points, targets, total_points)
     return PackedBatch(buf, meta.nbytes, o_pts, o_tgt, total, counts, rows, total_chunks, multi_chunk, bool(use_background))
 
 
@@ -246,19 +255,10 @@ class _Packed:
         self.row_off = np.concatenate(([0], np.cumsum(rows))).astype(np.int32)
         meta, self.total_chunks, self.multi_chunk = build_meta(counts, rows, chunk_points())
         if self.on_host:
-            o_pts = _align16(meta.nbytes)
-            o_tgt = o_pts + _align16(8 * n_pts)
-            total = o_tgt + _align16(4 * n_pts)
+            o_pts, o_tgt, total = _pack_into(None, meta, points, targets, self.total_points)
             ring = _staging.setdefault(device, _Staging())
             slot, host = ring.take(total)
-            view = host.numpy()
-            view[:meta.nbytes].view(np.int32)[:] = meta
-            if self.total_points:
-                hp = view[o_pts:o_pts + 8 * self.total_points].view(np.float32).reshape(-1, 2)
-                np.concatenate([_host_f32(p) for p in points if p.shape[0]], axis=0, out=hp)
-                if targets is not None:
-                    ht = view[o_tgt:o_tgt + 4 * self.total_points].view(np.float32)
-                    np.concatenate([_host_f32(t) for t in targets if t.shape[0]], out=ht)
+            _pack_into(host.numpy(), meta, points, targets, self.total_points)
             dev_buf = host[:total].to(device, non_blocking=True)
             ring.sent(slot, device)
             self.meta = dev_buf[:meta.nbytes].view(torch.int32)

@@ -23,12 +23,10 @@ Interface and communicators as in ``bl_sharded`` (``LocalComm`` runs the ranks i
 import ctypes
 
 import numpy as np
-import torch
-from torch.nn import Module
 
 from .. import _native
 from . import bl as _bl
-from .bl_sharded import SLICE_BYTES, IpcComm, LocalComm, _PackedAll, plan_err_offset  # noqa: F401  (re-exported)
+from .bl_sharded import IpcComm, LocalComm, _cached_plan, _PeerBL, _PeerPlan  # noqa: F401  (IpcComm, LocalComm: re-exported)
 
 FORCE_CHUNK = None   # experiments: points per chunk of the band plan, whatever the world size
 TAIL_SPLIT = 0       # experiments: cut the last quarter of every image's chunks into this many pieces (build_meta)
@@ -49,57 +47,33 @@ def band_chunk_points(total_points, world, hp, wp):
     return int(min(_bl.chunk_points(), max(256, -(-want // 32) * 32)))
 
 
-class BandPlan:
+class BandPlan(_PeerPlan):
     """What the ranks agree on, from the head counts and the grid shape alone (host, deterministic)."""
 
     def __init__(self, counts, use_bg, world, owners, hp, wp, chunk):
-        counts = np.asarray(counts, dtype=np.int64)
-        b = len(counts)
-        if b == 0:
-            raise ValueError("empty batch")
-        self.batch, self.world, self.use_bg, self.hp, self.wp, self.chunk = b, int(world), bool(use_bg), int(hp), int(wp), int(chunk)
-        owners = np.asarray(owners if owners is not None else np.arange(b) * world // b, dtype=np.int64)
-        if owners.shape != (b,) or owners.min() < 0 or owners.max() >= world:
-            raise ValueError("owners must give one rank in [0, world) per image")
-        self.owners, self.counts = owners, counts
-        self.rows = np.where(counts == 0, 1, counts + (1 if use_bg else 0))
-        self.total_points, self.total_rows = int(counts.sum()), int(self.rows.sum())
-        self.meta, self.total_chunks, self.multi_chunk = _bl.build_meta(counts, self.rows, self.chunk, TAIL_SPLIT)
-        self.owned = [np.nonzero(owners == r)[0] for r in range(world)]
-        self.layout = _native.BLLayout()
-        _native.check(_native.lib().dgvcc_bl_shard_workspace_layout(self.total_rows, self.total_chunks, b, hp, wp, world,
-                                                                    self.layout), "dgvcc_bl_shard_workspace_layout")
+        super().__init__(counts, use_bg, world, owners, hp, wp)
+        self.chunk = int(chunk)
+        self.meta, self.total_chunks, self.multi_chunk = _bl.build_meta(self.counts, self.rows, self.chunk, TAIL_SPLIT)
+        self._query_layout()
         # bands: whole rows of pixel tiles (rows_per_thread grid rows each), as equal as they come
         tile_rows = self.layout.rows_per_thread
         n_tr = -(-hp // tile_rows)
         cut = (np.arange(world + 1, dtype=np.int64) * n_tr) // world
         self.band_lo = np.minimum(cut[:-1] * tile_rows, hp)
         self.band_hi = np.minimum(cut[1:] * tile_rows, hp)
-        self._build()
+        self._build_tables()
+        for r, sh in enumerate(self.shards):
+            sh.band_lo, sh.band_hi = int(self.band_lo[r]), int(self.band_hi[r])
 
     def meta_for(self, rank):
         """The int32 table of include/dgvcc_b200.h: the same on every rank, every chunk scheduled."""
         return self.meta
 
-    def _build(self):
+    def _exchange(self, flag, add):
         w, L, b = self.world, self.layout, self.batch
         m4, row4 = 4 * self.hp * self.wp, 4 * self.wp
         P = _native
-        per = [[[] for _ in range(P.BL_PHASES)] for _ in range(w)]
-        wait = np.zeros((w, P.BL_PHASES), dtype=np.uint32)
-        signal = np.zeros((w, P.BL_PHASES), dtype=np.uint32)
         owner_mask = np.zeros((w, b), dtype=np.uint32)
-
-        def flag(phase, src, dst):
-            if dst != src:
-                wait[dst, phase] |= np.uint32(1 << src)
-                signal[src, phase] |= np.uint32(1 << dst)
-
-        def add(phase, src, src_off, dst, dst_off, nbytes):
-            step = SLICE_BYTES if (src_off | dst_off | nbytes) % 16 == 0 else 1 << 30
-            for o in range(0, nbytes, step):
-                per[src][phase].append((src_off + o, dst_off + o, min(step, nbytes - o), dst))
-
         for i in range(b):
             own = int(self.owners[i])
             k_local = int(np.searchsorted(self.owned[own], i))
@@ -115,36 +89,7 @@ class BandPlan:
         for r in range(w):        # count shares: everybody -> everybody
             for q in range(w):
                 flag(P.BL_PH_CNT, r, q)
-        self.slices, self.shards, self.aux, self._dev = [], [], [], {}
-        for r in range(w):
-            rows, first = [], [0]
-            for ph in range(P.BL_PHASES):
-                rows += per[r][ph]
-                first.append(len(rows))
-            arr = np.zeros((max(len(rows), 1), 3), dtype=np.int64)   # (src_off, dst_off, bytes | dst_rank << 32)
-            if rows:
-                t = np.asarray(rows, dtype=np.int64)
-                arr[:len(rows), 0], arr[:len(rows), 1] = t[:, 0], t[:, 1]
-                arr[:len(rows), 2] = t[:, 2] | (t[:, 3] << 32)
-            self.slices.append(arr)
-            self.aux.append(owner_mask[r].copy())
-            sh = _native.BLShard()
-            sh.rank, sh.world = r, w
-            sh.band_lo, sh.band_hi = int(self.band_lo[r]), int(self.band_hi[r])
-            for ph in range(P.BL_PHASES + 1):
-                sh.push_first[ph] = first[ph]
-            for ph in range(P.BL_PHASES):
-                sh.wait_mask[ph], sh.signal_mask[ph] = int(wait[r, ph]), int(signal[r, ph])
-            self.shards.append(sh)
-
-    def tables_on(self, rank, device):
-        """(slices, owner_mask) of ``rank`` as device tensors (uploaded once per plan)."""
-        key = (rank, str(device))
-        t = self._dev.get(key)
-        if t is None:
-            t = self._dev[key] = (torch.from_numpy(self.slices[rank]).to(device),
-                                  torch.from_numpy(self.aux[rank].view(np.int32)).to(device))
-        return t
+        return [owner_mask[r].copy() for r in range(w)]
 
 
 _plan_cache = {}
@@ -154,65 +99,10 @@ def plan_bands(counts, use_bg, world, owners, hp, wp, chunk=None):
     """Cached ``BandPlan`` (forward and backward of one step share it; a benchmark hits it every step)."""
     key = (tuple(int(c) for c in counts), bool(use_bg), int(world), None if owners is None else tuple(int(o) for o in owners),
            int(hp), int(wp), int(chunk or band_chunk_points(sum(int(c) for c in counts), world, hp, wp)), int(TAIL_SPLIT))
-    plan = _plan_cache.get(key)
-    if plan is None:
-        if len(_plan_cache) > 64:
-            _plan_cache.clear()
-        plan = _plan_cache[key] = BandPlan(counts, use_bg, world, owners, hp, wp, key[-2])
-    return plan
+    return _cached_plan(_plan_cache, key, lambda: BandPlan(counts, use_bg, world, owners, hp, wp, key[-2]))
 
 
-class _BandedFn(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, density_local, mod, plan, packed, st, inv_batch):
-        comm, pp = mod.comm, mod.post_prob
-        dev, r = comm.device, comm.rank
-        _native.require_cuda(st, "BandShardedBL.forward")
-        hp, wp, L = plan.hp, plan.wp, plan.layout
-        n_own = len(plan.owned[r])
-        dens = density_local.detach().reshape(n_own, hp, wp).to(torch.float32).contiguous() if n_own else None
-        if L.total > comm.nbytes:
-            raise RuntimeError(f"sharded workspace of {comm.nbytes} bytes is too small for this batch ({L.total} bytes); "
-                               "create the communicator with a larger nbytes")
-        comm.epoch += 1
-        shard = plan.shards[r]
-        shard.epoch = comm.epoch
-        shard.fuse_waits = int(comm.fuse_waits)
-        slices, owner_mask = plan.tables_on(r, dev)
-        loss = torch.empty((1,), dtype=torch.float32, device=dev)
-        rc = _native.lib().dgvcc_bl_band_forward(
-            _native.ptr(packed.pts), _native.ptr(packed.targets), _native.ptr(packed.meta), _native.ptr(st), _native.ptr(dens),
-            plan.batch, hp, wp, plan.total_rows, plan.total_chunks, float(pp.stride), float(pp.sigma), float(pp.bg_ratio),
-            int(pp.use_bg), int(mod.exact_cull), inv_batch, ctypes.byref(shard), _native.ptr(slices), _native.ptr(owner_mask),
-            _native.ptr(comm.peer_table), _native.ptr(comm.workspace), comm.nbytes, _native.ptr(loss), _native.stream_ptr(dev),
-            mod._event_handles("fwd", 7))
-        _native.check(rc, "dgvcc_bl_band_forward")
-        ctx.saved = (mod, plan, packed, (slices, owner_mask), inv_batch, comm.epoch, density_local.shape, density_local.dtype, n_own)
-        return loss.reshape(())
-
-    @staticmethod
-    def backward(ctx, grad_loss):
-        mod, plan, packed, (slices, owner_mask), inv_batch, epoch, shape, dtype, n_own = ctx.saved
-        comm, pp = mod.comm, mod.post_prob
-        dev, r = comm.device, comm.rank
-        if epoch != comm.epoch:
-            raise RuntimeError("BandShardedBL: backward of a step whose shared workspace was already re-used by a later "
-                               "forward (one forward/backward pair at a time per communicator)")
-        shard = plan.shards[r]
-        shard.epoch = epoch
-        shard.fuse_waits = int(comm.fuse_waits)
-        g = grad_loss.detach().to(device=dev, dtype=torch.float32).reshape(1).contiguous()
-        grad = torch.empty((max(n_own, 1), plan.hp, plan.wp), dtype=torch.float32, device=dev)
-        rc = _native.lib().dgvcc_bl_band_backward(
-            _native.ptr(packed.pts), _native.ptr(packed.meta), plan.batch, plan.hp, plan.wp, plan.total_rows,
-            plan.total_chunks, float(pp.stride), float(pp.sigma), int(pp.use_bg), int(mod.exact_cull), inv_batch,
-            _native.ptr(g), ctypes.byref(shard), _native.ptr(slices), _native.ptr(owner_mask), _native.ptr(comm.peer_table),
-            _native.ptr(comm.workspace), comm.nbytes, _native.ptr(grad), _native.stream_ptr(dev), mod._event_handles("bwd", 3))
-        _native.check(rc, "dgvcc_bl_band_backward")
-        return (grad[:n_own].reshape(shape).to(dtype),) + (None,) * 5
-
-
-class BandShardedBL(Module):
+class BandShardedBL(_PeerBL):
     """``BL`` for one batch spread over ``comm.world`` GPUs by row bands of the density grid (module docstring)."""
 
     FWD_PHASES = ["issue DENS copy (side stream)", "grid build + minima", "z (+ finish)", "[wait DENS] counts (+CNT out)",
@@ -220,59 +110,30 @@ class BandShardedBL(Module):
     BWD_PHASES = ["grad (+ finish, GRAD out)", "[wait GRAD] gather"]
 
     def __init__(self, sigma, c_size, stride, background_ratio, use_background, device, comm):
-        super().__init__()
-        self.post_prob = _bl.Post_Prob(sigma, c_size, stride, background_ratio, use_background, device)
-        self.bay_loss = _bl.Bay_Loss(use_background, device)
-        self.comm = comm
-        self.exact_cull = True
+        super().__init__(sigma, c_size, stride, background_ratio, use_background, device, comm)
         self.chunk = None    # points per chunk (None: band_chunk_points)
-        self._last = None    # (key, packed): a benchmark / test that feeds the same lists again skips the re-pack
 
-    def forward(self, points, st_sizes, target_list, pre_density_local, owners=None):
+    def _plan(self, counts, owners, hp, wp):
+        return plan_bands(counts, self.post_prob.use_bg, self.comm.world, owners, hp, wp, self.chunk)
+
+    def _forward(self, plan, packed, st, dens, inv_batch, shard, tables, loss, backward_follows):
+        """dgvcc_bl_band_forward: the loss is complete when it returns (every rank finds it for itself)."""
         comm, pp = self.comm, self.post_prob
-        dev = comm.device
-        points = _bl._as_point_list(points)
-        counts = [int(p.shape[0]) for p in points]
-        hp, wp = int(pre_density_local.shape[-2]), int(pre_density_local.shape[-1])
-        plan = plan_bands(counts, pp.use_bg, comm.world, owners, hp, wp, self.chunk)
-        if pre_density_local.shape[0] != len(plan.owned[comm.rank]):
-            raise ValueError(f"rank {comm.rank} owns {len(plan.owned[comm.rank])} images of this batch but was given "
-                             f"{pre_density_local.shape[0]} density maps")
-        key = (id(plan), tuple(id(p) for p in points), tuple(id(t) for t in target_list))
-        if self._last is not None and self._last[0] == key:
-            packed = self._last[1]
-        else:
-            packed = _PackedAll(points, target_list, plan, comm.rank, dev)
-            self._last = (key, packed, points, target_list)   # the lists are kept alive so that the ids stay meaningful
-        st = st_sizes.to(device=dev, dtype=torch.float32).contiguous()
-        return _BandedFn.apply(pre_density_local, self, plan, packed, st, 1.0 / plan.batch)
+        rc = _native.lib().dgvcc_bl_band_forward(
+            _native.ptr(packed.pts), _native.ptr(packed.targets), _native.ptr(packed.meta), _native.ptr(st), _native.ptr(dens),
+            plan.batch, plan.hp, plan.wp, plan.total_rows, plan.total_chunks, float(pp.stride), float(pp.sigma),
+            float(pp.bg_ratio), int(pp.use_bg), int(self.exact_cull), inv_batch, ctypes.byref(shard), _native.ptr(tables[0]),
+            _native.ptr(tables[1]), _native.ptr(comm.peer_table), _native.ptr(comm.workspace), comm.nbytes, _native.ptr(loss),
+            _native.stream_ptr(comm.device), self._event_handles("fwd"))
+        _native.check(rc, "dgvcc_bl_band_forward")
+        return None
 
-    def _event_handles(self, which, n):
-        """None, or ctypes array of cudaEvent_t for the per-phase timing (``profile = True``)."""
-        if not getattr(self, "profile", False):
-            return None
-        evs = [torch.cuda.Event(enable_timing=True) for _ in range(n)]
-        for e in evs:
-            e.record()  # materialises the handle
-        self._events = getattr(self, "_events", {})
-        self._events[which] = evs
-        return (ctypes.c_void_p * n)(*[e.cuda_event for e in evs])
-
-    def phase_ms(self):
-        """{phase: ms} of the last profiled step (synchronises)."""
-        torch.cuda.synchronize(self.comm.device)
-        out = {}
-        for which, names in (("fwd", self.FWD_PHASES), ("bwd", self.BWD_PHASES)):
-            evs = self._events[which]
-            for k, name in enumerate(names):
-                out[f"{which}: {name}"] = evs[k].elapsed_time(evs[k + 1])
-        return out
-
-    def check(self):
-        """Synchronise and raise if a wait of the exchange protocol timed out (a peer died or fell out of step)."""
-        torch.cuda.synchronize(self.comm.device)
-        off = plan_err_offset(self.comm.world)
-        err = int(self.comm.workspace[off:off + 4].view(torch.int32).item())
-        if err:
-            ph, src = (err - 1) % 16, (err - 1) // 16
-            raise RuntimeError(f"BandShardedBL rank {self.comm.rank}: no flag of phase {ph} from rank {src} within 2 s")
+    def _backward(self, plan, packed, inv_batch, g, shard, tables, grad, deferred):
+        comm, pp = self.comm, self.post_prob
+        rc = _native.lib().dgvcc_bl_band_backward(
+            _native.ptr(packed.pts), _native.ptr(packed.meta), plan.batch, plan.hp, plan.wp, plan.total_rows,
+            plan.total_chunks, float(pp.stride), float(pp.sigma), int(pp.use_bg), int(self.exact_cull), inv_batch,
+            _native.ptr(g), ctypes.byref(shard), _native.ptr(tables[0]), _native.ptr(tables[1]), _native.ptr(comm.peer_table),
+            _native.ptr(comm.workspace), comm.nbytes, _native.ptr(grad), _native.stream_ptr(comm.device),
+            self._event_handles("bwd"))
+        _native.check(rc, "dgvcc_bl_band_backward")

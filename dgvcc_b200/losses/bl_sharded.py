@@ -20,9 +20,11 @@ contiguous blocks, what a data-parallel model produces), in image order.
 ``plan_shards`` (host only, numpy) is the whole bookkeeping: chunk table, per-rank ranges, push slices, wait /
 signal masks.  ``LocalComm`` runs several "ranks" inside one process on one GPU (one stream each) -- the parity
 tests use it, the kernels and the protocol are the same as with one process per GPU.
+
+The row-band split (``bl_banded``) shares this module's communicators and host layer: the plan base ``_PeerPlan``
+(owners, workspace layout, exchange tables), the module base ``_PeerBL`` and the autograd function ``_PeerFn``.
 """
 import ctypes
-from math import ceil  # noqa: F401  (kept for parity with losses/bl.py helpers)
 
 import numpy as np
 import torch
@@ -34,10 +36,12 @@ from . import bl as _bl
 SLICE_BYTES = 32 * 1024   # one CTA of the push kernel moves at most this much
 
 
-class ShardPlan:
-    """Everything the ranks need to agree on, computed from the head counts alone (host, deterministic)."""
+class _PeerPlan:
+    """What the ranks of either peer split agree on, computed from the head counts alone (host, deterministic): the
+    owners of the images' density, the posterior rows, the symmetric workspace layout and the exchange tables.  A
+    split's constructor adds its partition, then calls ``_query_layout`` and ``_build_tables``."""
 
-    def __init__(self, counts, use_bg, world, owners, hp, wp, chunk):
+    def __init__(self, counts, use_bg, world, owners, hp, wp):
         counts = np.asarray(counts, dtype=np.int64)
         b = len(counts)
         if b == 0:
@@ -47,13 +51,87 @@ class ShardPlan:
         if owners.shape != (b,) or owners.min() < 0 or owners.max() >= world:
             raise ValueError("owners must give one rank in [0, world) per image")
         self.owners, self.counts = owners, counts
-        rows = np.where(counts == 0, 1, counts + (1 if use_bg else 0))
-        self.rows = rows
+        self.rows = np.where(counts == 0, 1, counts + (1 if use_bg else 0))
+        self.total_points, self.total_rows = int(counts.sum()), int(self.rows.sum())
+        self.owned = [np.nonzero(owners == r)[0] for r in range(world)]          # images whose density lives on rank r
+
+    def _query_layout(self):
+        self.layout = _native.BLLayout()
+        _native.check(_native.lib().dgvcc_bl_shard_workspace_layout(self.total_rows, self.total_chunks, self.batch, self.hp,
+                                                                    self.wp, self.world, self.layout),
+                      "dgvcc_bl_shard_workspace_layout")
+
+    def _build_tables(self):
+        """Who sends what to whom.  DENS and OUT are copy launches described by slices; the other phases are fused into
+        the kernels, which only need destination masks (``aux``) -- and every phase needs its wait / signal masks.  The
+        split's ``_exchange(flag, add)`` names the transfers and returns the ``aux`` array of every rank; the split
+        fills its own ``BLShard`` fields afterwards."""
+        w, n_ph = self.world, _native.BL_PHASES
+        per = [[[] for _ in range(n_ph)] for _ in range(w)]        # per[src][phase] = [(src_off, dst_off, bytes, dst)]
+        wait = np.zeros((w, n_ph), dtype=np.uint32)
+        signal = np.zeros((w, n_ph), dtype=np.uint32)
+
+        def flag(phase, src, dst):
+            if dst != src:
+                wait[dst, phase] |= np.uint32(1 << src)
+                signal[src, phase] |= np.uint32(1 << dst)
+
+        def add(phase, src, src_off, dst, dst_off, nbytes):
+            step = SLICE_BYTES if (src_off | dst_off | nbytes) % 16 == 0 else 1 << 30
+            for o in range(0, nbytes, step):
+                per[src][phase].append((src_off + o, dst_off + o, min(step, nbytes - o), dst))
+
+        self.aux = self._exchange(flag, add)
+        self.slices, self.shards, self._dev = [], [], {}
+        for r in range(w):
+            rows, first = [], [0]
+            for ph in range(n_ph):
+                rows += per[r][ph]
+                first.append(len(rows))
+            arr = np.zeros((max(len(rows), 1), 3), dtype=np.int64)   # (src_off, dst_off, bytes | dst_rank << 32): 24-byte records
+            if rows:
+                t = np.asarray(rows, dtype=np.int64)
+                arr[:len(rows), 0], arr[:len(rows), 1] = t[:, 0], t[:, 1]
+                arr[:len(rows), 2] = t[:, 2] | (t[:, 3] << 32)
+            self.slices.append(arr)
+            sh = _native.BLShard()
+            sh.rank, sh.world = r, w
+            for ph in range(n_ph + 1):
+                sh.push_first[ph] = first[ph]
+            for ph in range(n_ph):
+                sh.wait_mask[ph], sh.signal_mask[ph] = int(wait[r, ph]), int(signal[r, ph])
+            self.shards.append(sh)
+
+    def tables_on(self, rank, device):
+        """(slices, aux) of ``rank`` as device tensors (uploaded once per plan)."""
+        key = (rank, str(device))
+        t = self._dev.get(key)
+        if t is None:
+            t = self._dev[key] = (torch.from_numpy(self.slices[rank]).to(device),
+                                  torch.from_numpy(self.aux[rank].view(np.int32)).to(device))
+        return t
+
+
+def _cached_plan(cache, key, make):
+    """``cache[key]``, made by ``make()`` when missing (a cache of more than 64 plans is emptied first)."""
+    plan = cache.get(key)
+    if plan is None:
+        if len(cache) > 64:
+            cache.clear()
+        plan = cache[key] = make()
+    return plan
+
+
+class ShardPlan(_PeerPlan):
+    """The plan of the point-chunk split: chunk table, per-rank point spans, and the exchange of every phase."""
+
+    def __init__(self, counts, use_bg, world, owners, hp, wp, chunk):
+        super().__init__(counts, use_bg, world, owners, hp, wp)
+        b, counts = self.batch, self.counts
         pt_off = np.concatenate(([0], np.cumsum(counts)))
-        row_off = np.concatenate(([0], np.cumsum(rows)))
+        row_off = np.concatenate(([0], np.cumsum(self.rows)))
         self.pt_off, self.row_off = pt_off, row_off
-        total = int(pt_off[-1])
-        self.total_points, self.total_rows = total, int(row_off[-1])
+        total = self.total_points
         bounds = (np.arange(world + 1, dtype=np.int64) * total) // world   # rank r sweeps points [bounds[r], bounds[r+1])
         self.bounds = bounds
         rank_of = lambda pos: min(int(np.searchsorted(bounds[1:], pos, side="right")), world - 1)  # noqa: E731
@@ -84,11 +162,13 @@ class ShardPlan:
         self.img_lo = np.array([self.c_img[self.chunk_lo[r]] if self.chunk_hi[r] > self.chunk_lo[r] else 0 for r in range(world)])
         self.img_hi = np.array([self.c_img[self.chunk_hi[r] - 1] + 1 if self.chunk_hi[r] > self.chunk_lo[r] else 0
                                 for r in range(world)])
-        self.owned = [np.nonzero(owners == r)[0] for r in range(world)]          # images whose density lives on rank r
-        self.layout = _native.BLLayout()
-        _native.check(_native.lib().dgvcc_bl_shard_workspace_layout(self.total_rows, self.total_chunks, b, hp, wp, world,
-                                                                    self.layout), "dgvcc_bl_shard_workspace_layout")
-        self._build_slices()
+        self._query_layout()
+        self._build_tables()
+        for r, sh in enumerate(self.shards):
+            sh.chunk_lo, sh.chunk_hi = int(self.chunk_lo[r]), int(self.chunk_hi[r])
+            sh.pt_lo, sh.pt_hi = int(self.bounds[r]), int(self.bounds[r + 1])
+            sh.img_lo, sh.img_hi = int(self.img_lo[r]), int(self.img_hi[r])
+            sh.row_lo, sh.row_hi = int(self.row_off[sh.img_lo]), int(self.row_off[sh.img_hi])
 
     # ------------------------------------------------------------------------------------------------ meta table
     def meta_for(self, rank):
@@ -112,37 +192,20 @@ class ShardPlan:
         return self.meta_for(None)
 
     # ------------------------------------------------------------------------------------------------ exchange plan
-    def _build_slices(self):
-        """Who sends what to whom.  DENS and OUT are copy launches described by slices; the other phases are fused into
-        the kernels, which only need destination masks (``aux``) -- and every phase needs its wait / signal masks."""
+    def _exchange(self, flag, add):
         w, L, m4 = self.world, self.layout, 4 * self.hp * self.wp
         P = _native
-        per = [[[] for _ in range(P.BL_PHASES)] for _ in range(w)]        # per[src][phase] = [(src_off, dst_off, bytes, dst)]
-        wait = np.zeros((w, P.BL_PHASES), dtype=np.uint32)
-        signal = np.zeros((w, P.BL_PHASES), dtype=np.uint32)
         c, b = self.total_chunks, self.batch
         zmask = np.zeros((w, c), dtype=np.uint32)      # per rank: destinations of a chunk's minima / denominator share
         gmask = np.zeros((w, c), dtype=np.uint32)      # rank that finishes the chunk's image (0: this rank itself)
         img_mask = np.zeros((w, b), dtype=np.uint32)   # the image's other ranks
         owner_mask = np.zeros((w, b), dtype=np.uint32)  # owner of the image's gradient (0: the finishing rank itself)
-
-        def flag(phase, src, dst):
-            if dst != src:
-                wait[dst, phase] |= np.uint32(1 << src)
-                signal[src, phase] |= np.uint32(1 << dst)
-
-        def add(phase, src, src_off, dst, dst_off, nbytes, flagged=True):
-            step = SLICE_BYTES if (src_off | dst_off | nbytes) % 16 == 0 else 1 << 30
-            for o in range(0, nbytes, step):
-                per[src][phase].append((src_off + o, dst_off + o, min(step, nbytes - o), dst))
-            if flagged:
-                flag(phase, src, dst)
-
         for i in range(b):
             g, lead, own = self.groups[i], int(self.lead[i]), int(self.owners[i])
             k_local = int(np.searchsorted(self.owned[own], i))
             for q in g:                                   # density: owner -> every rank that sweeps the image
                 add(P.BL_PH_DENS, own, k_local * m4, q, L.dens + i * m4, m4)
+                flag(P.BL_PH_DENS, own, q)
             c0, c1 = int(self.icb[i]), int(self.icb[i + 1])
             for ch in range(c0, c1):
                 r = int(self.c_owner[ch])
@@ -163,40 +226,8 @@ class ShardPlan:
             if own != lead:                               # finished gradient -> owner
                 owner_mask[lead, i] = np.uint32(1 << own)
                 flag(P.BL_PH_GRAD, lead, own)
-            add(P.BL_PH_OUT, own, L.gfinal + i * m4, own, k_local * m4, m4, flagged=False)
-        self.slices, self.shards, self.aux, self._dev = [], [], [], {}
-        for r in range(w):
-            rows, first = [], [0]
-            for ph in range(P.BL_PHASES):
-                rows += per[r][ph]
-                first.append(len(rows))
-            arr = np.zeros((max(len(rows), 1), 3), dtype=np.int64)   # (src_off, dst_off, bytes | dst_rank << 32): 24-byte records
-            if rows:
-                t = np.asarray(rows, dtype=np.int64)
-                arr[:len(rows), 0], arr[:len(rows), 1] = t[:, 0], t[:, 1]
-                arr[:len(rows), 2] = t[:, 2] | (t[:, 3] << 32)
-            self.slices.append(arr)
-            self.aux.append(np.concatenate([zmask[r], gmask[r], img_mask[r], owner_mask[r]]).astype(np.uint32))
-            sh = _native.BLShard()
-            sh.rank, sh.world = r, w
-            sh.chunk_lo, sh.chunk_hi = int(self.chunk_lo[r]), int(self.chunk_hi[r])
-            sh.pt_lo, sh.pt_hi = int(self.bounds[r]), int(self.bounds[r + 1])
-            sh.img_lo, sh.img_hi = int(self.img_lo[r]), int(self.img_hi[r])
-            sh.row_lo, sh.row_hi = int(self.row_off[sh.img_lo]), int(self.row_off[sh.img_hi])
-            for ph in range(P.BL_PHASES + 1):
-                sh.push_first[ph] = first[ph]
-            for ph in range(P.BL_PHASES):
-                sh.wait_mask[ph], sh.signal_mask[ph] = int(wait[r, ph]), int(signal[r, ph])
-            self.shards.append(sh)
-
-    def tables_on(self, rank, device):
-        """(slices, aux) of ``rank`` as device tensors (uploaded once per plan)."""
-        key = (rank, str(device))
-        t = self._dev.get(key)
-        if t is None:
-            t = self._dev[key] = (torch.from_numpy(self.slices[rank]).to(device),
-                                  torch.from_numpy(self.aux[rank].view(np.int32)).to(device))
-        return t
+            add(P.BL_PH_OUT, own, L.gfinal + i * m4, own, k_local * m4, m4)
+        return [np.concatenate([zmask[r], gmask[r], img_mask[r], owner_mask[r]]).astype(np.uint32) for r in range(w)]
 
 
 _plan_cache = {}
@@ -224,12 +255,7 @@ def plan_shards(counts, use_bg, world, owners, hp, wp, chunk=None):
     plan of the previous step is the common hit: forward and backward of one step share it)."""
     key = (tuple(int(c) for c in counts), bool(use_bg), int(world), None if owners is None else tuple(int(o) for o in owners),
            int(hp), int(wp), int(chunk or shard_chunk_points(sum(int(c) for c in counts), world)))
-    plan = _plan_cache.get(key)
-    if plan is None:
-        if len(_plan_cache) > 64:
-            _plan_cache.clear()
-        plan = _plan_cache[key] = ShardPlan(counts, use_bg, world, owners, hp, wp, key[-1])
-    return plan
+    return _cached_plan(_plan_cache, key, lambda: ShardPlan(counts, use_bg, world, owners, hp, wp, key[-1]))
 
 
 # ------------------------------------------------------------------------------------------------------ communicators
@@ -319,57 +345,42 @@ class LocalComm(IpcComm):
 
 
 # ------------------------------------------------------------------------------------------------------------ autograd
-class _ShardedFn(torch.autograd.Function):
+class _PeerFn(torch.autograd.Function):
+    """One rank's forward / backward of either peer split; the native launches are the module's ``_forward`` /
+    ``_backward`` (one ctypes call each)."""
+
     @staticmethod
     def forward(ctx, density_local, mod, plan, packed, st, inv_batch):
-        comm, pp = mod.comm, mod.post_prob
+        comm = mod.comm
         dev, r = comm.device, comm.rank
-        _native.require_cuda(st, "ChunkShardedBL.forward")
-        hp, wp, L = plan.hp, plan.wp, plan.layout
+        _native.require_cuda(st, f"{type(mod).__name__}.forward")
         n_own = len(plan.owned[r])
-        dens = density_local.detach().reshape(n_own, hp, wp).to(torch.float32).contiguous() if n_own else None
-        if L.total > comm.nbytes:
-            raise RuntimeError(f"sharded workspace of {comm.nbytes} bytes is too small for this batch ({L.total} bytes); "
-                               "create the communicator with a larger nbytes")
+        dens = density_local.detach().reshape(n_own, plan.hp, plan.wp).to(torch.float32).contiguous() if n_own else None
+        if plan.layout.total > comm.nbytes:
+            raise RuntimeError(f"sharded workspace of {comm.nbytes} bytes is too small for this batch ({plan.layout.total} "
+                               "bytes); create the communicator with a larger nbytes")
         comm.epoch += 1
         shard = plan.shards[r]
-        shard.epoch = comm.epoch
-        slices, aux = plan.tables_on(r, dev)
-        shard.fuse_waits = int(comm.fuse_waits)
+        shard.epoch, shard.fuse_waits = comm.epoch, int(comm.fuse_waits)
+        tables = plan.tables_on(r, dev)
         loss = torch.empty((1,), dtype=torch.float32, device=dev)
-        # deferred loss: only when a backward pass will follow (it carries the closing launches)
-        defer = bool(mod.defer_loss and ctx.needs_input_grad[0])
-        rc = _native.lib().dgvcc_bl_shard_forward(
-            _native.ptr(packed.pts), _native.ptr(packed.targets), _native.ptr(packed.meta), _native.ptr(st), _native.ptr(dens),
-            plan.batch, hp, wp, plan.total_rows, plan.total_chunks, plan.multi_chunk, float(pp.stride), float(pp.sigma),
-            float(pp.bg_ratio), int(pp.use_bg), int(mod.exact_cull), inv_batch, ctypes.byref(shard), _native.ptr(slices),
-            _native.ptr(aux), _native.ptr(comm.peer_table), _native.ptr(comm.workspace), comm.nbytes, _native.ptr(loss),
-            int(defer), _native.stream_ptr(dev), mod._event_handles("fwd", 9))
-        _native.check(rc, "dgvcc_bl_shard_forward")
-        ctx.saved = (mod, plan, packed, (slices, aux), inv_batch, comm.epoch, density_local.shape, density_local.dtype, n_own,
-                     loss if defer else None)
+        deferred = mod._forward(plan, packed, st, dens, inv_batch, shard, tables, loss, ctx.needs_input_grad[0])
+        ctx.saved = (mod, plan, packed, tables, inv_batch, comm.epoch, density_local.shape, density_local.dtype, n_own, deferred)
         return loss.reshape(())
 
     @staticmethod
     def backward(ctx, grad_loss):
-        mod, plan, packed, (slices, aux), inv_batch, epoch, shape, dtype, n_own, deferred = ctx.saved
-        comm, pp = mod.comm, mod.post_prob
-        dev, r = comm.device, comm.rank
+        mod, plan, packed, tables, inv_batch, epoch, shape, dtype, n_own, deferred = ctx.saved
+        comm = mod.comm
+        dev = comm.device
         if epoch != comm.epoch:
-            raise RuntimeError("ChunkShardedBL: backward of a step whose shared workspace was already re-used by a later "
-                               "forward (one forward/backward pair at a time per communicator)")
-        shard = plan.shards[r]
-        shard.epoch = epoch
-        shard.fuse_waits = int(comm.fuse_waits)
+            raise RuntimeError(f"{type(mod).__name__}: backward of a step whose shared workspace was already re-used by a "
+                               "later forward (one forward/backward pair at a time per communicator)")
+        shard = plan.shards[comm.rank]
+        shard.epoch, shard.fuse_waits = epoch, int(comm.fuse_waits)
         g = grad_loss.detach().to(device=dev, dtype=torch.float32).reshape(1).contiguous()
         grad = torch.empty((max(n_own, 1), plan.hp, plan.wp), dtype=torch.float32, device=dev)
-        rc = _native.lib().dgvcc_bl_shard_backward(
-            _native.ptr(packed.pts), _native.ptr(packed.meta), plan.batch, plan.hp, plan.wp, plan.total_rows,
-            plan.total_chunks, float(pp.stride), float(pp.sigma), int(pp.use_bg), int(mod.exact_cull), inv_batch,
-            _native.ptr(g), ctypes.byref(shard), _native.ptr(slices), _native.ptr(aux), _native.ptr(comm.peer_table),
-            _native.ptr(comm.workspace), comm.nbytes, _native.ptr(grad), _native.ptr(deferred), _native.stream_ptr(dev),
-            mod._event_handles("bwd", 5))
-        _native.check(rc, "dgvcc_bl_shard_backward")
+        mod._backward(plan, packed, inv_batch, g, shard, tables, grad, deferred)
         return (grad[:n_own].reshape(shape).to(dtype),) + (None,) * 5
 
 
@@ -378,26 +389,20 @@ class _PackedAll:
 
     def __init__(self, points, targets, plan, rank, device):
         meta = plan.meta_for(rank)
-        n = max(plan.total_points, 1)
-        o_pts = _bl._align16(meta.nbytes)
-        o_tgt = o_pts + _bl._align16(8 * n)
-        total = o_tgt + _bl._align16(4 * n)
+        o_pts, o_tgt, total = _bl._pack_into(None, meta, points, targets, plan.total_points)
         host = torch.empty((total,), dtype=torch.uint8, pin_memory=True)
-        view = host.numpy()
-        view[:meta.nbytes].view(np.int32)[:] = meta
-        if plan.total_points:
-            np.concatenate([_bl._host_f32(p.cpu()).reshape(-1, 2) for p in points if p.numel()], axis=0,
-                           out=view[o_pts:o_pts + 8 * plan.total_points].view(np.float32).reshape(-1, 2))
-            np.concatenate([_bl._host_f32(t.cpu()).reshape(-1) for t in targets if t.numel()],
-                           out=view[o_tgt:o_tgt + 4 * plan.total_points].view(np.float32))
+        _bl._pack_into(host.numpy(), meta, points, targets, plan.total_points)
         buf = host.to(device, non_blocking=True)
+        n = max(plan.total_points, 1)
         self.meta = buf[:meta.nbytes].view(torch.int32)
         self.pts = buf[o_pts:o_pts + 8 * n].view(torch.float32).view(-1, 2)
         self.targets = buf[o_tgt:o_tgt + 4 * n].view(torch.float32)
 
 
-class ChunkShardedBL(Module):
-    """``BL`` for one batch spread over ``comm.world`` GPUs by point chunks (module docstring)."""
+class _PeerBL(Module):
+    """What both peer splits of ``BL`` share: the forward (plan, re-pack cache, ``_PeerFn``), the per-phase timing and
+    the error check.  A split supplies ``_plan``, the launches ``_forward`` / ``_backward`` and the names of the phases
+    its launches time (``FWD_PHASES`` / ``BWD_PHASES``: one event before each phase and one after the last)."""
 
     def __init__(self, sigma, c_size, stride, background_ratio, use_background, device, comm):
         super().__init__()
@@ -405,40 +410,32 @@ class ChunkShardedBL(Module):
         self.bay_loss = _bl.Bay_Loss(use_background, device)
         self.comm = comm
         self.exact_cull = True
-        # The images' losses come from all ranks: waiting for them is a barrier over the whole group that the backward pass
-        # does not need.  With defer_loss (and a backward pass to follow) the forward returns at once and the backward
-        # launches close with that wait: the returned tensor holds the loss once ``backward()`` has been called --
-        # the usual order of a training step (``loss.backward(); loss.item()``).  False: complete after forward.
-        self.defer_loss = False
         self._last = None   # (key, packed): a benchmark / test that feeds the same lists again skips the re-pack
 
     def forward(self, points, st_sizes, target_list, pre_density_local, owners=None):
-        comm, pp = self.comm, self.post_prob
+        comm = self.comm
         dev = comm.device
         points = _bl._as_point_list(points)
         counts = [int(p.shape[0]) for p in points]
         hp, wp = int(pre_density_local.shape[-2]), int(pre_density_local.shape[-1])
-        plan = plan_shards(counts, pp.use_bg, comm.world, owners, hp, wp)
+        plan = self._plan(counts, owners, hp, wp)
         if pre_density_local.shape[0] != len(plan.owned[comm.rank]):
             raise ValueError(f"rank {comm.rank} owns {len(plan.owned[comm.rank])} images of this batch but was given "
                              f"{pre_density_local.shape[0]} density maps")
-        key = (id(points[0]) if points else 0, id(plan), tuple(id(p) for p in points), tuple(id(t) for t in target_list))
+        key = (id(plan), tuple(id(p) for p in points), tuple(id(t) for t in target_list))
         if self._last is not None and self._last[0] == key:
             packed = self._last[1]
         else:
             packed = _PackedAll(points, target_list, plan, comm.rank, dev)
             self._last = (key, packed, points, target_list)   # the lists are kept alive so that the ids stay meaningful
         st = st_sizes.to(device=dev, dtype=torch.float32).contiguous()
-        return _ShardedFn.apply(pre_density_local, self, plan, packed, st, 1.0 / plan.batch)
+        return _PeerFn.apply(pre_density_local, self, plan, packed, st, 1.0 / plan.batch)
 
-    FWD_PHASES = ["issue DENS copy (side stream)", "grid build + minima", "z (+Z out)", "[wait Z, DENS] finish_z", "counts",
-                  "reduce_counts (+CNT out)", "[wait CNT] select (+LOSS out)", "[wait LOSS] loss"]
-    BWD_PHASES = ["grad (+GPART out)", "[wait GPART] reduce (+GRAD out)", "[wait GRAD] gather", "[wait LOSS] deferred loss"]
-
-    def _event_handles(self, which, n):
+    def _event_handles(self, which):
         """None, or ctypes array of cudaEvent_t for the per-phase timing (``profile = True``)."""
         if not getattr(self, "profile", False):
             return None
+        n = len(self.FWD_PHASES if which == "fwd" else self.BWD_PHASES) + 1
         evs = [torch.cuda.Event(enable_timing=True) for _ in range(n)]
         for e in evs:
             e.record()  # materialises the handle
@@ -463,7 +460,49 @@ class ChunkShardedBL(Module):
         err = int(self.comm.workspace[off:off + 4].view(torch.int32).item())
         if err:
             ph, src = (err - 1) % 16, (err - 1) // 16
-            raise RuntimeError(f"ChunkShardedBL rank {self.comm.rank}: no flag of phase {ph} from rank {src} within 2 s")
+            raise RuntimeError(f"{type(self).__name__} rank {self.comm.rank}: no flag of phase {ph} from rank {src} within 2 s")
+
+
+class ChunkShardedBL(_PeerBL):
+    """``BL`` for one batch spread over ``comm.world`` GPUs by point chunks (module docstring)."""
+
+    FWD_PHASES = ["issue DENS copy (side stream)", "grid build + minima", "z (+Z out)", "[wait Z, DENS] finish_z", "counts",
+                  "reduce_counts (+CNT out)", "[wait CNT] select (+LOSS out)", "[wait LOSS] loss"]
+    BWD_PHASES = ["grad (+GPART out)", "[wait GPART] reduce (+GRAD out)", "[wait GRAD] gather", "[wait LOSS] deferred loss"]
+
+    def __init__(self, sigma, c_size, stride, background_ratio, use_background, device, comm):
+        super().__init__(sigma, c_size, stride, background_ratio, use_background, device, comm)
+        # The images' losses come from all ranks: waiting for them is a barrier over the whole group that the backward pass
+        # does not need.  With defer_loss (and a backward pass to follow) the forward returns at once and the backward
+        # launches close with that wait: the returned tensor holds the loss once ``backward()`` has been called --
+        # the usual order of a training step (``loss.backward(); loss.item()``).  False: complete after forward.
+        self.defer_loss = False
+
+    def _plan(self, counts, owners, hp, wp):
+        return plan_shards(counts, self.post_prob.use_bg, self.comm.world, owners, hp, wp)
+
+    def _forward(self, plan, packed, st, dens, inv_batch, shard, tables, loss, backward_follows):
+        """dgvcc_bl_shard_forward; returns ``loss`` when the backward pass is to complete it (defer_loss), else None."""
+        comm, pp = self.comm, self.post_prob
+        defer = bool(self.defer_loss and backward_follows)   # the backward pass carries the closing launches
+        rc = _native.lib().dgvcc_bl_shard_forward(
+            _native.ptr(packed.pts), _native.ptr(packed.targets), _native.ptr(packed.meta), _native.ptr(st), _native.ptr(dens),
+            plan.batch, plan.hp, plan.wp, plan.total_rows, plan.total_chunks, plan.multi_chunk, float(pp.stride),
+            float(pp.sigma), float(pp.bg_ratio), int(pp.use_bg), int(self.exact_cull), inv_batch, ctypes.byref(shard),
+            _native.ptr(tables[0]), _native.ptr(tables[1]), _native.ptr(comm.peer_table), _native.ptr(comm.workspace),
+            comm.nbytes, _native.ptr(loss), int(defer), _native.stream_ptr(comm.device), self._event_handles("fwd"))
+        _native.check(rc, "dgvcc_bl_shard_forward")
+        return loss if defer else None
+
+    def _backward(self, plan, packed, inv_batch, g, shard, tables, grad, deferred):
+        comm, pp = self.comm, self.post_prob
+        rc = _native.lib().dgvcc_bl_shard_backward(
+            _native.ptr(packed.pts), _native.ptr(packed.meta), plan.batch, plan.hp, plan.wp, plan.total_rows,
+            plan.total_chunks, float(pp.stride), float(pp.sigma), int(pp.use_bg), int(self.exact_cull), inv_batch,
+            _native.ptr(g), ctypes.byref(shard), _native.ptr(tables[0]), _native.ptr(tables[1]), _native.ptr(comm.peer_table),
+            _native.ptr(comm.workspace), comm.nbytes, _native.ptr(grad), _native.ptr(deferred),
+            _native.stream_ptr(comm.device), self._event_handles("bwd"))
+        _native.check(rc, "dgvcc_bl_shard_backward")
 
 
 def plan_err_offset(world):
