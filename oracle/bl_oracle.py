@@ -41,24 +41,35 @@ def sq_distances(points, hp, wp, stride, dtype=torch.float32):
     return dis.reshape(dis.size(0), -1)
 
 
-def posterior_from_dis(dis, st_size, sigma, bg_ratio, use_bg):
-    """Softmax over points (+ background row appended last).  bl.py:38-44."""
+def ieee_sqrt(t):
+    """Correctly rounded square root: torch.sqrt on CUDA, where the reference trains, and the kernels' __fsqrt_rn.
+    torch's CPU sqrt of a long fp32 tensor (the MKL vector path) is one ulp off in about 0.7 % of the elements -- the
+    fixtures under tests/golden hold those roots -- and one ulp of the root moves a pixel's background argument
+    (bl.py:41) by up to ~10 ulp.  The fp64 root rounded once to fp32 is the IEEE fp32 root."""
+    if t.dtype == torch.float32:
+        return torch.sqrt(t.double()).to(torch.float32)
+    return torch.sqrt(t)
+
+
+def posterior_from_dis(dis, st_size, sigma, bg_ratio, use_bg, sqrt=torch.sqrt):
+    """Softmax over points (+ background row appended last).  bl.py:38-44.  ``sqrt``: ``ieee_sqrt`` for the roots of
+    the reference's CUDA run (the default, torch's CPU sqrt, reproduces its CPU run and the fixtures)."""
     if use_bg:
         min_dis = torch.clamp(torch.min(dis, dim=0, keepdim=True)[0], min=0.0)
         d = st_size * bg_ratio
-        bg_dis = (d - torch.sqrt(min_dis)) ** 2
+        bg_dis = (d - sqrt(min_dis)) ** 2
         dis = torch.cat([dis, bg_dis], 0)
     dis = -dis / (2.0 * sigma ** 2)
     return torch.softmax(dis, dim=0)
 
 
 def posterior(points, st_size, hp, wp, stride, sigma, bg_ratio=1.0, use_bg=True,
-              dtype=torch.float32):
+              dtype=torch.float32, sqrt=torch.sqrt):
     """Posterior matrix of ONE image, [N(+1), H'*W'], or None when it has no points."""
     if len(points) == 0:
         return None
     st = torch.as_tensor(st_size, dtype=dtype)
-    return posterior_from_dis(sq_distances(points, hp, wp, stride, dtype), st, sigma, bg_ratio, use_bg)
+    return posterior_from_dis(sq_distances(points, hp, wp, stride, dtype), st, sigma, bg_ratio, use_bg, sqrt)
 
 
 def trimmed_l1(residual):
@@ -77,7 +88,7 @@ def image_target(targets, n_rows, use_bg, dtype=torch.float32):
 
 
 def bl_forward_backward(points, st_sizes, targets, density, stride, sigma,
-                        bg_ratio=1.0, use_bg=True, dtype=torch.float32):
+                        bg_ratio=1.0, use_bg=True, dtype=torch.float32, sqrt=torch.sqrt):
     """Materialising oracle: loss, d loss / d density, per-image expected counts.
 
     ``density`` is [B,1,H',W'].  Uses autograd exactly like the reference
@@ -88,7 +99,7 @@ def bl_forward_backward(points, st_sizes, targets, density, stride, sigma,
     loss = 0
     counts = []
     for i in range(B):
-        prob = posterior(points[i], st_sizes[i], hp, wp, stride, sigma, bg_ratio, use_bg, dtype)
+        prob = posterior(points[i], st_sizes[i], hp, wp, stride, sigma, bg_ratio, use_bg, dtype, sqrt)
         if prob is None:
             pre_count = torch.sum(dens[i]).reshape(1)
             target = torch.zeros((1,), dtype=dtype)
@@ -104,7 +115,7 @@ def bl_forward_backward(points, st_sizes, targets, density, stride, sigma,
 
 def bl_forward_backward_chunked(points, st_sizes, targets, density, stride, sigma,
                                 bg_ratio=1.0, use_bg=True, dtype=torch.float32,
-                                chunk_rows=16):
+                                chunk_rows=16, sqrt=torch.sqrt):
     """Same numbers without holding [N+1, M]: row bands of the grid, explicit gradient.
 
     Per-pixel independence of the posterior makes band-wise evaluation exact;
@@ -134,7 +145,7 @@ def bl_forward_backward_chunked(points, st_sizes, targets, density, stride, sigm
 
         def band_prob(r0, r1):
             dis = (y_dis[:, r0:r1].unsqueeze(2) + x_dis.unsqueeze(1)).reshape(len(pts), -1)
-            return posterior_from_dis(dis, st, sigma, bg_ratio, use_bg)
+            return posterior_from_dis(dis, st, sigma, bg_ratio, use_bg, sqrt)
 
         for r0 in range(0, hp, chunk_rows):
             r1 = min(hp, r0 + chunk_rows)

@@ -21,14 +21,15 @@ def _region(keep, name, n):
     return ws[off:off + 4 * n].view(torch.float32)
 
 
-def run_cuda(points, st_sizes, targets, density, stride, sigma, bg_ratio, use_bg, c_size=None, exact_cull=False):
+def run_cuda(points, st_sizes, targets, density, stride, sigma, bg_ratio, use_bg, c_size=None, exact_cull=False, keep=None):
+    """``keep``: a dict that receives the step's workspace and layout (``_region`` reads them)."""
     from dgvcc_b200.losses.bl import BL
     dev = torch.device("cuda:0")
     b, _, hp, wp = density.shape
     mod = BL(sigma, c_size or max(hp, wp) * stride, stride, bg_ratio, use_bg, dev)
     mod.exact_cull = exact_cull
     d = density.to(dev).clone().requires_grad_(True)
-    keep = {}
+    keep = {} if keep is None else keep
     loss = mod([p.to(dev) for p in points], st_sizes.to(dev), [t.to(dev) for t in targets], d, _keep=keep)
     loss.backward()
     torch.cuda.synchronize()
