@@ -52,6 +52,7 @@ class DmapPlan(ctypes.Structure):
 
 
 DMAP_META_COLS = 12  # DGVCC_DMAP_META_COLS
+DTYPE_F16, DTYPE_BF16 = 1, 2  # DGVCC_DTYPE_F16, DGVCC_DTYPE_BF16
 DEN_META_COLS = 8    # DGVCC_DEN_META_COLS
 
 # name -> (restype, argtypes); every symbol include/dgvcc_b200.h declares must appear here
@@ -113,6 +114,16 @@ SIGNATURES = {
                                        c_size_t, c_void_p, c_void_p]),
     "dgvcc_isw_loss_backward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                                         c_int, c_void_p, c_size_t, c_void_p, c_void_p]),
+    "dgvcc_isw_instnorm_forward_h": (c_int, [c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p,
+                                             c_void_p]),
+    "dgvcc_isw_instnorm_backward_h": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p,
+                                              c_void_p]),
+    "dgvcc_isw_covariance_h": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_size_t, c_void_p,
+                                       c_void_p]),
+    "dgvcc_isw_covariance_backward_h": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_size_t,
+                                                c_void_p, c_void_p]),
+    "dgvcc_isw_loss_backward_h": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
+                                          c_int, c_void_p, c_size_t, c_void_p, c_void_p]),
     "dgvcc_isw_sx_tc": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
     "dgvcc_isw_covstat_var": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "dgvcc_isw_topk_mask": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),

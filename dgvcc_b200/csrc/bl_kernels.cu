@@ -1998,7 +1998,7 @@ static T* at(const void* ws, int64_t off) { return reinterpret_cast<T*>((char*)w
 using namespace dgvcc;
 using namespace dgvcc::bl;
 
-extern "C" int dgvcc_abi_version(void) { return 9; }
+extern "C" int dgvcc_abi_version(void) { return 10; }
 extern "C" int dgvcc_bounds_checked(void) { return DGVCC_BOUNDS_CHECKED; }
 
 extern "C" int dgvcc_bl_workspace_layout(int64_t total_rows, int total_chunks, int batch, int hp, int wp,

@@ -23,6 +23,14 @@
 //              quarter w % 4, warps 2-5 the left 64 columns, warps 6-9 the right 64) and store the tile
 // Pipeline: full[s] (TMA -> converters), ready[s] (converters -> MMA), empty[s] (MMA -> TMA) over
 // STAGES shared-memory stages; acc_full[set] (MMA -> drain), acc_empty[set] (drain -> MMA).
+//
+// Half-precision input (isw_gram_tc_kernel<__half / __nv_bfloat16>): TMA loads the 32 k x 128 row half tiles (64-byte
+// rows, no swizzle) behind the two fp32 tiles of the stage, and the converters widen them into those fp32 tiles in the
+// 128B-swizzled layout TMA writes for fp32 input.  A widened half value is its own TF32 hi and its lo is exactly 0, so
+// the cross accumulator is dropped: one MMA per k step, TMEM 2 x 128 columns, same enable flags, SEG_KB segments and
+// drain order, hence the same partials bit for bit as the fp32 kernel on the upcast map.
+#include <type_traits>
+
 #include "tc_common.cuh"
 #include "../../include/dgvcc_b200.h"
 
@@ -36,11 +44,17 @@ constexpr int STAGES = 3;
 constexpr bool HI_BY_TRUNCATION = true;     // hi = what the tensor core reads of the raw tile (see the converter loop)
 constexpr int SEG_KB = 16;                  // k blocks accumulated in TMEM before a drain (512 k = 64 steps)
 constexpr int TILE_BYTES = TILE_M * BLOCK_K * 4;  // 16 KB
-constexpr int STAGE_BYTES = 4 * TILE_BYTES;       // A_hi, B_hi, A_lo, B_lo
+constexpr int HTILE_BYTES = TILE_M * BLOCK_K * 2; // 8 KB: a half-precision tile as TMA delivers it
 constexpr int CONVERTER_WARPS = 8;                // two per SM sub-partition
 constexpr int THREADS = 64 + 32 * CONVERTER_WARPS;
-constexpr int TMEM_COLS = 512;  // two accumulator sets, each: hi*hi^T (128 columns) + cross terms (128 columns)
-constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /*alignment slack*/ + 256 /*barriers*/;
+template <typename T> struct Cfg {
+    static constexpr bool HALF = !std::is_same<T, float>::value;
+    // fp32: A_hi, B_hi, A_lo, B_lo.  half: A, B (fp32, widened), then the two half tiles TMA wrote
+    static constexpr int STAGE_BYTES = HALF ? 2 * TILE_BYTES + 2 * HTILE_BYTES : 4 * TILE_BYTES;
+    // two accumulator sets, each: hi*hi^T (128 columns) + cross terms (128 columns; none for half input)
+    static constexpr int TMEM_COLS = HALF ? 256 : 512;
+    static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /*alignment slack*/ + 256 /*barriers*/;
+};
 
 using namespace dgvcc::tc;
 
@@ -50,14 +64,19 @@ __device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr) { return umma_
 // kind::tf32, fp32 accumulate, A and B K-major, M = N = 128.
 constexpr uint32_t IDESC = umma_idesc_tf32(TILE_M, TILE_M, false);
 
+int launch_half(const void* x, int dtype, int batch, int c, int hw, int splits, int k_per_split, float* part, void* stream);
+
 struct Args {
     int c, hw, batch, splits, k_per_split, tiles_1d, n_tiles;
     int pair;     // c <= 64: one CTA holds two samples (64 rows each) in its 128-row tile
     float* part;  // [batch][splits][n_tiles][tile][tile], tile = 64 in pair mode, else 128
 };
 
+template <typename T>
 __global__ void __launch_bounds__(THREADS, 1)
 isw_gram_tc_kernel(const __grid_constant__ CUtensorMap tmap, const Args a) {
+    constexpr bool HALF = Cfg<T>::HALF;
+    constexpr int STAGE_BYTES = Cfg<T>::STAGE_BYTES, TMEM_COLS = Cfg<T>::TMEM_COLS;
     extern __shared__ uint8_t smem_raw[];
     // 1024-byte alignment for the 128B-swizzled tiles
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -114,10 +133,17 @@ isw_gram_tc_kernel(const __grid_constant__ CUtensorMap tmap, const Args a) {
                 const uint32_t ph = (kb / STAGES) & 1;
                 mbar_wait(empty_bar(s), ph ^ 1u);
                 const uint32_t stage = base + s * STAGE_BYTES;
-                mbar_arrive_expect_tx(full_bar(s), diag ? TILE_BYTES : 2 * TILE_BYTES);
-                // pair mode: the box is {32 k, 64 rows, 2 samples} = the same 128 x 128-byte tile
-                tma_load_3d(stage, &tmap, full_bar(s), k0 + kb * BLOCK_K, ti * TILE_M, b);
-                if (!diag) tma_load_3d(stage + TILE_BYTES, &tmap, full_bar(s), k0 + kb * BLOCK_K, tj * TILE_M, b);
+                // pair mode: the box is {32 k, 64 rows, 2 samples} = the same 128-row tile
+                if constexpr (HALF) {
+                    mbar_arrive_expect_tx(full_bar(s), diag ? HTILE_BYTES : 2 * HTILE_BYTES);
+                    const uint32_t h = stage + 2 * TILE_BYTES;
+                    tma_load_3d(h, &tmap, full_bar(s), k0 + kb * BLOCK_K, ti * TILE_M, b);
+                    if (!diag) tma_load_3d(h + HTILE_BYTES, &tmap, full_bar(s), k0 + kb * BLOCK_K, tj * TILE_M, b);
+                } else {
+                    mbar_arrive_expect_tx(full_bar(s), diag ? TILE_BYTES : 2 * TILE_BYTES);
+                    tma_load_3d(stage, &tmap, full_bar(s), k0 + kb * BLOCK_K, ti * TILE_M, b);
+                    if (!diag) tma_load_3d(stage + TILE_BYTES, &tmap, full_bar(s), k0 + kb * BLOCK_K, tj * TILE_M, b);
+                }
             }
         }
     } else if (warp == 1) {
@@ -136,15 +162,24 @@ isw_gram_tc_kernel(const __grid_constant__ CUtensorMap tmap, const Args a) {
                 const uint32_t stage = base + s * STAGE_BYTES;
                 const uint64_t a_hi = umma_desc(stage);
                 const uint64_t b_hi = umma_desc(stage + (diag ? 0 : TILE_BYTES));
-                const uint64_t a_lo = umma_desc(stage + 2 * TILE_BYTES);
-                const uint64_t b_lo = umma_desc(stage + (diag ? 2 : 3) * TILE_BYTES);
-                const uint32_t d_main = tmem_d + (uint32_t)set * 2 * TILE_M, d_cross = d_main + TILE_M;
+                if constexpr (HALF) {  // lo == 0: hi hi^T only
+                    const uint32_t d_main = tmem_d + (uint32_t)set * TILE_M;
 #pragma unroll
-                for (int ks = 0; ks < BLOCK_K / UMMA_K; ++ks) {
-                    const uint64_t adv = (uint64_t)((ks * UMMA_K * 4) >> 4);  // +32 B inside the swizzle row
-                    umma_tf32(d_main, a_hi + adv, b_hi + adv, IDESC, (kin | ks) != 0);
-                    umma_tf32(d_cross, a_hi + adv, b_lo + adv, IDESC, (kin | ks) != 0);
-                    umma_tf32(d_cross, a_lo + adv, b_hi + adv, IDESC, 1u);
+                    for (int ks = 0; ks < BLOCK_K / UMMA_K; ++ks) {
+                        const uint64_t adv = (uint64_t)((ks * UMMA_K * 4) >> 4);
+                        umma_tf32(d_main, a_hi + adv, b_hi + adv, IDESC, (kin | ks) != 0);
+                    }
+                } else {
+                    const uint64_t a_lo = umma_desc(stage + 2 * TILE_BYTES);
+                    const uint64_t b_lo = umma_desc(stage + (diag ? 2 : 3) * TILE_BYTES);
+                    const uint32_t d_main = tmem_d + (uint32_t)set * 2 * TILE_M, d_cross = d_main + TILE_M;
+#pragma unroll
+                    for (int ks = 0; ks < BLOCK_K / UMMA_K; ++ks) {
+                        const uint64_t adv = (uint64_t)((ks * UMMA_K * 4) >> 4);  // +32 B inside the swizzle row
+                        umma_tf32(d_main, a_hi + adv, b_hi + adv, IDESC, (kin | ks) != 0);
+                        umma_tf32(d_cross, a_hi + adv, b_lo + adv, IDESC, (kin | ks) != 0);
+                        umma_tf32(d_cross, a_lo + adv, b_hi + adv, IDESC, 1u);
+                    }
                 }
                 umma_commit(empty_bar(s));  // frees the stage once these MMAs have read it
                 if (kin == SEG_KB - 1 || kb == n_kb - 1) umma_commit(acc_full_bar(set));
@@ -167,7 +202,18 @@ isw_gram_tc_kernel(const __grid_constant__ CUtensorMap tmap, const Args a) {
             const int set = seg & 1;
             mbar_wait(acc_full_bar(set), (uint32_t)(seg >> 1) & 1u);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            if (useful) {
+            if constexpr (HALF) {
+                if (useful) {
+#pragma unroll
+                    for (int h = 0; h < 2; ++h) {
+                        uint32_t r[32];
+                        tmem_ld32(tmem_d + ((uint32_t)lane_base << 16) + (uint32_t)(set * TILE_M + col_begin + 32 * h), r);
+                        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+                        for (int q = 0; q < 32; ++q) acc[32 * h + q] += __uint_as_float(r[q]);
+                    }
+                }
+            } else if (useful) {
 #pragma unroll
                 for (int h = 0; h < 2; ++h) {
                     uint32_t r[32], x[32];
@@ -190,6 +236,21 @@ isw_gram_tc_kernel(const __grid_constant__ CUtensorMap tmap, const Args a) {
             const uint32_t ph = (kb / STAGES) & 1;
             mbar_wait(full_bar(s), ph);
             uint8_t* stage = base_ptr + s * STAGE_BYTES;
+            if constexpr (HALF) {
+                // widen [A; B] (128 or 256 rows of 32 half values) into the fp32 tiles: one float4 per thread and step,
+                // 16-byte chunk k4 of row r at chunk k4 ^ (r % 8) of the 128-byte row (the 128B swizzle)
+                const T* src = reinterpret_cast<const T*>(stage + 2 * TILE_BYTES);
+#pragma unroll 4
+                for (int i = ctid; i < (diag ? 1 : 2) * TILE_M * (BLOCK_K / 4); i += 32 * CONVERTER_WARPS) {
+                    const int r = i >> 3, k4 = i & 7;
+                    *reinterpret_cast<float4*>(stage + r * 128 + ((k4 ^ (r & 7)) << 4)) = widen4(src + r * BLOCK_K + 4 * k4);
+                }
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                __syncwarp();
+                if (lane == 0) mbar_arrive(ready_bar(s));
+                while (drained < n_seg - 1 && kb >= (drained + 1) * SEG_KB + 1) drain(drained++);
+                continue;
+            }
             const int n_vec = (diag ? 1 : 2) * (TILE_BYTES / 16);  // float4s of A_hi (and B_hi, contiguous after it)
             float4* hi = reinterpret_cast<float4*>(stage);
             float4* lo = reinterpret_cast<float4*>(stage + 2 * TILE_BYTES);
@@ -277,7 +338,8 @@ extern "C" int dgvcc_isw_gram_tc_partials(const float* x, int batch, int c, int 
 
     static PerDeviceOnce once;
     if (once.first())
-        DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_gram_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+        DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_gram_tc_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                  Cfg<float>::SMEM_BYTES));
     Args a;
     a.c = c; a.hw = hw; a.batch = batch; a.splits = splits; a.k_per_split = k_per_split;
     a.pair = pair;
@@ -285,6 +347,39 @@ extern "C" int dgvcc_isw_gram_tc_partials(const float* x, int batch, int c, int 
     a.n_tiles = a.tiles_1d * (a.tiles_1d + 1) / 2;
     a.part = part;
     const int grid_z = pair ? ceil_div(batch, 2) : batch;
-    isw_gram_tc_kernel<<<dim3(a.n_tiles, splits, grid_z), THREADS, SMEM_BYTES, (cudaStream_t)stream>>>(tmap, a);
+    isw_gram_tc_kernel<float><<<dim3(a.n_tiles, splits, grid_z), THREADS, Cfg<float>::SMEM_BYTES, (cudaStream_t)stream>>>(tmap, a);
     return (int)cudaGetLastError();
+}
+
+template <typename T>
+static int gram_tc_half(const void* x, int batch, int c, int hw, int splits, int k_per_split, float* part, void* stream) {
+    const int pair = c <= 64;
+    CUtensorMap tmap;
+    if (!make_tmap_3d(&tmap, HalfIn<T>::TMA, 2, x, (uint64_t)hw, (uint64_t)c, (uint64_t)batch, BLOCK_K, pair ? 64 : TILE_M,
+                      CU_TENSOR_MAP_SWIZZLE_NONE, pair ? 2 : 1))
+        return DGVCC_ERR_UNSUPPORTED;
+    static PerDeviceOnce once;
+    if (once.first())
+        DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_gram_tc_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                  Cfg<T>::SMEM_BYTES));
+    Args a;
+    a.c = c; a.hw = hw; a.batch = batch; a.splits = splits; a.k_per_split = k_per_split;
+    a.pair = pair;
+    a.tiles_1d = pair ? 1 : ceil_div(c, TILE_M);
+    a.n_tiles = a.tiles_1d * (a.tiles_1d + 1) / 2;
+    a.part = part;
+    const int grid_z = pair ? ceil_div(batch, 2) : batch;
+    isw_gram_tc_kernel<T><<<dim3(a.n_tiles, splits, grid_z), THREADS, Cfg<T>::SMEM_BYTES, (cudaStream_t)stream>>>(tmap, a);
+    return (int)cudaGetLastError();
+}
+
+// The same partials from a half-precision map (dtype DGVCC_DTYPE_F16 / _BF16).  TMA needs 16-byte global strides
+// (hw % 8 == 0) and a 16-byte aligned base; c % 4 == 0 keeps one shape rule for the Gram and dX = S X (isw_sx_tc.cu).
+int dgvcc::isw_tc::launch_half(const void* x, int dtype, int batch, int c, int hw, int splits, int k_per_split, float* part,
+                               void* stream) {
+    if (!x || !part || batch <= 0 || c <= 0 || hw <= 0 || splits <= 0 || k_per_split <= 0) return DGVCC_ERR_ARG;
+    if (dtype != DGVCC_DTYPE_F16 && dtype != DGVCC_DTYPE_BF16) return DGVCC_ERR_ARG;
+    if (hw % 8 != 0 || c < 32 || c % 4 != 0 || k_per_split % BLOCK_K != 0 || ((uintptr_t)x & 15u)) return DGVCC_ERR_UNSUPPORTED;
+    return dtype == DGVCC_DTYPE_F16 ? gram_tc_half<__half>(x, batch, c, hw, splits, k_per_split, part, stream)
+                                    : gram_tc_half<__nv_bfloat16>(x, batch, c, hw, splits, k_per_split, part, stream);
 }

@@ -13,7 +13,10 @@
 //   isw_sx_simt_kernel          : dX_b = S_b X_b  (exact fp32; the tensor-core version is isw_sx_tc.cu)
 //                                                                                 autograd of :37
 // Deterministic: no float atomics; split-K partials are added in split order.
-#include "common.cuh"
+// Half-precision feature maps (fp16 / bf16, the *_h entry points): the instance norm is templated over the element type
+// and the Gram / dX = S X run the half variants of the tensor-core kernels; every value is the one the fp32 path computes
+// on the upcast map (DESIGN section 5).
+#include "tc_common.cuh"
 #include "../../include/dgvcc_b200.h"
 
 namespace dgvcc {
@@ -33,32 +36,45 @@ __device__ __forceinline__ float block_sum(float v, float* scratch) {
     return t;  // same value on every thread, fixed order
 }
 
+// Element access of the instance norm: fp32 as it is, fp16 / bf16 widened exactly on load and rounded to nearest on store.
+template <typename T> struct Elem {
+    static __device__ __forceinline__ float load(T v) { return dgvcc::tc::HalfIn<T>::widen(v); }
+    static __device__ __forceinline__ T store(float v) { return dgvcc::tc::HalfIn<T>::narrow(v); }
+};
+template <> struct Elem<float> {
+    static __device__ __forceinline__ float load(float v) { return v; }
+    static __device__ __forceinline__ float store(float v) { return v; }
+};
+
 // One CTA per (b, c) plane of HW elements: mean, biased variance (two-pass on the cached plane), normalise.
+// T = __half / __nv_bfloat16: the plane is cached in the input type (twice the plane fits) and y is written as RN(y).
+template <typename T>
 __global__ void __launch_bounds__(NORM_THREADS)
-isw_instnorm_fwd_kernel(const float* __restrict__ x, int hw, float eps, float* __restrict__ y,
+isw_instnorm_fwd_kernel(const T* __restrict__ x, int hw, float eps, T* __restrict__ y,
                         float* __restrict__ mean_out, float* __restrict__ invstd_out) {
-    extern __shared__ float plane[];  // hw floats when they fit, else unused
+    extern __shared__ float plane_f32[];  // hw elements when they fit, else unused
+    T* plane = reinterpret_cast<T*>(plane_f32);
     __shared__ float scratch[NORM_THREADS / 32];
     const size_t base = (size_t)blockIdx.x * hw;
     const bool cached = gridDim.y == 1;  // launch with gridDim.y == 2 to signal "does not fit in smem"
-    const float* src = x + base;
+    const T* src = x + base;
     float s = 0.f;
     for (int i = threadIdx.x; i < hw; i += NORM_THREADS) {
-        const float v = src[i];
+        const T v = src[i];
         if (cached) plane[i] = v;
-        s += v;
+        s += Elem<T>::load(v);
     }
     const float mean = block_sum(s, scratch) / (float)hw;
     float q = 0.f;
     for (int i = threadIdx.x; i < hw; i += NORM_THREADS) {
-        const float d = (cached ? plane[i] : src[i]) - mean;
+        const float d = Elem<T>::load(cached ? plane[i] : src[i]) - mean;
         q = fmaf(d, d, q);
     }
     const float var = block_sum(q, scratch) / (float)hw;
     const float invstd = 1.0f / sqrtf(var + eps);
     if (blockIdx.y == 0) {
         for (int i = threadIdx.x; i < hw; i += NORM_THREADS)
-            y[base + i] = ((cached ? plane[i] : src[i]) - mean) * invstd;
+            y[base + i] = Elem<T>::store((Elem<T>::load(cached ? plane[i] : src[i]) - mean) * invstd);
         if (threadIdx.x == 0) { mean_out[blockIdx.x] = mean; invstd_out[blockIdx.x] = invstd; }
     }
 }
@@ -80,6 +96,30 @@ isw_instnorm_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ 
     const float is = invstd[blockIdx.x];
     for (int i = threadIdx.x; i < hw; i += NORM_THREADS)
         dx[base + i] = is * (dy[base + i] - m1 - y[base + i] * m2);
+}
+
+// The same for a half-precision plane, from x, mean and invstd instead of a saved fp32 y: y is recomputed with the
+// forward's operations ((v - mean) * invstd: a sub and a mul, nothing to contract), so it is the forward's fp32 y bit for
+// bit; dx is written as RN(dx).
+template <typename T>
+__global__ void __launch_bounds__(NORM_THREADS)
+isw_instnorm_bwd_half_kernel(const T* __restrict__ dy, const T* __restrict__ x, const float* __restrict__ mean,
+                             const float* __restrict__ invstd, int hw, T* __restrict__ dx) {
+    __shared__ float scratch[NORM_THREADS / 32];
+    const size_t base = (size_t)blockIdx.x * hw;
+    const float mu = mean[blockIdx.x], is = invstd[blockIdx.x];
+    float s1 = 0.f, s2 = 0.f;
+    for (int i = threadIdx.x; i < hw; i += NORM_THREADS) {
+        const float g = Elem<T>::load(dy[base + i]);
+        s1 += g;
+        s2 = fmaf(g, __fmul_rn(__fsub_rn(Elem<T>::load(x[base + i]), mu), is), s2);
+    }
+    const float m1 = block_sum(s1, scratch) / (float)hw;
+    const float m2 = block_sum(s2, scratch) / (float)hw;
+    for (int i = threadIdx.x; i < hw; i += NORM_THREADS) {
+        const float yv = __fmul_rn(__fsub_rn(Elem<T>::load(x[base + i]), mu), is);
+        dx[base + i] = Elem<T>::store(is * (Elem<T>::load(dy[base + i]) - m1 - yv * m2));
+    }
 }
 
 // ------------------------------------------------------------------------------- SIMT Gram
@@ -566,22 +606,51 @@ isw_sx_simt_kernel(const float* __restrict__ s, const float* __restrict__ x, int
 using namespace dgvcc;
 using namespace dgvcc::isw;
 
-extern "C" int dgvcc_isw_instnorm_forward(const float* x, int planes, int hw, float eps, float* y, float* mean,
-                                          float* invstd, void* stream) {
-    DGVCC_DEVICE_GUARD(stream);
-    if (!x || !y || !mean || !invstd || planes <= 0 || hw <= 0) return DGVCC_ERR_ARG;
-    const size_t smem = (size_t)hw * sizeof(float);
+template <typename T>
+static int instnorm_forward(const T* x, int planes, int hw, float eps, T* y, float* mean, float* invstd, void* stream) {
+    const size_t smem = (size_t)hw * sizeof(T);
     const bool fits = smem <= 200 * 1024;
     if (fits && smem > 48 * 1024) {  // opt in once per device to the largest plane the kernel caches (not per call: the
                                      // call is not allowed while a stream is being captured into a CUDA graph)
         static PerDeviceOnce once;
         if (once.first())
-            DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_instnorm_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+            DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_instnorm_fwd_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                                       200 * 1024));
     }
     // gridDim.y == 2 tells the kernel the plane is not cached (only y-block 0 writes)
-    isw_instnorm_fwd_kernel<<<dim3(planes, fits ? 1 : 2), NORM_THREADS, fits ? smem : 0, (cudaStream_t)stream>>>(
+    isw_instnorm_fwd_kernel<T><<<dim3(planes, fits ? 1 : 2), NORM_THREADS, fits ? smem : 0, (cudaStream_t)stream>>>(
         x, hw, eps, y, mean, invstd);
+    return (int)cudaGetLastError();
+}
+
+extern "C" int dgvcc_isw_instnorm_forward(const float* x, int planes, int hw, float eps, float* y, float* mean,
+                                          float* invstd, void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    if (!x || !y || !mean || !invstd || planes <= 0 || hw <= 0) return DGVCC_ERR_ARG;
+    return instnorm_forward(x, planes, hw, eps, y, mean, invstd, stream);
+}
+
+static bool half_dtype(int dtype) { return dtype == DGVCC_DTYPE_F16 || dtype == DGVCC_DTYPE_BF16; }
+
+extern "C" int dgvcc_isw_instnorm_forward_h(const void* x, int dtype, int planes, int hw, float eps, void* y, float* mean,
+                                            float* invstd, void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    if (!x || !y || !mean || !invstd || planes <= 0 || hw <= 0 || !half_dtype(dtype)) return DGVCC_ERR_ARG;
+    if (dtype == DGVCC_DTYPE_F16)
+        return instnorm_forward((const __half*)x, planes, hw, eps, (__half*)y, mean, invstd, stream);
+    return instnorm_forward((const __nv_bfloat16*)x, planes, hw, eps, (__nv_bfloat16*)y, mean, invstd, stream);
+}
+
+extern "C" int dgvcc_isw_instnorm_backward_h(const void* dy, const void* x, const float* mean, const float* invstd, int dtype,
+                                             int planes, int hw, void* dx, void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    if (!dy || !x || !mean || !invstd || !dx || planes <= 0 || hw <= 0 || !half_dtype(dtype)) return DGVCC_ERR_ARG;
+    if (dtype == DGVCC_DTYPE_F16)
+        isw_instnorm_bwd_half_kernel<<<planes, NORM_THREADS, 0, (cudaStream_t)stream>>>(
+            (const __half*)dy, (const __half*)x, mean, invstd, hw, (__half*)dx);
+    else
+        isw_instnorm_bwd_half_kernel<<<planes, NORM_THREADS, 0, (cudaStream_t)stream>>>(
+            (const __nv_bfloat16*)dy, (const __nv_bfloat16*)x, mean, invstd, hw, (__nv_bfloat16*)dx);
     return (int)cudaGetLastError();
 }
 
@@ -666,6 +735,17 @@ IswWs carve(void* ws, int batch, int c, int hw) {
 extern "C" int dgvcc_isw_gram_tc_partials(const float* x, int batch, int c, int hw, int splits, int k_per_split,
                                           float* part, void* stream);
 
+namespace dgvcc { namespace isw_tc {
+int launch_half(const void* x, int dtype, int batch, int c, int hw, int splits, int k_per_split, float* part, void* stream);
+} }
+
+// The one shape rule of the half-precision Gram and dX = S X (isw_gram_tc.cu, isw_sx_tc.cu): TMA needs 16-byte row strides
+// (hw % 8 == 0) and 16-byte aligned bases; c >= 32 and c % 4 == 0 as for the fp32 dX = S X.  Other shapes return
+// DGVCC_ERR_UNSUPPORTED from every *_h Gram / dX entry point, forward and backward alike, and run upcast to fp32.
+static bool half_tc_tiles(const void* x, const void* out, int c, int hw) {
+    return hw % 8 == 0 && c % 4 == 0 && c >= 32 && !(((uintptr_t)x | (uintptr_t)out) & 15u);
+}
+
 // Gram of every sample on the tensor cores where the shape tiles (else exact fp32 on CUDA cores), finished as
 // out = X X^T / denom (+ eps * eye when eye is given).
 static int launch_gram(const float* f_map, const float* eye, float denom, float eps, int batch, int c, int hw,
@@ -698,6 +778,26 @@ extern "C" int dgvcc_isw_covariance(const float* f_map, const float* eye, int ba
     return launch_gram(f_map, eye, (float)(hw - 1), 1e-5f, batch, c, hw, use_tensor_cores, w, f_cor, (cudaStream_t)stream);
 }
 
+// The half-precision map: the tensor-core Gram only (the caller checked half_tc_tiles), same split plan and finish.
+extern "C" int dgvcc_isw_covariance_h(const void* f_map, int dtype, const float* eye, int batch, int c, int hw,
+                                      void* workspace, size_t workspace_bytes, float* f_cor, void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    if (!f_map || !eye || !workspace || !f_cor || !isw_shape_ok(batch, c, hw) || hw <= 1 || !half_dtype(dtype))
+        return DGVCC_ERR_ARG;
+    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
+    if (!half_tc_tiles(f_map, f_map, c, hw)) return DGVCC_ERR_UNSUPPORTED;
+    const IswWs w = carve(workspace, batch, c, hw);
+    cudaStream_t st = (cudaStream_t)stream;
+    int splits, kps, n_tiles, tile;
+    gram_plan_tc(batch, c, hw, &splits, &kps, &n_tiles, &tile);
+    const int rc = dgvcc::isw_tc::launch_half(f_map, dtype, batch, c, hw, splits, kps, w.part, (void*)st);
+    if (rc != DGVCC_OK) return rc;
+    const int yblocks = (tile / 32) * (tile / 32);
+    isw_cov_finish_kernel<<<dim3(n_tiles, yblocks, batch), 256, 0, st>>>(w.part, c, (float)(hw - 1), splits, tile, eye, 1e-5f,
+                                                                         f_cor);
+    return (int)cudaGetLastError();
+}
+
 extern "C" int dgvcc_isw_loss_forward(const float* f_cor, const float* mask, const float* margin,
                                       const float* num_remove_cov, int batch, int c, int hw, void* workspace,
                                       size_t workspace_bytes, float* loss_out, void* stream) {
@@ -717,6 +817,11 @@ extern "C" int dgvcc_isw_loss_forward(const float* f_cor, const float* mask, con
 namespace dgvcc { namespace isw_sx {
 int launch(const float* s, const float* x, int batch, int c, int hw, float* dx, const float* scale, bool a_is_tf32_exact,
            void* stream);
+} }
+
+namespace dgvcc { namespace isw_sx {
+int launch_half(const float* s, const void* x, int dtype, int batch, int c, int hw, void* dx, const float* scale,
+                bool a_is_tf32_exact, void* stream);
 } }
 
 // the shapes / alignments dgvcc::isw_sx::launch accepts
@@ -769,6 +874,41 @@ extern "C" int dgvcc_isw_covariance_backward(const float* f_map, const float* gr
     isw_cov_grad_kernel<<<dim3(ceil_div(c * c, 256), batch), 256, 0, st>>>(grad_f_cor, c, hw, w.s);
     DGVCC_RETURN_IF_CUDA(cudaGetLastError());
     return launch_sx(w.s, f_map, batch, c, hw, use_tensor_cores, grad_f_map, st);
+}
+
+extern "C" int dgvcc_isw_loss_backward_h(const void* f_map, int dtype, const float* f_cor, const float* mask,
+                                         const float* num_remove_cov, const float* grad_loss, int batch, int c, int hw,
+                                         int mask_is_binary, void* workspace, size_t workspace_bytes, void* grad_f_map,
+                                         void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    if (!f_map || !f_cor || !mask || !num_remove_cov || !grad_loss || !workspace || !grad_f_map ||
+        !isw_shape_ok(batch, c, hw) || !half_dtype(dtype))
+        return DGVCC_ERR_ARG;
+    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
+    if (!half_tc_tiles(f_map, grad_f_map, c, hw)) return DGVCC_ERR_UNSUPPORTED;
+    const IswWs w = carve(workspace, batch, c, hw);
+    cudaStream_t st = (cudaStream_t)stream;
+    // binary mask: factored S = alpha * T and the EXACT GEMM, as dgvcc_isw_loss_backward
+    isw_loss_grad_kernel<<<dim3(ceil_div(c, 32), ceil_div(c, 32), batch), 256, 0, st>>>(
+        f_cor, mask, w.off, num_remove_cov, grad_loss, c, hw, batch, w.s, mask_is_binary ? w.alpha : nullptr);
+    DGVCC_RETURN_IF_CUDA(cudaGetLastError());
+    return dgvcc::isw_sx::launch_half(w.s, f_map, dtype, batch, c, hw, grad_f_map, mask_is_binary ? w.alpha : nullptr,
+                                      mask_is_binary != 0, (void*)st);
+}
+
+extern "C" int dgvcc_isw_covariance_backward_h(const void* f_map, int dtype, const float* grad_f_cor, int batch, int c,
+                                               int hw, void* workspace, size_t workspace_bytes, void* grad_f_map,
+                                               void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    if (!f_map || !grad_f_cor || !workspace || !grad_f_map || !isw_shape_ok(batch, c, hw) || !half_dtype(dtype))
+        return DGVCC_ERR_ARG;
+    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
+    if (!half_tc_tiles(f_map, grad_f_map, c, hw)) return DGVCC_ERR_UNSUPPORTED;
+    const IswWs w = carve(workspace, batch, c, hw);
+    cudaStream_t st = (cudaStream_t)stream;
+    isw_cov_grad_kernel<<<dim3(ceil_div(c * c, 256), batch), 256, 0, st>>>(grad_f_cor, c, hw, w.s);
+    DGVCC_RETURN_IF_CUDA(cudaGetLastError());
+    return dgvcc::isw_sx::launch_half(w.s, f_map, dtype, batch, c, hw, grad_f_map, nullptr, false, (void*)st);
 }
 
 extern "C" int dgvcc_isw_covstat_var(const float* f_cor, const float* reverse_eye, int batch, int c, float* var_out,

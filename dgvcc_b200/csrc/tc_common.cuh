@@ -2,6 +2,8 @@
 // loads, UMMA issue / commit, TMEM loads, TF32 rounding, and the driver entry point for tensor maps.
 #pragma once
 #include <cuda.h>
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 
 #include "common.cuh"
 
@@ -116,19 +118,54 @@ inline EncodeTiledFn encode_tiled_fn() {
     return fn;
 }
 
+// 3-D tensor map {inner, rows, batch} of elem_bytes-wide elements with a {box_inner, box_rows, box_batch} box.
+inline bool make_tmap_3d(CUtensorMap* map, CUtensorMapDataType type, uint32_t elem_bytes, const void* base, uint64_t inner,
+                         uint64_t rows, uint64_t batch, uint32_t box_inner, uint32_t box_rows, CUtensorMapSwizzle swizzle,
+                         uint32_t box_batch) {
+    EncodeTiledFn enc = encode_tiled_fn();
+    if (!enc) return false;
+    const cuuint64_t dims[3] = {inner, rows, batch};
+    const cuuint64_t strides[2] = {inner * elem_bytes, inner * rows * elem_bytes};
+    const cuuint32_t box[3] = {box_inner, box_rows, box_batch};
+    const cuuint32_t estr[3] = {1, 1, 1};
+    return enc(map, type, 3, (void*)base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle,
+               CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
 // fp32 3-D tensor map {inner, rows, batch} with a {32 floats (one 128-byte swizzle row), box_rows, box_batch} box.
 inline bool make_tmap_f32_3d(CUtensorMap* map, const float* base, uint64_t inner, uint64_t rows, uint64_t batch,
                              uint32_t box_rows, CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B,
                              uint32_t box_batch = 1) {
-    EncodeTiledFn enc = encode_tiled_fn();
-    if (!enc) return false;
-    const cuuint64_t dims[3] = {inner, rows, batch};
-    const cuuint64_t strides[2] = {inner * 4, inner * rows * 4};
-    const cuuint32_t box[3] = {32, box_rows, box_batch};
-    const cuuint32_t estr[3] = {1, 1, 1};
-    return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, (void*)base, dims, strides, box, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+    return make_tmap_3d(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, base, inner, rows, batch, 32, box_rows, swizzle, box_batch);
+}
+
+// Half-precision input (fp16 / bf16) of the ISW tensor-core kernels.  Every finite value widens to fp32 exactly, with
+// zero low 13 mantissa bits: it IS its own TF32 hi part, and the lo part of the 3xTF32 split is exactly 0.
+template <typename T> struct HalfIn;
+template <> struct HalfIn<__half> {
+    static constexpr CUtensorMapDataType TMA = CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+    static __device__ __forceinline__ float widen(__half v) { return __half2float(v); }
+    static __device__ __forceinline__ __half narrow(float v) { return __float2half_rn(v); }
+};
+template <> struct HalfIn<__nv_bfloat16> {
+    static constexpr CUtensorMapDataType TMA = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    static __device__ __forceinline__ float widen(__nv_bfloat16 v) { return __bfloat162float(v); }
+    static __device__ __forceinline__ __nv_bfloat16 narrow(float v) { return __float2bfloat16_rn(v); }
+};
+
+// four consecutive half-precision elements (8 bytes) widened to a float4
+template <typename T>
+__device__ __forceinline__ float4 widen4(const T* p) {
+    const uint2 raw = *reinterpret_cast<const uint2*>(p);
+    const T* h = reinterpret_cast<const T*>(&raw);
+    return make_float4(HalfIn<T>::widen(h[0]), HalfIn<T>::widen(h[1]), HalfIn<T>::widen(h[2]), HalfIn<T>::widen(h[3]));
+}
+
+// four fp32 values rounded to nearest into four consecutive half-precision elements (one 8-byte store)
+template <typename T>
+__device__ __forceinline__ void narrow4(T* p, float a, float b, float c, float d) {
+    T h[4] = {HalfIn<T>::narrow(a), HalfIn<T>::narrow(b), HalfIn<T>::narrow(c), HalfIn<T>::narrow(d)};
+    *reinterpret_cast<uint2*>(p) = *reinterpret_cast<const uint2*>(h);
 }
 
 }  // namespace tc

@@ -11,6 +11,12 @@ The Gram X X^T is the only dense contraction of the path: csrc/isw_gram_tc.cu ru
 tcgen05 tensor cores (3xTF32 split, fp32 accumulation in TMEM) where the shape tiles, otherwise
 the exact-fp32 CUDA-core kernel of csrc/isw_kernels.cu.  ``margin`` / ``num_remove_cov`` may be
 Python numbers or 0-dim tensors, as in the reference (cov_settings.py:47,73).
+
+fp16 / bf16 feature maps (``torch.autocast`` training) run natively: the kernels read and write the half tensors, and
+autograd keeps the half map (plus the per-plane mean / invstd of the instance norm) instead of fp32 copies.  The
+results are those of the fp32 path on the upcast map, bit for bit: y and the gradients come back in the input dtype,
+``f_cor`` and the loss are fp32.  Shapes the half tensor-core kernels do not tile (HW % 8 != 0, C < 32, C % 4 != 0,
+a misaligned view) and ``DGVCC_ISW_TENSOR_CORES=0`` take the upcast route; the forward's choice holds for its backward.
 """
 import os
 
@@ -33,11 +39,27 @@ def _f32c(t, dev=None):
     return t.detach().to(device=dev if dev is not None else t.device, dtype=torch.float32).contiguous()
 
 
+_HALF = {torch.float16: _native.DTYPE_F16, torch.bfloat16: _native.DTYPE_BF16}
+
+
+def _half3d(f_map):
+    """(dtype code, contiguous half [B,C,HW] view) when ``f_map`` is fp16 / bf16 and the tensor cores are on, else
+    (None, None): the caller then takes the fp32 route of ``_as3d``."""
+    dt = _HALF.get(f_map.dtype)
+    if dt is None or not _use_tc():
+        return None, None
+    _native.require_cuda(f_map, "instance_whitening")
+    b, c, h, w = f_map.shape
+    return dt, f_map.detach().contiguous().view(b, c, h * w)
+
+
 def _as3d(f_map):
     _native.require_cuda(f_map, "instance_whitening")
     b, c, h, w = f_map.shape
     return _f32c(f_map).view(b, c, h * w), b, c, h * w
 
+
+_UNSUPPORTED = -3  # DGVCC_ERR_UNSUPPORTED
 
 _ws_bytes = {}
 
@@ -69,6 +91,17 @@ class _InstanceNorm(torch.autograd.Function):
     def forward(ctx, x, eps):
         _native.require_cuda(x, "InstanceWhitening")
         b, c, h, w = x.shape
+        ctx.half = _HALF.get(x.dtype)
+        if ctx.half is not None:  # y = RN(fp32 y) in the input dtype; the backward recomputes fp32 y from x
+            xc = x.detach().contiguous()
+            y = torch.empty_like(xc)
+            mean = torch.empty((b * c,), dtype=torch.float32, device=x.device)
+            invstd = torch.empty_like(mean)
+            _native.check(_native.lib().dgvcc_isw_instnorm_forward_h(
+                _native.ptr(xc), ctx.half, b * c, h * w, eps, _native.ptr(y), _native.ptr(mean), _native.ptr(invstd),
+                _native.stream_ptr(x.device)), "dgvcc_isw_instnorm_forward_h")
+            ctx.save_for_backward(xc, mean, invstd)
+            return y
         xc = _f32c(x)
         y = torch.empty_like(xc)
         mean = torch.empty((b * c,), dtype=torch.float32, device=x.device)
@@ -82,6 +115,15 @@ class _InstanceNorm(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, dy):
+        if ctx.half is not None:
+            xc, mean, invstd = ctx.saved_tensors
+            b, c, h, w = xc.shape
+            g = dy.contiguous()
+            dx = torch.empty_like(xc)
+            _native.check(_native.lib().dgvcc_isw_instnorm_backward_h(
+                _native.ptr(g), _native.ptr(xc), _native.ptr(mean), _native.ptr(invstd), ctx.half, b * c, h * w,
+                _native.ptr(dx), _native.stream_ptr(xc.device)), "dgvcc_isw_instnorm_backward_h")
+            return dx, None
         y, invstd = ctx.saved_tensors
         b, c, h, w = y.shape
         g = _f32c(dy)
@@ -108,6 +150,21 @@ class InstanceWhitening(nn.Module):
 class _Covariance(torch.autograd.Function):
     @staticmethod
     def forward(ctx, f_map, eye):
+        ctx.half, x = _half3d(f_map)
+        if ctx.half is not None:
+            b, c, hw = x.shape
+            dev = x.device
+            ws, n = _workspace(b, c, hw, dev)
+            f_cor = torch.empty((b, c, c), dtype=torch.float32, device=dev)
+            rc = _native.lib().dgvcc_isw_covariance_h(_native.ptr(x), ctx.half, _native.ptr(_f32c(eye, dev)), b, c, hw,
+                                                      _native.ptr(ws), n, _native.ptr(f_cor), _native.stream_ptr(dev))
+            if rc == _UNSUPPORTED:
+                ctx.half = None
+            else:
+                _native.check(rc, "dgvcc_isw_covariance_h")
+                ctx.save_for_backward(x)
+                ctx.meta = (f_map.shape, f_map.dtype)
+                return f_cor
         x, b, c, hw = _as3d(f_map)
         dev = x.device
         ws, n = _workspace(b, c, hw, dev)
@@ -128,6 +185,11 @@ class _Covariance(torch.autograd.Function):
         ws, n = _workspace(b, c, hw, dev)
         g = _f32c(d_fcor)
         dx = torch.empty_like(x)
+        if ctx.half is not None:
+            _native.check(_native.lib().dgvcc_isw_covariance_backward_h(
+                _native.ptr(x), ctx.half, _native.ptr(g), b, c, hw, _native.ptr(ws), n, _native.ptr(dx),
+                _native.stream_ptr(dev)), "dgvcc_isw_covariance_backward_h")
+            return dx.view(ctx.meta[0]), None
         _native.check(_native.lib().dgvcc_isw_covariance_backward(
             _native.ptr(x), _native.ptr(g), b, c, hw, _use_tc(), _native.ptr(ws), n, _native.ptr(dx),
             _native.stream_ptr(dev)), "dgvcc_isw_covariance_backward")
@@ -153,7 +215,11 @@ def _mask_is_binary(mask):
 class _WhiteningLoss(torch.autograd.Function):
     @staticmethod
     def forward(ctx, f_map, eye, mask_matrix, margin, num_remove_cov):
-        x, b, c, hw = _as3d(f_map)
+        ctx.half, x = _half3d(f_map)
+        if ctx.half is None:
+            x, b, c, hw = _as3d(f_map)
+        else:
+            b, c, hw = x.shape
         dev = x.device
         lib = _native.lib()
         ws, n = _workspace(b, c, hw, dev)
@@ -164,8 +230,17 @@ class _WhiteningLoss(torch.autograd.Function):
             raise ValueError(f"mask_matrix must be [{c},{c}], got {tuple(mask.shape)}")
         mg, nr = _scalar(margin, dev), _scalar(num_remove_cov, dev)
         stream = _native.stream_ptr(dev)
-        _native.check(lib.dgvcc_isw_covariance(_native.ptr(x), _native.ptr(eye32), b, c, hw, _use_tc(), _native.ptr(ws), n,
-                                               _native.ptr(f_cor), stream), "dgvcc_isw_covariance")
+        if ctx.half is not None:
+            rc = lib.dgvcc_isw_covariance_h(_native.ptr(x), ctx.half, _native.ptr(eye32), b, c, hw, _native.ptr(ws), n,
+                                            _native.ptr(f_cor), stream)
+            if rc == _UNSUPPORTED:  # a shape the half tensor-core kernels do not tile: upcast, as for every other dtype
+                ctx.half = None
+                x = _as3d(f_map)[0]
+            else:
+                _native.check(rc, "dgvcc_isw_covariance_h")
+        if ctx.half is None:
+            _native.check(lib.dgvcc_isw_covariance(_native.ptr(x), _native.ptr(eye32), b, c, hw, _use_tc(), _native.ptr(ws),
+                                                   n, _native.ptr(f_cor), stream), "dgvcc_isw_covariance")
         loss = torch.empty((1,), dtype=torch.float32, device=dev)
         _native.check(lib.dgvcc_isw_loss_forward(_native.ptr(f_cor), _native.ptr(mask), _native.ptr(mg), _native.ptr(nr),
                                                  b, c, hw, _native.ptr(ws), n, _native.ptr(loss), stream),
@@ -182,6 +257,11 @@ class _WhiteningLoss(torch.autograd.Function):
         dev = x.device
         g = _f32c(grad_loss, dev).reshape(1)
         dx = torch.empty_like(x)
+        if ctx.half is not None:
+            _native.check(_native.lib().dgvcc_isw_loss_backward_h(
+                _native.ptr(x), ctx.half, _native.ptr(f_cor), _native.ptr(mask), _native.ptr(nr), _native.ptr(g), b, c, hw,
+                int(binary), _native.ptr(ws), n, _native.ptr(dx), _native.stream_ptr(dev)), "dgvcc_isw_loss_backward_h")
+            return dx.view(shape), None, None, None, None
         _native.check(_native.lib().dgvcc_isw_loss_backward(
             _native.ptr(x), _native.ptr(f_cor), _native.ptr(mask), _native.ptr(nr), _native.ptr(g), b, c, hw, _use_tc(),
             int(binary), _native.ptr(ws), n, _native.ptr(dx), _native.stream_ptr(dev)), "dgvcc_isw_loss_backward")

@@ -25,6 +25,10 @@ extern "C" {
 #define DGVCC_ERR_WORKSPACE (-2)
 #define DGVCC_ERR_UNSUPPORTED (-3)
 
+/* Element type of the `const void*` feature maps of the *_h entry points. */
+#define DGVCC_DTYPE_F16 1
+#define DGVCC_DTYPE_BF16 2
+
 /* ABI version; bumped when a signature changes. */
 int dgvcc_abi_version(void);
 
@@ -424,6 +428,27 @@ int dgvcc_isw_covstat_var(const float* f_cor, const float* reverse_eye, int batc
  * index order (torch.topk leaves that open).  k = int(num_off_diagonal - margin) is the caller's (:63-65). */
 int dgvcc_isw_topk_mask(const float* stats, int n_stats, int count, int n, int k, const float* prev_mask,
                         float* values, float* mask, void* stream);
+
+/* Half-precision feature maps (autocast training): x, y, dy, dx, f_map and grad_f_map are fp16 or bf16 (dtype
+ * DGVCC_DTYPE_F16 / DGVCC_DTYPE_BF16, any other value is DGVCC_ERR_ARG); mean, invstd, eye, f_cor and the gradients
+ * of f_cor / the loss stay fp32.  Every output is what the fp32 entry points above compute on the map upcast to fp32,
+ * rounded to nearest where it is half precision.  The loss forward, the workspace size and the covstat kernel are
+ * shared with the fp32 path (they read the fp32 f_cor).
+ * The instance norm takes any shape; its backward recomputes y from x, mean and invstd (no saved fp32 y).
+ * The Gram and dX = S X run on the tensor cores only: for hw % 8 != 0, c < 32, c % 4 != 0 or a feature-map pointer
+ * that is not 16-byte aligned they return DGVCC_ERR_UNSUPPORTED (forward and backward alike), and the caller upcasts. */
+int dgvcc_isw_instnorm_forward_h(const void* x, int dtype, int planes, int hw, float eps, void* y, float* mean,
+                                 float* invstd, void* stream);
+int dgvcc_isw_instnorm_backward_h(const void* dy, const void* x, const float* mean, const float* invstd, int dtype,
+                                  int planes, int hw, void* dx, void* stream);
+int dgvcc_isw_covariance_h(const void* f_map, int dtype, const float* eye, int batch, int c, int hw, void* workspace,
+                           size_t workspace_bytes, float* f_cor, void* stream);
+int dgvcc_isw_covariance_backward_h(const void* f_map, int dtype, const float* grad_f_cor, int batch, int c, int hw,
+                                    void* workspace, size_t workspace_bytes, void* grad_f_map, void* stream);
+int dgvcc_isw_loss_backward_h(const void* f_map, int dtype, const float* f_cor, const float* mask,
+                              const float* num_remove_cov, const float* grad_loss, int batch, int c, int hw,
+                              int mask_is_binary, void* workspace, size_t workspace_bytes, void* grad_f_map,
+                              void* stream);
 
 /* The tensor-core Gram on its own (split-K partial tiles, tests / profiling):
  * part [batch][splits][upper-triangular 128x128 tiles][128][128]. */
