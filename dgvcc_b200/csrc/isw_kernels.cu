@@ -606,11 +606,16 @@ isw_sx_simt_kernel(const float* __restrict__ s, const float* __restrict__ x, int
 using namespace dgvcc;
 using namespace dgvcc::isw;
 
+// Dynamic shared memory a launch of isw_instnorm_fwd_kernel gets without the opt-in.  The kernel's static shared memory
+// (its scratch, plus the 1 KB the runtime reserves per block: 1056 bytes in `cuobjdump -res-usage`) counts against the
+// same 48 KB, so a 48 KB plane needs the opt-in too; 2 KB of slack keeps the rule clear of the static size.
+constexpr size_t NORM_SMEM_NO_OPT_IN = 48 * 1024 - 2048;
+
 template <typename T>
 static int instnorm_forward(const T* x, int planes, int hw, float eps, T* y, float* mean, float* invstd, void* stream) {
     const size_t smem = (size_t)hw * sizeof(T);
     const bool fits = smem <= 200 * 1024;
-    if (fits && smem > 48 * 1024) {  // opt in once per device to the largest plane the kernel caches (not per call: the
+    if (fits && smem > NORM_SMEM_NO_OPT_IN) {  // opt in once per device to the largest plane the kernel caches (not per call: the
                                      // call is not allowed while a stream is being captured into a CUDA graph)
         static PerDeviceOnce once;
         if (once.first())
