@@ -52,20 +52,51 @@ def _to_device(array, dev):
     return host.to(dev, non_blocking=True)
 
 
-def _check_points(points, height, width):
+def _as_points(points):
     pts = np.ascontiguousarray(np.asarray(points), dtype=np.float64)  # KDTree(points.copy()) works in float64
     if pts.ndim != 2 or pts.shape[1] != 2:
         raise ValueError(f"points must be [N,2], got {pts.shape}")
-    # the reference writes pt2d[int(y), int(x)]: numpy raises IndexError below -size
-    if len(pts) and (np.trunc(pts[:, 1]).min() < -height or np.trunc(pts[:, 0]).min() < -width):
-        raise IndexError("point index out of bounds for the image (negative beyond its size)")
+    return pts
+
+
+def _require_finite(pts):
+    """The adaptive reference builds KDTree(points) before anything else, and KDTree raises ValueError on NaN / inf.
+    The kernels would turn such a head into pixel 0 ((int)NaN) and a NaN sigma into the identity filter."""
+    if not np.isfinite(pts).all():
+        bad = int(np.argmin(np.isfinite(pts).all(axis=1)))
+        raise ValueError(f"points must be finite, head {bad} is {tuple(pts[bad])}")
+
+
+def _check_points(points, height, width, adaptive):
+    pts = _as_points(points)
+    if adaptive:
+        _require_finite(pts)
+    # the reference's per-head loop (dmap_gen.py:41-42): `int(y) < height and int(x) < width` (int() of NaN raises
+    # ValueError, of +-inf OverflowError; x is not converted when y is already out of range), then pt2d[int(y), int(x)]
+    # (numpy raises IndexError below -size).  The first head that raises decides, in index order.
+    fin = np.isfinite(pts)
+    ty, tx = np.trunc(pts[:, 1]), np.trunc(pts[:, 0])
+    with np.errstate(invalid="ignore"):
+        y_bad = ~fin[:, 1]
+        x_bad = ~y_bad & (ty < height) & ~fin[:, 0]
+        neg = fin.all(axis=1) & (ty < height) & (tx < width) & ((ty < -height) | (tx < -width))
+    fails = y_bad | x_bad | neg
+    if fails.any():
+        i = int(np.argmax(fails))
+        if neg[i]:
+            raise IndexError(f"head {i} {tuple(pts[i])}: index out of bounds for the image (negative beyond its size)")
+        v = pts[i, 1] if y_bad[i] else pts[i, 0]
+        if np.isnan(v):
+            raise ValueError(f"head {i} {tuple(pts[i])}: cannot convert float NaN to integer")
+        raise OverflowError(f"head {i} {tuple(pts[i])}: cannot convert float infinity to integer")
     return pts
 
 
 def knn_sigma(points, device=None):
     """(distances [N,4] f64, locations [N,4] i64, sigma [N] f64) of dmap_gen.py:34-36,45-48, as host arrays."""
-    dev = _device(device)
     pts = np.ascontiguousarray(np.asarray(points), dtype=np.float64)
+    _require_finite(pts)
+    dev = _device(device)
     n = len(pts)
     if n == 0:
         return np.zeros((0, 4)), np.zeros((0, 4), dtype=np.int64), np.zeros((0,))
@@ -144,8 +175,8 @@ def _density(img, points, adaptive, device=None):
     height, width = int(img.shape[0]), int(img.shape[1])
     if len(points) == 0:  # dmap_gen.py:28-29
         return np.zeros((height, width), dtype=np.float32)
+    pts = _check_points(points, height, width, adaptive)
     dev = _device(device)
-    pts = _check_points(points, height, width)
     host = _pinned((height, width), torch.float32)
     host.copy_(_density_device(height, width, pts, adaptive, dev), non_blocking=True)
     torch.cuda.current_stream(dev).synchronize()
@@ -165,11 +196,12 @@ def gaussian_filter_density_fixed(img, points, device=None):
 def gaussian_filter_density_batch(shapes, points_list, fixed=False, device=None):
     """A list of images through ONE set of launches (kNN, prepare, two culling passes, splat), one packed
     device-to-host copy and one synchronisation; returns a list of [H,W] float32 arrays (views of one buffer)."""
-    dev = _device(device)
     shapes = [(int(h), int(w)) for h, w in shapes]
     if not shapes:
         return []
-    pts = [_check_points(p, h, w) if len(p) else np.zeros((0, 2)) for (h, w), p in zip(shapes, points_list)]
+    # every image is checked (in the caller's order, like one reference call per image) before anything is launched
+    pts = [_check_points(p, h, w, not fixed) if len(p) else np.zeros((0, 2)) for (h, w), p in zip(shapes, points_list)]
+    dev = _device(device)
     out, offsets = _density_batch_device(shapes, pts, not fixed, dev)
     host = _pinned(out.shape, torch.float32)
     host.copy_(out, non_blocking=True)

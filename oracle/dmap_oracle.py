@@ -26,10 +26,11 @@ def knn4(points):
 
 
 def adaptive_sigmas(points):
-    """sigma per point, dmap_gen.py:45-48: 0.1 * (d1 + d2 + d3) when there are more than 3 points, else 15."""
+    """sigma per point, dmap_gen.py:45-48: 0.1 * (d1 + d2 + d3) when there are more than 3 points, else 15.
+    The tree is built for any number of points (dmap_gen.py:34-36), so NaN / inf heads raise ValueError here."""
     n = len(points)
+    d, _ = knn4(points)
     if n > 3:
-        d, _ = knn4(points)
         return (d[:, 1] + d[:, 2] + d[:, 3]) * 0.1
     return np.full((n,), 15.0)
 
@@ -71,14 +72,16 @@ def kernel1d(sigma, truncate):
     return phi / phi.sum(), radius
 
 
-def density_closed_form(shape, points, fixed=False, sigmas=None):
+def density_closed_form(shape, points, fixed=False, sigmas=None, truncate=None):
+    """``truncate``: scipy's, 7/4 (fixed) or 4 (adaptive) by default."""
     h, w = shape
     density = np.zeros(shape, dtype=np.float32)
     if len(points) == 0:
         return density
     if sigmas is None:
         sigmas = np.full(len(points), 4.0) if fixed else adaptive_sigmas(points)
-    truncate = 7 / 4 if fixed else 4.0
+    if truncate is None:
+        truncate = 7 / 4 if fixed else 4.0
     for i, pt in enumerate(points):
         iy, ix = int(pt[1]), int(pt[0])
         if not (iy < h and ix < w):

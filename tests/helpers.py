@@ -80,3 +80,13 @@ def load_sw_cases():
             c["ref"] = [{k[len(p):]: z[k] for k in z.files if k.startswith(p)} for p in prefix]
             cases[name] = c
     return cases
+
+
+def assert_map_close(got, ref, what):
+    """Density-map gate (SURVEY.md section 8d): rtol 1e-5 with atol 1e-7*max|ref|; returns the number of pixels that are
+    not bit-identical."""
+    assert got.dtype == np.float32 and got.shape == ref.shape
+    tol = 1e-5 * np.abs(ref) + 1e-7 * float(np.abs(ref).max() if ref.size else 0)
+    bad = np.abs(got.astype(np.float64) - ref) > tol
+    assert not bad.any(), f"{what}: {int(bad.sum())} pixels out of tolerance, max err {np.abs(got - ref).max()}"
+    return int((got != ref).sum())

@@ -11,7 +11,7 @@ import pytest
 
 from dgvcc_b200 import synthetic
 from oracle import dmap_oracle
-from helpers import GOLDEN
+from helpers import GOLDEN, assert_map_close
 
 pytestmark = pytest.mark.gpu
 
@@ -21,14 +21,6 @@ CASES = ["a40", "a4", "a3", "a1", "a0", "a25f32", "oob", "dup"]
 @pytest.fixture(scope="module")
 def fixtures():
     return np.load(os.path.join(GOLDEN, "dmap_cases.npz"))
-
-
-def assert_map_close(got, ref, what):
-    assert got.dtype == np.float32 and got.shape == ref.shape
-    tol = 1e-5 * np.abs(ref) + 1e-7 * float(np.abs(ref).max() if ref.size else 0)
-    bad = np.abs(got.astype(np.float64) - ref) > tol
-    assert not bad.any(), f"{what}: {int(bad.sum())} pixels out of tolerance, max err {np.abs(got - ref).max()}"
-    return int((got != ref).sum())
 
 
 @pytest.mark.parametrize("name", CASES)
