@@ -157,6 +157,7 @@ SIGNATURES = {
                                                                                    c_void_p]),
     "dgvcc_probe_ex2": (c_int, [c_void_p, c_int, POINTER(c_int64), c_void_p]),
     "dgvcc_probe_ffma": (c_int, [c_void_p, c_int, POINTER(c_int64), c_void_p]),
+    "dgvcc_probe_ex2_fma": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     "dgvcc_probe_tf32": (c_int, [c_void_p, c_int, POINTER(c_int64), c_void_p]),
 }
 

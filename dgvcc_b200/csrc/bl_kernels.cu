@@ -28,8 +28,8 @@
 // reference's fp32 sequence bit for bit -- no FMA contraction in the distance expansion
 // (explicit _rn intrinsics), IEEE sqrt, IEEE division by 2*sigma^2 (exact scaling when it is
 // a power of two, otherwise a Markstein-corrected reciprocal multiply that is correctly
-// rounded).  Only exp (one MUFU.EX2 fed by one fused multiply-add, see pair_exp) and the summation order
-// differ, ~1e-6.
+// rounded).  Only exp (one MUFU.EX2, or ex2_fma for an eighth of the pixels, fed by one fused multiply-add, see pair_exp)
+// and the summation order differ, ~1e-6.
 #include <stdlib.h>
 #include <string.h>
 
@@ -64,6 +64,20 @@ struct Geom {
     float half;        // stride / 2
 };
 
+// Which exponentials leave MUFU.EX2, the sweeps' bottleneck, for the FMA pipe (ex2_fma): those of the pixels on global
+// grid rows 6, 7 (mod 8) in odd 32-column blocks, an eighth.  A quarter (every column) was slower: FFMA2 takes the FMA
+// pipe for two cycles, so 17 issue slots per converted pair left the sweeps co-bound on both pipes.  The rule belongs
+// to the pixel, not to the tile, so every pixel tile shape -- one GPU, the sharded layouts, exact_cull -- and Z, the
+// counts, the gradient and the posteriors compute the same bits for a (point, pixel) pair.  Rows 2q, 2q + 1 and column
+// col0 + 32c of a tile starting at row_base:
+template <int R, int C>
+__device__ __forceinline__ bool fma_pair(int row_base, int col0, int q, int c) {
+    const bool rows67 = R % 8 == 0 ? q % 4 == 3 : ((row_base + 2 * q) & 7) == 6;   // row_base is a multiple of R
+    const bool odd = C == 2 ? c == 1 : ((col0 >> 5) & 1) != 0;                      // col0 = 32 * C * block + lane
+    return rows67 && odd;   // compile-time for the 8x2 tile, warp-uniform otherwise
+}
+__device__ __forceinline__ bool fma_pixel(int row, int col) { return (row & 7) >= 6 && ((col >> 5) & 1); }
+
 // -dis / s, rounded exactly like the reference's true division.
 template <bool POW2>
 __device__ __forceinline__ float neg_div(float dis, const Scale& k) {
@@ -80,20 +94,12 @@ __device__ __forceinline__ float neg_div(float dis, const Scale& k) {
 // slope) moves every exponent of one pixel by the same amount, which cancels in e / sum(e); what is left
 // is |t| * 2^-23 per term, the same size as rounding (a - amax) and its product with log2e separately.
 // The kernels are instruction-issue bound next to MUFU, so one instruction fewer per pair is ~5 %.
+// on_fma (see fma_pair): 2^t from ex2_fma1, the same bits as a lane of the sweeps' packed ex2_fma.
 template <bool POW2>
-__device__ __forceinline__ float pair_exp(float dis, float k2, const Scale& k) {
-    if (POW2) return ex2_ftz(__fmaf_rn(dis, k.k1, k2));
-    return ex2_ftz(__fmaf_rn(neg_div<false>(dis, k), LOG2E, k2));
+__device__ __forceinline__ float pair_exp(float dis, float k2, const Scale& k, bool on_fma) {
+    const float t = POW2 ? __fmaf_rn(dis, k.k1, k2) : __fmaf_rn(neg_div<false>(dis, k), LOG2E, k2);
+    return on_fma ? ex2_fma1(t) : ex2_ftz(t);
 }
-
-// Two fp32 values in one 64-bit register: Blackwell's packed add/mul/fma.f32x2 (SASS FADD2 / FMUL2 / FFMA2)
-// do the work of two scalar instructions in one issue slot; each lane is an ordinary IEEE round-to-nearest op.
-typedef unsigned long long f2;
-__device__ __forceinline__ f2 pack2(float lo, float hi) { f2 r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi)); return r; }
-__device__ __forceinline__ void unpack2(f2 v, float& lo, float& hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v)); }
-__device__ __forceinline__ f2 add2(f2 a, f2 b) { f2 r; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b)); return r; }
-__device__ __forceinline__ f2 mul2(f2 a, f2 b) { f2 r; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b)); return r; }
-__device__ __forceinline__ f2 fma2(f2 a, f2 b, f2 c) { f2 r; asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c)); return r; }
 
 // Broadcast copies of the Scale constants for the packed path.
 struct Scale2 {
@@ -102,9 +108,9 @@ struct Scale2 {
         : k1(pack2(k.k1, k.k1)), neg_s(pack2(-k.s, -k.s)), r(pack2(k.r, k.r)), neg_l(pack2(-LOG2E, -LOG2E)) {}
 };
 
-// pair_exp for two pixels at once (same arithmetic per lane as the scalar version).
+// pair_exp for two pixels at once (same arithmetic per lane as the scalar version); on_fma: see fma_pair.
 template <bool POW2>
-__device__ __forceinline__ f2 pair_exp2(f2 dis, f2 k2, const Scale2& k) {
+__device__ __forceinline__ f2 pair_exp2(f2 dis, f2 k2, const Scale2& k, bool on_fma) {
     f2 t;
     if (POW2) {
         t = fma2(dis, k.k1, k2);
@@ -114,6 +120,7 @@ __device__ __forceinline__ f2 pair_exp2(f2 dis, f2 k2, const Scale2& k) {
         const f2 rem = fma2(q, k.neg_s, dis);
         t = fma2(fma2(rem, k.r, q), k.neg_l, k2);
     }
+    if (on_fma) return ex2_fma(t);
     float t0, t1;
     unpack2(t, t0, t1);
     return pack2(ex2_ftz(t0), ex2_ftz(t1));
@@ -518,7 +525,8 @@ __device__ __forceinline__ float tile_max(const float (&v)[R][C]) {
 }
 
 // Exact-zero culling of the exponential sweeps (opt-in): exp(a - amax) is computed as one MUFU.EX2 with
-// flush-to-zero, so it is exactly +0 whenever (a - amax) * log2(e) < -126.  With a <= -lb/s for every pixel
+// flush-to-zero (or by ex2_fma, which has the same zero set), so it is exactly +0 whenever (a - amax) * log2(e) < -126.
+// With a <= -lb/s for every pixel
 // of the tile and amax >= the tile's smallest amax, a point is skipped when that bound is below -128 --
 // every term it would have contributed is an exact zero, and the results are bit-identical.
 struct ExpCull {
@@ -987,7 +995,8 @@ __device__ __forceinline__ bool bl_z_body(const float2* __restrict__ pts_all, co
                 const float xd = axis_sqdist(xs.x, xs.y, px.cxm2[c], px.cxx[c]);
                 const f2 xd2 = pack2(xd, xd);
 #pragma unroll
-                for (int q = 0; q < R / 2; ++q) zp[q][c] = add2(zp[q][c], pair_exp2<POW2>(add2(yd[q], xd2), k2p[q][c], k2s));
+                for (int q = 0; q < R / 2; ++q)
+                    zp[q][c] = add2(zp[q][c], pair_exp2<POW2>(add2(yd[q], xd2), k2p[q][c], k2s, fma_pair<R, C>(px.row_base, px.col0, q, c)));
             }
         }
     }
@@ -1185,7 +1194,7 @@ bl_counts_kernel(const float2* __restrict__ pts_all, const int32_t* __restrict__
                         const f2 xd2 = pack2(xd, xd);
 #pragma unroll
                         for (int q = 0; q < R / 2; ++q)
-                            s2 = fma2(pair_exp2<POW2>(add2(yd[q], xd2), k2p[q][c], k2s), wdp[q][c], s2);
+                            s2 = fma2(pair_exp2<POW2>(add2(yd[q], xd2), k2p[q][c], k2s, fma_pair<R, C>(px.row_base, px.col0, q, c)), wdp[q][c], s2);
                     }
                     float s_even, s_odd;
                     unpack2(s2, s_even, s_odd);
@@ -1517,7 +1526,7 @@ __device__ __forceinline__ bool bl_grad_body(const float2* __restrict__ pts_all,
                 const f2 xd2 = pack2(xd, xd);
 #pragma unroll
                 for (int q = 0; q < R / 2; ++q)
-                    accp[q][c] = fma2(pair_exp2<POW2>(add2(yd[q], xd2), k2p[q][c], k2s), w2, accp[q][c]);
+                    accp[q][c] = fma2(pair_exp2<POW2>(add2(yd[q], xd2), k2p[q][c], k2s, fma_pair<R, C>(px.row_base, px.col0, q, c)), w2, accp[q][c]);
             }
         }
     }
@@ -1704,7 +1713,7 @@ bl_posterior_kernel(const float2* __restrict__ pts_all, const int32_t* __restric
                 const float xd = axis_sqdist(xs.x, xs.y, px.cxm2[c], px.cxx[c]);
 #pragma unroll
                 for (int r = 0; r < R; ++r) {
-                    const float p = pair_exp<POW2>(__fadd_rn(yd[r], xd), neg_amax[r][c], k) * rz[r][c];
+                    const float p = pair_exp<POW2>(__fadd_rn(yd[r], xd), neg_amax[r][c], k, fma_pixel(px.row_base + r, px.col0 + 32 * c)) * rz[r][c];
                     if (px.ok(r, c)) prob[(size_t)(n0 + i) * M + px.pix(r, c)] = p;
                 }
             }

@@ -79,6 +79,74 @@ __device__ __forceinline__ float ex2_ftz(float x) {
     return y;
 }
 
+// Two fp32 values in one 64-bit register: Blackwell's packed add/mul/fma.f32x2 (SASS FADD2 / FMUL2 / FFMA2)
+// do the work of two scalar instructions in one issue slot; each lane is an ordinary IEEE round-to-nearest op.
+typedef unsigned long long f2;
+__device__ __forceinline__ f2 pack2(float lo, float hi) { f2 r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi)); return r; }
+__device__ __forceinline__ void unpack2(f2 v, float& lo, float& hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v)); }
+__device__ __forceinline__ f2 add2(f2 a, f2 b) { f2 r; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b)); return r; }
+__device__ __forceinline__ f2 mul2(f2 a, f2 b) { f2 r; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b)); return r; }
+__device__ __forceinline__ f2 fma2(f2 a, f2 b, f2 c) { f2 r; asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c)); return r; }
+
+// t clamped to [-127, 128]; NaN stays NaN (max.NaN / min.NaN, where fmaxf / fminf would return the bound).
+__device__ __forceinline__ float ex2_fma_clamp(float t) {
+    float r;
+    asm("max.NaN.f32 %0, %1, 0fC2FE0000;\n\tmin.NaN.f32 %0, %0, 0f43000000;" : "=f"(r) : "f"(t));
+    return r;
+}
+
+// 2^t for both lanes on the FMA and ALU pipes only, a stand-in for ex2_ftz wherever MUFU is the bottleneck.
+// t = n + f with n = RN(t) (the 1.5 * 2^23 trick: no F2I, which would share MUFU's pipe) and f in [-0.5, 0.5];
+// 2^f is a degree-6 polynomial with p(0) = 1 (relative minimax, error 3.9e-9, fp32 coefficients), evaluated by Horner
+// in FFMA2; 2^n is built in the exponent field and applied by one flush-to-zero multiply.  Like ex2.approx.ftz.f32:
+//   * the result is +0 exactly for t < -126: n = -127 gives the factor +0, and n = -126 with f < 0 gives a subnormal
+//     that the multiply flushes -- the zero set ExpCull relies on;
+//   * NaN gives NaN, -inf gives +0, +inf gives +inf, 2^n is exact for integer t;
+//   * max relative error over every fp32 t in [-126, 0] is 7.8e-8 (MUFU.EX2: 1.4e-7), see profiles/r3_bl_fma_exp.md.
+// For t > 127.5 it returns +inf where MUFU still returns a finite value; exponents of the loss are <= 2^-8.
+__device__ __forceinline__ f2 ex2_fma(f2 t) {
+    float t0, t1;
+    unpack2(t, t0, t1);
+    const f2 tc = pack2(ex2_fma_clamp(t0), ex2_fma_clamp(t1));
+    const f2 fi = add2(tc, pack2(12582912.f, 12582912.f));   // n in the low mantissa bits
+    const f2 n = add2(fi, pack2(-12582912.f, -12582912.f));  // exact
+    const f2 f = fma2(n, pack2(-1.f, -1.f), tc);              // exact
+    f2 p = pack2(1.54697322e-4f, 1.54697322e-4f);
+    p = fma2(p, f, pack2(1.34100008e-3f, 1.34100008e-3f));
+    p = fma2(p, f, pack2(9.61803086e-3f, 9.61803086e-3f));
+    p = fma2(p, f, pack2(5.55029735e-2f, 5.55029735e-2f));
+    p = fma2(p, f, pack2(2.40226507e-1f, 2.40226507e-1f));
+    p = fma2(p, f, pack2(6.93147242e-1f, 6.93147242e-1f));
+    p = fma2(p, f, pack2(1.f, 1.f));
+    float fi0, fi1;
+    unpack2(fi, fi0, fi1);
+    // (n + 127) << 23: the low bits of fi hold n in two's complement; n = 128 gives +inf, n = -127 gives +0
+    const f2 s = pack2(__int_as_float((__float_as_int(fi0) << 23) + 0x3f800000),
+                       __int_as_float((__float_as_int(fi1) << 23) + 0x3f800000));
+    f2 r;
+    asm("mul.rn.ftz.f32x2 %0, %1, %2;" : "=l"(r) : "l"(p), "l"(s));
+    return r;
+}
+
+// ex2_fma on one lane with the same operations (fma.rn / add.rn / mul.rn.ftz are IEEE per lane)
+__device__ __forceinline__ float ex2_fma1(float t) {
+    const float tc = ex2_fma_clamp(t);
+    const float fi = __fadd_rn(tc, 12582912.f);
+    const float n = __fadd_rn(fi, -12582912.f);
+    const float f = __fmaf_rn(n, -1.f, tc);
+    float p = 1.54697322e-4f;
+    p = __fmaf_rn(p, f, 1.34100008e-3f);
+    p = __fmaf_rn(p, f, 9.61803086e-3f);
+    p = __fmaf_rn(p, f, 5.55029735e-2f);
+    p = __fmaf_rn(p, f, 2.40226507e-1f);
+    p = __fmaf_rn(p, f, 6.93147242e-1f);
+    p = __fmaf_rn(p, f, 1.f);
+    const float s = __int_as_float((__float_as_int(fi) << 23) + 0x3f800000);
+    float r;
+    asm("mul.rn.ftz.f32 %0, %1, %2;" : "=f"(r) : "f"(p), "f"(s));
+    return r;
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(FULL_MASK, v, o);

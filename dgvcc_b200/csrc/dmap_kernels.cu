@@ -353,14 +353,6 @@ dmap_knn_prep_kernel(const double2* __restrict__ pts, const int64_t* __restrict_
     if ((threadIdx.x & 31) == __ffs(peers) - 1 && warp_max > img_max_bits[img]) atomicMax(img_max_bits + img, warp_max);
 }
 
-// Two fp32 values in one 64-bit register for Blackwell's packed add / mul / fma.f32x2 (SASS FADD2 / FMUL2 / FFMA2).
-typedef unsigned long long f2;
-__device__ __forceinline__ f2 pack2(float lo, float hi) { f2 r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi)); return r; }
-__device__ __forceinline__ void unpack2(f2 v, float& lo, float& hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v)); }
-__device__ __forceinline__ f2 add2(f2 a, f2 b) { f2 r; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b)); return r; }
-__device__ __forceinline__ f2 mul2(f2 a, f2 b) { f2 r; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b)); return r; }
-__device__ __forceinline__ f2 fma2(f2 a, f2 b, f2 c) { f2 r; asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c)); return r; }
-
 // Upper bound, in fp32, of what the fp32 evaluation of a squared distance can return when the exact fp64 value is
 // below `thr`.  With u = 2^-24, M >= every |coordinate| of the image and d2 the exact value, the fp32 result is within
 //     E(d2) <= 5.7 u M sqrt(d2) + 4.2 u d2 + 16 u^2 M^2

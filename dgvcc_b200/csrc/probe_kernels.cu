@@ -93,6 +93,23 @@ __global__ void __launch_bounds__(128, 1) probe_tf32_kernel(float* sink, int ite
     }
 }
 
+// ex2.approx.ftz.f32 and ex2_fma of every t[i]; ex2_fma takes the values two at a time, like the sweeps' row pairs.
+__global__ void __launch_bounds__(256) probe_ex2_fma_kernel(const float* __restrict__ t, int n, float* __restrict__ mufu,
+                                                            float* __restrict__ fma) {
+    const int64_t i = 2 * ((int64_t)blockIdx.x * blockDim.x + threadIdx.x);
+    if (i >= n) return;
+    const bool pair = i + 1 < n;
+    const float t0 = t[i], t1 = pair ? t[i + 1] : t0;
+    float e0, e1;
+    unpack2(ex2_fma(pack2(t0, t1)), e0, e1);
+    mufu[i] = ex2_ftz(t0);
+    fma[i] = e0;
+    if (pair) {
+        mufu[i + 1] = ex2_ftz(t1);
+        fma[i + 1] = e1;
+    }
+}
+
 static int probe_grid() {
     int dev = 0, sms = 148;
     if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -116,6 +133,14 @@ extern "C" int dgvcc_probe_ffma(float* sink, int iters, int64_t* ops_out, void* 
     const int grid = dgvcc::probe_grid();
     dgvcc::probe_ffma_kernel<<<grid, dgvcc::PROBE_THREADS, 0, (cudaStream_t)stream>>>(sink, iters);
     if (ops_out) *ops_out = (int64_t)grid * dgvcc::PROBE_THREADS * dgvcc::PROBE_CHAINS * iters;
+    return (int)cudaGetLastError();
+}
+
+extern "C" int dgvcc_probe_ex2_fma(const float* t, int n, float* mufu_out, float* fma_out, void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    if (!t || !mufu_out || !fma_out || n <= 0) return DGVCC_ERR_ARG;
+    const int grid = (int)(((int64_t)n + 511) / 512);
+    dgvcc::probe_ex2_fma_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(t, n, mufu_out, fma_out);
     return (int)cudaGetLastError();
 }
 

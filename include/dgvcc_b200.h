@@ -482,6 +482,10 @@ int dgvcc_bay_crop_targets(const void* gt_xy, const void* dists, int n, int is_d
  * ------------------------------------------------------------------------- */
 int dgvcc_probe_ex2(float* sink, int iters, int64_t* ops_out, void* stream);
 int dgvcc_probe_ffma(float* sink, int iters, int64_t* ops_out, void* stream);
+/* mufu_out[i] = ex2.approx.ftz.f32(t[i]) and fma_out[i] = 2^t[i] from the FMA-pipe exponential that the Bayesian-loss
+ * sweeps use for an eighth of their pixels (ex2_fma, csrc/common.cuh), for i < n (device arrays): the accuracy check of
+ * that function against MUFU.EX2. */
+int dgvcc_probe_ex2_fma(const float* t, int n, float* mufu_out, float* fma_out, void* stream);
 /* Tensor-pipe probe: every SM issues `iters` x 4 back-to-back tcgen05.mma.kind::tf32 (M=128, N=256, K=8, operands
  * in shared memory, accumulators in TMEM); *flops_out = TF32 flops executed.  The Gram's roofline denominator
  * (SURVEY.md 8d: "Tensor peak for TF32 must also be measured on the box"). */
