@@ -138,6 +138,17 @@ SIGNATURES = {
     "dgvcc_ortho_loss_forward": (c_int, [c_void_p, c_int, c_int, c_void_p, c_size_t, c_void_p, c_void_p]),
     "dgvcc_ortho_loss_backward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_size_t,
                                           c_void_p, c_void_p, c_void_p]),
+    "dgvcc_isw_gram_h": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_size_t, c_void_p, c_void_p]),
+    "dgvcc_ortho_loss_backward_h": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p, c_size_t,
+                                            c_void_p, c_void_p, c_void_p]),
+    "dgvcc_lw_standardize_stats_h": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p,
+                                             c_void_p]),
+    "dgvcc_lw_gram_h": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_size_t,
+                                c_void_p, c_void_p]),
+    "dgvcc_lw_loss_backward_h": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                         c_int, c_void_p, c_size_t, c_void_p, c_void_p]),
+    "dgvcc_lw_standardize_backward_h": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
+                                                c_int, c_int, c_void_p, c_void_p]),
     "dgvcc_isw_gram_tc_partials": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "dgvcc_bay_knn_mean": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "dgvcc_bay_crop_targets": (c_int, [c_void_p, c_void_p, c_int, c_int, c_double, c_double, c_double, c_double, c_void_p,

@@ -29,6 +29,14 @@
 // 128B-swizzled layout TMA writes for fp32 input.  A widened half value is its own TF32 hi and its lo is exactly 0, so
 // the cross accumulator is dropped: one MMA per k step, TMEM 2 x 128 columns, same enable flags, SEG_KB segments and
 // drain order, hence the same partials bit for bit as the fp32 kernel on the upcast map.
+//
+// Standardise on load (isw_gram_tc_kernel<half, STD = true>, the Gram of lw_loss): TMA loads the half x tile as above, and
+// the converters compute  v = (x - mean_r) / sd_r  (times mask[sample, k] under a mask) with the IEEE operations of
+// lw_standardize_fwd_kernel, write v into the swizzled fp32 hi tile and  lo = RN_tf32(v - trunc_tf32(v))  beside it.  v has
+// low bits, so this variant keeps the fp32 kernel's 3 MMAs per k step, its cross accumulator and drains: the tensor core
+// sees exactly the operands the fp32 kernel sees on the materialised standardised map, and the partials are the same bits.
+// Where TMA zero-fills (k >= hw, rows past C, the missing second sample of an odd pair) the fp32 kernel reads y = 0, so the
+// converters write 0 there and read no statistics.  A stage (4 fp32 tiles + 2 half tiles = 80 KB) allows two stages.
 #include <type_traits>
 
 #include "tc_common.cuh"
@@ -40,20 +48,24 @@ namespace isw_tc {
 constexpr int TILE_M = 128;                 // rows of X per operand tile (= UMMA M = UMMA N)
 constexpr int BLOCK_K = 32;                 // fp32 per k block = one 128-byte swizzle row
 constexpr int UMMA_K = 8;                   // tf32 MMA k extent (32 bytes)
-constexpr int STAGES = 3;
 constexpr bool HI_BY_TRUNCATION = true;     // hi = what the tensor core reads of the raw tile (see the converter loop)
 constexpr int SEG_KB = 16;                  // k blocks accumulated in TMEM before a drain (512 k = 64 steps)
 constexpr int TILE_BYTES = TILE_M * BLOCK_K * 4;  // 16 KB
 constexpr int HTILE_BYTES = TILE_M * BLOCK_K * 2; // 8 KB: a half-precision tile as TMA delivers it
 constexpr int CONVERTER_WARPS = 8;                // two per SM sub-partition
 constexpr int THREADS = 64 + 32 * CONVERTER_WARPS;
-template <typename T> struct Cfg {
+template <typename T, bool STD = false> struct Cfg {
     static constexpr bool HALF = !std::is_same<T, float>::value;
-    // fp32: A_hi, B_hi, A_lo, B_lo.  half: A, B (fp32, widened), then the two half tiles TMA wrote
-    static constexpr int STAGE_BYTES = HALF ? 2 * TILE_BYTES + 2 * HTILE_BYTES : 4 * TILE_BYTES;
-    // two accumulator sets, each: hi*hi^T (128 columns) + cross terms (128 columns; none for half input)
-    static constexpr int TMEM_COLS = HALF ? 256 : 512;
-    static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /*alignment slack*/ + 256 /*barriers*/;
+    static constexpr bool LO = !HALF || STD;  // operands with a nonzero TF32 lo part: 3 MMAs per k step, cross accumulator
+    static constexpr int STAGES = STD ? 2 : 3;
+    // fp32: A_hi, B_hi, A_lo, B_lo.  half: A, B (fp32, widened), then the two half tiles TMA wrote.  STD: A_hi, B_hi, A_lo,
+    // B_lo, then the two half tiles
+    static constexpr int H_OFF = (LO ? 4 : 2) * TILE_BYTES;  // offset of the half tiles inside a stage
+    static constexpr int STAGE_BYTES = HALF ? H_OFF + 2 * HTILE_BYTES : 4 * TILE_BYTES;
+    // two accumulator sets, each: hi*hi^T (128 columns) + cross terms (128 columns; none for widened half input)
+    static constexpr int TMEM_COLS = LO ? 512 : 256;
+    static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /*alignment slack*/ + 256 /*barriers*/ +
+                                      (STD ? 2 * 2 * TILE_M * 4 : 0) /*mean, sd of the 256 rows*/;
 };
 
 using namespace dgvcc::tc;
@@ -65,18 +77,23 @@ __device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr) { return umma_
 constexpr uint32_t IDESC = umma_idesc_tf32(TILE_M, TILE_M, false);
 
 int launch_half(const void* x, int dtype, int batch, int c, int hw, int splits, int k_per_split, float* part, void* stream);
+int launch_std(const void* x, int dtype, const float* mean, const float* sd, const float* mask, int batch, int c, int hw,
+               int splits, int k_per_split, float* part, void* stream);
 
 struct Args {
     int c, hw, batch, splits, k_per_split, tiles_1d, n_tiles;
     int pair;     // c <= 64: one CTA holds two samples (64 rows each) in its 128-row tile
     float* part;  // [batch][splits][n_tiles][tile][tile], tile = 64 in pair mode, else 128
+    const float* mean;  // STD only: [batch * c] per-plane statistics, and the mask [batch, hw] or NULL
+    const float* sd;
+    const float* mask;
 };
 
-template <typename T>
+template <typename T, bool STD = false>
 __global__ void __launch_bounds__(THREADS, 1)
 isw_gram_tc_kernel(const __grid_constant__ CUtensorMap tmap, const Args a) {
-    constexpr bool HALF = Cfg<T>::HALF;
-    constexpr int STAGE_BYTES = Cfg<T>::STAGE_BYTES, TMEM_COLS = Cfg<T>::TMEM_COLS;
+    constexpr bool HALF = Cfg<T, STD>::HALF, LO = Cfg<T, STD>::LO;
+    constexpr int STAGES = Cfg<T, STD>::STAGES, STAGE_BYTES = Cfg<T, STD>::STAGE_BYTES, TMEM_COLS = Cfg<T, STD>::TMEM_COLS;
     extern __shared__ uint8_t smem_raw[];
     // 1024-byte alignment for the 128B-swizzled tiles
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -136,7 +153,7 @@ isw_gram_tc_kernel(const __grid_constant__ CUtensorMap tmap, const Args a) {
                 // pair mode: the box is {32 k, 64 rows, 2 samples} = the same 128-row tile
                 if constexpr (HALF) {
                     mbar_arrive_expect_tx(full_bar(s), diag ? HTILE_BYTES : 2 * HTILE_BYTES);
-                    const uint32_t h = stage + 2 * TILE_BYTES;
+                    const uint32_t h = stage + Cfg<T, STD>::H_OFF;
                     tma_load_3d(h, &tmap, full_bar(s), k0 + kb * BLOCK_K, ti * TILE_M, b);
                     if (!diag) tma_load_3d(h + HTILE_BYTES, &tmap, full_bar(s), k0 + kb * BLOCK_K, tj * TILE_M, b);
                 } else {
@@ -162,7 +179,7 @@ isw_gram_tc_kernel(const __grid_constant__ CUtensorMap tmap, const Args a) {
                 const uint32_t stage = base + s * STAGE_BYTES;
                 const uint64_t a_hi = umma_desc(stage);
                 const uint64_t b_hi = umma_desc(stage + (diag ? 0 : TILE_BYTES));
-                if constexpr (HALF) {  // lo == 0: hi hi^T only
+                if constexpr (!LO) {  // lo == 0: hi hi^T only
                     const uint32_t d_main = tmem_d + (uint32_t)set * TILE_M;
 #pragma unroll
                     for (int ks = 0; ks < BLOCK_K / UMMA_K; ++ks) {
@@ -202,7 +219,7 @@ isw_gram_tc_kernel(const __grid_constant__ CUtensorMap tmap, const Args a) {
             const int set = seg & 1;
             mbar_wait(acc_full_bar(set), (uint32_t)(seg >> 1) & 1u);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            if constexpr (HALF) {
+            if constexpr (!LO) {
                 if (useful) {
 #pragma unroll
                     for (int h = 0; h < 2; ++h) {
@@ -230,16 +247,92 @@ isw_gram_tc_kernel(const __grid_constant__ CUtensorMap tmap, const Args a) {
             if (lane == 0) mbar_arrive(acc_empty_bar(set));
         };
 
+        // STD: the statistics of the tile's 256 rows (A then B) go to shared memory once, thread ctid loading row ctid.
+        // This thread converts k chunk k4 of rows rr = ctid / 8 + 32 j (j < 4 on a diagonal tile) in every k block; a row
+        // that does not exist (past C, or the missing sample of an odd pair) has its bit of ok clear and is written as 0,
+        // like the rows TMA zero-fills for the fp32 kernel, and no statistics are read for it.
+        float* s_mu = reinterpret_cast<float*>(base_ptr + STAGES * STAGE_BYTES + 256);
+        float* s_sd = s_mu + 2 * TILE_M;
+        uint32_t ok = 0;
+        if constexpr (STD) {
+            auto row_of = [&](int rr, size_t& si) {  // false when row rr of [A; B] does not exist; else si = its plane
+                const int r = rr & (TILE_M - 1);
+                int sample, ch;
+                if (a.pair) { sample = b + (r >> 6); ch = r & 63; }
+                else { sample = b; ch = (rr < TILE_M ? ti : tj) * TILE_M + r; }
+                si = (size_t)sample * a.c + ch;
+                return sample < a.batch && ch < a.c && (rr < TILE_M || !diag);
+            };
+            size_t si;
+            if (row_of(ctid, si)) {
+                DGVCC_DEV_CHECK(si < (size_t)a.batch * a.c);
+                s_mu[ctid] = a.mean[si];
+                s_sd[ctid] = a.sd[si];
+            }
+#pragma unroll
+            for (int j = 0; j < 8; ++j)
+                if (row_of((ctid >> 3) + 32 * j, si)) ok |= 1u << j;
+            asm volatile("bar.sync 1, %0;" ::"n"(32 * CONVERTER_WARPS) : "memory");  // the converter warps only
+        }
+
         int drained = 0;
         for (int kb = 0; kb < n_kb; ++kb) {
             const int s = kb % STAGES;
             const uint32_t ph = (kb / STAGES) & 1;
             mbar_wait(full_bar(s), ph);
             uint8_t* stage = base_ptr + s * STAGE_BYTES;
-            if constexpr (HALF) {
+            if constexpr (STD) {
+                const T* src = reinterpret_cast<const T*>(stage + Cfg<T, STD>::H_OFF);
+                const int k4 = ctid & 7, kg = k0 + kb * BLOCK_K + 4 * k4;
+                const bool k_ok = kg < a.hw;  // hw % 4 == 0: the four k values are all inside or all outside
+                // mask values of the (at most two) samples of this tile at k = kg..kg+3
+                float4 m0 = make_float4(1.f, 1.f, 1.f, 1.f), m1 = m0;
+                if (a.mask && k_ok) {
+                    DGVCC_DEV_CHECK((size_t)b * a.hw + kg + 3 < (size_t)a.batch * a.hw);
+                    const float* mr = a.mask + (size_t)b * a.hw + kg;
+                    m0 = make_float4(mr[0], mr[1], mr[2], mr[3]);
+                    if (a.pair && b + 1 < a.batch) {
+                        mr += a.hw;
+                        m1 = make_float4(mr[0], mr[1], mr[2], mr[3]);
+                    }
+                }
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    if (j >= 4 && diag) break;
+                    const int rr = (ctid >> 3) + 32 * j;
+                    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+                    if (k_ok && (ok >> j & 1u)) {
+                        // the operations of lw_standardize_fwd_kernel: (x - mean) / sd, then * mask
+                        const float4 xv = widen4(src + rr * BLOCK_K + 4 * k4);
+                        const float mu = s_mu[rr], sd = s_sd[rr];
+                        v.x = __fdiv_rn(__fsub_rn(xv.x, mu), sd);
+                        v.y = __fdiv_rn(__fsub_rn(xv.y, mu), sd);
+                        v.z = __fdiv_rn(__fsub_rn(xv.z, mu), sd);
+                        v.w = __fdiv_rn(__fsub_rn(xv.w, mu), sd);
+                        if (a.mask) {
+                            const float4 m = a.pair && (rr & (TILE_M - 1)) >= 64 ? m1 : m0;
+                            v.x = __fmul_rn(v.x, m.x);
+                            v.y = __fmul_rn(v.y, m.y);
+                            v.z = __fmul_rn(v.z, m.z);
+                            v.w = __fmul_rn(v.w, m.w);
+                        }
+                    }
+                    // hi = v as the tensor core truncates it, lo = RN_tf32(v - trunc(v)) at the same swizzled place
+                    const int off = rr * 128 + ((k4 ^ (rr & 7)) << 4);
+                    *reinterpret_cast<float4*>(stage + off) = v;
+                    *reinterpret_cast<float4*>(stage + 2 * TILE_BYTES + off) =
+                        make_float4(tf32_round(v.x - tf32_trunc(v.x)), tf32_round(v.y - tf32_trunc(v.y)),
+                                    tf32_round(v.z - tf32_trunc(v.z)), tf32_round(v.w - tf32_trunc(v.w)));
+                }
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                __syncwarp();
+                if (lane == 0) mbar_arrive(ready_bar(s));
+                while (drained < n_seg - 1 && kb >= (drained + 1) * SEG_KB + 1) drain(drained++);
+                continue;
+            } else if constexpr (HALF) {
                 // widen [A; B] (128 or 256 rows of 32 half values) into the fp32 tiles: one float4 per thread and step,
                 // 16-byte chunk k4 of row r at chunk k4 ^ (r % 8) of the 128-byte row (the 128B swizzle)
-                const T* src = reinterpret_cast<const T*>(stage + 2 * TILE_BYTES);
+                const T* src = reinterpret_cast<const T*>(stage + Cfg<T, STD>::H_OFF);
 #pragma unroll 4
                 for (int i = ctid; i < (diag ? 1 : 2) * TILE_M * (BLOCK_K / 4); i += 32 * CONVERTER_WARPS) {
                     const int r = i >> 3, k4 = i & 7;
@@ -351,8 +444,9 @@ extern "C" int dgvcc_isw_gram_tc_partials(const float* x, int batch, int c, int 
     return (int)cudaGetLastError();
 }
 
-template <typename T>
-static int gram_tc_half(const void* x, int batch, int c, int hw, int splits, int k_per_split, float* part, void* stream) {
+template <typename T, bool STD>
+static int gram_tc_half(const void* x, const float* mean, const float* sd, const float* mask, int batch, int c, int hw,
+                        int splits, int k_per_split, float* part, void* stream) {
     const int pair = c <= 64;
     CUtensorMap tmap;
     if (!make_tmap_3d(&tmap, HalfIn<T>::TMA, 2, x, (uint64_t)hw, (uint64_t)c, (uint64_t)batch, BLOCK_K, pair ? 64 : TILE_M,
@@ -360,16 +454,18 @@ static int gram_tc_half(const void* x, int batch, int c, int hw, int splits, int
         return DGVCC_ERR_UNSUPPORTED;
     static PerDeviceOnce once;
     if (once.first())
-        DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_gram_tc_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                  Cfg<T>::SMEM_BYTES));
+        DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_gram_tc_kernel<T, STD>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                  Cfg<T, STD>::SMEM_BYTES));
     Args a;
     a.c = c; a.hw = hw; a.batch = batch; a.splits = splits; a.k_per_split = k_per_split;
     a.pair = pair;
     a.tiles_1d = pair ? 1 : ceil_div(c, TILE_M);
     a.n_tiles = a.tiles_1d * (a.tiles_1d + 1) / 2;
     a.part = part;
+    a.mean = mean; a.sd = sd; a.mask = mask;
     const int grid_z = pair ? ceil_div(batch, 2) : batch;
-    isw_gram_tc_kernel<T><<<dim3(a.n_tiles, splits, grid_z), THREADS, Cfg<T>::SMEM_BYTES, (cudaStream_t)stream>>>(tmap, a);
+    isw_gram_tc_kernel<T, STD><<<dim3(a.n_tiles, splits, grid_z), THREADS, Cfg<T, STD>::SMEM_BYTES, (cudaStream_t)stream>>>(
+        tmap, a);
     return (int)cudaGetLastError();
 }
 
@@ -380,6 +476,21 @@ int dgvcc::isw_tc::launch_half(const void* x, int dtype, int batch, int c, int h
     if (!x || !part || batch <= 0 || c <= 0 || hw <= 0 || splits <= 0 || k_per_split <= 0) return DGVCC_ERR_ARG;
     if (dtype != DGVCC_DTYPE_F16 && dtype != DGVCC_DTYPE_BF16) return DGVCC_ERR_ARG;
     if (hw % 8 != 0 || c < 32 || c % 4 != 0 || k_per_split % BLOCK_K != 0 || ((uintptr_t)x & 15u)) return DGVCC_ERR_UNSUPPORTED;
-    return dtype == DGVCC_DTYPE_F16 ? gram_tc_half<__half>(x, batch, c, hw, splits, k_per_split, part, stream)
-                                    : gram_tc_half<__nv_bfloat16>(x, batch, c, hw, splits, k_per_split, part, stream);
+    return dtype == DGVCC_DTYPE_F16
+               ? gram_tc_half<__half, false>(x, nullptr, nullptr, nullptr, batch, c, hw, splits, k_per_split, part, stream)
+               : gram_tc_half<__nv_bfloat16, false>(x, nullptr, nullptr, nullptr, batch, c, hw, splits, k_per_split, part,
+                                                    stream);
+}
+
+// The partials of the standardised map  y = (x - mean) / sd  (* mask)  from the half-precision x, y never materialised:
+// the same bits as dgvcc_isw_gram_tc_partials on y.  mean, sd [batch * c]; mask [batch, hw] or NULL.  Same shape rule as
+// launch_half.
+int dgvcc::isw_tc::launch_std(const void* x, int dtype, const float* mean, const float* sd, const float* mask, int batch,
+                              int c, int hw, int splits, int k_per_split, float* part, void* stream) {
+    if (!x || !mean || !sd || !part || batch <= 0 || c <= 0 || hw <= 0 || splits <= 0 || k_per_split <= 0) return DGVCC_ERR_ARG;
+    if (dtype != DGVCC_DTYPE_F16 && dtype != DGVCC_DTYPE_BF16) return DGVCC_ERR_ARG;
+    if (hw % 8 != 0 || c < 32 || c % 4 != 0 || k_per_split % BLOCK_K != 0 || ((uintptr_t)x & 15u)) return DGVCC_ERR_UNSUPPORTED;
+    return dtype == DGVCC_DTYPE_F16
+               ? gram_tc_half<__half, true>(x, mean, sd, mask, batch, c, hw, splits, k_per_split, part, stream)
+               : gram_tc_half<__nv_bfloat16, true>(x, mean, sd, mask, batch, c, hw, splits, k_per_split, part, stream);
 }

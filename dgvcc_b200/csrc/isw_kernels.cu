@@ -364,24 +364,36 @@ isw_covstat_var_kernel(const float* __restrict__ f_cor, const float* __restrict_
 
 // One CTA per (n, c) plane.  yhat = standardised plane (kept for the backward), ym = yhat * mask (the Gram input;
 // not written when there is no mask: ym == yhat).
+// STATS (half-precision x, lw_loss's native route): only mean, sd and invstd of the plane are written -- the values the
+// fp32 instantiation computes on the upcast plane; the fused Gram and dY = S Y standardise on load from them.
+template <typename T, bool STATS>
 __global__ void __launch_bounds__(NORM_THREADS)
-lw_standardize_fwd_kernel(const float* __restrict__ x, const float* __restrict__ mask, int channels, int hw, float eps,
-                          float* __restrict__ yhat, float* __restrict__ ym, float* __restrict__ invstd_out) {
+lw_standardize_fwd_kernel(const T* __restrict__ x, const float* __restrict__ mask, int channels, int hw, float eps,
+                          float* __restrict__ yhat, float* __restrict__ ym, float* __restrict__ invstd_out,
+                          float* __restrict__ mean_out, float* __restrict__ sd_out) {
     __shared__ float scratch[NORM_THREADS / 32];
     const size_t base = (size_t)blockIdx.x * hw;
     float s = 0.f;
-    for (int i = threadIdx.x; i < hw; i += NORM_THREADS) s += x[base + i];
+    for (int i = threadIdx.x; i < hw; i += NORM_THREADS) s += Elem<T>::load(x[base + i]);
     const float mean = block_sum(s, scratch) / (float)hw;
     float q = 0.f;
     for (int i = threadIdx.x; i < hw; i += NORM_THREADS) {
-        const float d = x[base + i] - mean;
+        const float d = Elem<T>::load(x[base + i]) - mean;
         q = fmaf(d, d, q);
     }
     const float var = block_sum(q, scratch) / (float)(hw - 1);  // torch.var: unbiased; hw == 1 -> nan like torch
     const float sd = sqrtf(var + eps);
+    if constexpr (STATS) {
+        if (threadIdx.x == 0) {
+            mean_out[blockIdx.x] = mean;
+            sd_out[blockIdx.x] = sd;
+            invstd_out[blockIdx.x] = 1.0f / sd;
+        }
+        return;
+    }
     const float* mrow = mask ? mask + (size_t)(blockIdx.x / channels) * hw : nullptr;
     for (int i = threadIdx.x; i < hw; i += NORM_THREADS) {
-        const float v = (x[base + i] - mean) / sd;
+        const float v = (Elem<T>::load(x[base + i]) - mean) / sd;
         yhat[base + i] = v;
         if (mrow) ym[base + i] = v * mrow[i];
     }
@@ -407,6 +419,35 @@ lw_standardize_bwd_kernel(const float* __restrict__ dy, const float* __restrict_
     for (int i = threadIdx.x; i < hw; i += NORM_THREADS) {
         const float g = mrow ? dy[base + i] * mrow[i] : dy[base + i];
         dx[base + i] = is * (g - m1 - yhat[base + i] * m2);
+    }
+}
+
+// The same for a half-precision x: yhat is recomputed from x, mean and sd with the forward's operations ((x - mean) / sd:
+// a sub and a true division, nothing to contract), so it is the fp32 route's yhat bit for bit; dx is written as RN(dx).
+template <typename T>
+__global__ void __launch_bounds__(NORM_THREADS)
+lw_standardize_bwd_half_kernel(const float* __restrict__ dy, const T* __restrict__ x, const float* __restrict__ mean,
+                               const float* __restrict__ sd, const float* __restrict__ invstd, const float* __restrict__ mask,
+                               int channels, int hw, T* __restrict__ dx) {
+    __shared__ float scratch[NORM_THREADS / 32];
+    const size_t base = (size_t)blockIdx.x * hw;
+    const float* mrow = mask ? mask + (size_t)(blockIdx.x / channels) * hw : nullptr;
+    const float mu = mean[blockIdx.x], sdv = sd[blockIdx.x];
+    // the rounding sequence is spelled out: it is the one nvcc compiles lw_standardize_bwd_kernel to (g = dy * m rounded
+    // in the sums; g - m1 contracted to fma(dy, m, -m1) in the output, then fma(yhat, -m2, .) and the product with is)
+    float s1 = 0.f, s2 = 0.f;
+    for (int i = threadIdx.x; i < hw; i += NORM_THREADS) {
+        const float g = mrow ? __fmul_rn(dy[base + i], mrow[i]) : dy[base + i];
+        s1 = __fadd_rn(s1, g);
+        s2 = __fmaf_rn(g, __fdiv_rn(__fsub_rn(Elem<T>::load(x[base + i]), mu), sdv), s2);
+    }
+    const float m1 = block_sum(s1, scratch) / (float)hw;
+    const float m2 = block_sum(s2, scratch) / (float)(hw - 1);
+    const float is = invstd[blockIdx.x];
+    for (int i = threadIdx.x; i < hw; i += NORM_THREADS) {
+        const float t = mrow ? __fmaf_rn(dy[base + i], mrow[i], -m1) : __fsub_rn(dy[base + i], m1);
+        const float yhat = __fdiv_rn(__fsub_rn(Elem<T>::load(x[base + i]), mu), sdv);
+        dx[base + i] = Elem<T>::store(__fmul_rn(is, __fmaf_rn(yhat, -m2, t)));
     }
 }
 
@@ -742,6 +783,8 @@ extern "C" int dgvcc_isw_gram_tc_partials(const float* x, int batch, int c, int 
 
 namespace dgvcc { namespace isw_tc {
 int launch_half(const void* x, int dtype, int batch, int c, int hw, int splits, int k_per_split, float* part, void* stream);
+int launch_std(const void* x, int dtype, const float* mean, const float* sd, const float* mask, int batch, int c, int hw,
+               int splits, int k_per_split, float* part, void* stream);
 } }
 
 // The one shape rule of the half-precision Gram and dX = S X (isw_gram_tc.cu, isw_sx_tc.cu): TMA needs 16-byte row strides
@@ -827,6 +870,8 @@ int launch(const float* s, const float* x, int batch, int c, int hw, float* dx, 
 namespace dgvcc { namespace isw_sx {
 int launch_half(const float* s, const void* x, int dtype, int batch, int c, int hw, void* dx, const float* scale,
                 bool a_is_tf32_exact, void* stream);
+int launch_std(const float* s, const void* x, int dtype, const float* mean, const float* sd, const float* mask, int batch,
+               int c, int hw, float* dy, void* stream);
 } }
 
 // the shapes / alignments dgvcc::isw_sx::launch accepts
@@ -938,7 +983,9 @@ extern "C" int dgvcc_lw_standardize_forward(const float* x, const float* mask, i
                                             float* yhat, float* y_masked, float* invstd, void* stream) {
     DGVCC_DEVICE_GUARD(stream);
     if (!x || !yhat || !invstd || batch <= 0 || c <= 0 || hw <= 0 || (mask && !y_masked)) return DGVCC_ERR_ARG;
-    lw_standardize_fwd_kernel<<<batch * c, NORM_THREADS, 0, (cudaStream_t)stream>>>(x, mask, c, hw, eps, yhat, y_masked, invstd);
+    lw_standardize_fwd_kernel<float, false><<<batch * c, NORM_THREADS, 0, (cudaStream_t)stream>>>(x, mask, c, hw, eps, yhat,
+                                                                                                  y_masked, invstd, nullptr,
+                                                                                                  nullptr);
     return (int)cudaGetLastError();
 }
 
@@ -1015,4 +1062,109 @@ extern "C" int dgvcc_ortho_loss_backward(const float* x, const float* y, const f
     const int rc = launch_sx(sx, y, 1, c, p, use_tensor_cores, grad_x, st);
     if (rc != DGVCC_OK) return rc;
     return launch_sx(sy, x, 1, c, p, use_tensor_cores, grad_y, st);
+}
+
+// ------------------------------------------------------- auxiliary Gram losses: half-precision entry points
+// Everything below returns what the fp32 entry points above return on the map upcast to fp32 (DESIGN section 5b); the
+// Gram and dX = S X run on the tensor cores only, under the shape rule half_tc_tiles.
+
+// The tensor-core partials (Gram of the half map, or of lw's standardised map) finished as X X^T: no scaling, no eps.
+static int finish_gram(int batch, int c, int tile, int n_tiles, int splits, const IswWs& w, float* gram, cudaStream_t st) {
+    const int yblocks = (tile / 32) * (tile / 32);
+    isw_cov_finish_kernel<<<dim3(n_tiles, yblocks, batch), 256, 0, st>>>(w.part, c, 1.0f, splits, tile, nullptr, 0.f, gram);
+    return (int)cudaGetLastError();
+}
+
+extern "C" int dgvcc_isw_gram_h(const void* f_map, int dtype, int batch, int c, int hw, void* workspace,
+                                size_t workspace_bytes, float* gram, void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    if (!f_map || !workspace || !gram || !isw_shape_ok(batch, c, hw) || !half_dtype(dtype)) return DGVCC_ERR_ARG;
+    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
+    if (!half_tc_tiles(f_map, f_map, c, hw)) return DGVCC_ERR_UNSUPPORTED;
+    const IswWs w = carve(workspace, batch, c, hw);
+    cudaStream_t st = (cudaStream_t)stream;
+    int splits, kps, n_tiles, tile;
+    gram_plan_tc(batch, c, hw, &splits, &kps, &n_tiles, &tile);
+    const int rc = dgvcc::isw_tc::launch_half(f_map, dtype, batch, c, hw, splits, kps, w.part, (void*)st);
+    if (rc != DGVCC_OK) return rc;
+    return finish_gram(batch, c, tile, n_tiles, splits, w, gram, st);
+}
+
+// x, y, grad_x, grad_y [c, p] half; gram_zz from dgvcc_isw_gram_h on z = [x; y].
+extern "C" int dgvcc_ortho_loss_backward_h(const void* x, const void* y, int dtype, const float* gram_zz,
+                                           const float* grad_loss, int c, int p, void* workspace, size_t workspace_bytes,
+                                           void* grad_x, void* grad_y, void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    if (!x || !y || !gram_zz || !grad_loss || !workspace || !grad_x || !grad_y || c > 16384 || !isw_shape_ok(1, 2 * c, p) ||
+        !half_dtype(dtype))
+        return DGVCC_ERR_ARG;
+    if (workspace_bytes < dgvcc_isw_workspace_bytes(1, 2 * c, p)) return DGVCC_ERR_WORKSPACE;
+    if (!half_tc_tiles(x, grad_x, c, p) || !half_tc_tiles(y, grad_y, c, p)) return DGVCC_ERR_UNSUPPORTED;
+    const IswWs w = carve(workspace, 1, 2 * c, p);
+    cudaStream_t st = (cudaStream_t)stream;
+    float* sx = w.s;
+    float* sy = w.s + (size_t)c * c;
+    ortho_grad_s_kernel<<<ceil_div(c * c, 256), 256, 0, st>>>(gram_zz, grad_loss, c, sx, sy);
+    DGVCC_RETURN_IF_CUDA(cudaGetLastError());
+    const int rc = dgvcc::isw_sx::launch_half(sx, y, dtype, 1, c, p, grad_x, nullptr, false, (void*)st);
+    if (rc != DGVCC_OK) return rc;
+    return dgvcc::isw_sx::launch_half(sy, x, dtype, 1, c, p, grad_y, nullptr, false, (void*)st);
+}
+
+extern "C" int dgvcc_lw_standardize_stats_h(const void* x, int dtype, int batch, int c, int hw, float eps, float* mean,
+                                            float* sd, float* invstd, void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    if (!x || !mean || !sd || !invstd || !isw_shape_ok(batch, c, hw) || !half_dtype(dtype)) return DGVCC_ERR_ARG;
+    if (dtype == DGVCC_DTYPE_F16)
+        lw_standardize_fwd_kernel<__half, true><<<batch * c, NORM_THREADS, 0, (cudaStream_t)stream>>>(
+            (const __half*)x, nullptr, c, hw, eps, nullptr, nullptr, invstd, mean, sd);
+    else
+        lw_standardize_fwd_kernel<__nv_bfloat16, true><<<batch * c, NORM_THREADS, 0, (cudaStream_t)stream>>>(
+            (const __nv_bfloat16*)x, nullptr, c, hw, eps, nullptr, nullptr, invstd, mean, sd);
+    return (int)cudaGetLastError();
+}
+
+extern "C" int dgvcc_lw_gram_h(const void* x, int dtype, const float* mean, const float* sd, const float* mask, int batch,
+                               int c, int hw, void* workspace, size_t workspace_bytes, float* gram, void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    if (!x || !mean || !sd || !workspace || !gram || !isw_shape_ok(batch, c, hw) || !half_dtype(dtype)) return DGVCC_ERR_ARG;
+    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
+    if (!half_tc_tiles(x, x, c, hw)) return DGVCC_ERR_UNSUPPORTED;
+    const IswWs w = carve(workspace, batch, c, hw);
+    cudaStream_t st = (cudaStream_t)stream;
+    int splits, kps, n_tiles, tile;
+    gram_plan_tc(batch, c, hw, &splits, &kps, &n_tiles, &tile);
+    const int rc = dgvcc::isw_tc::launch_std(x, dtype, mean, sd, mask, batch, c, hw, splits, kps, w.part, (void*)st);
+    if (rc != DGVCC_OK) return rc;
+    return finish_gram(batch, c, tile, n_tiles, splits, w, gram, st);
+}
+
+extern "C" int dgvcc_lw_loss_backward_h(const void* x, int dtype, const float* mean, const float* sd, const float* mask,
+                                        const float* gram, const float* grad_loss, int batch, int c, int hw, void* workspace,
+                                        size_t workspace_bytes, float* grad_y, void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    if (!x || !mean || !sd || !gram || !grad_loss || !workspace || !grad_y || !isw_shape_ok(batch, c, hw) ||
+        !half_dtype(dtype))
+        return DGVCC_ERR_ARG;
+    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
+    if (!half_tc_tiles(x, grad_y, c, hw)) return DGVCC_ERR_UNSUPPORTED;
+    const IswWs w = carve(workspace, batch, c, hw);
+    cudaStream_t st = (cudaStream_t)stream;
+    lw_grad_s_kernel<<<dim3(ceil_div(c * c, 256), batch), 256, 0, st>>>(gram, grad_loss, c, w.s);
+    DGVCC_RETURN_IF_CUDA(cudaGetLastError());
+    return dgvcc::isw_sx::launch_std(w.s, x, dtype, mean, sd, mask, batch, c, hw, grad_y, (void*)st);
+}
+
+extern "C" int dgvcc_lw_standardize_backward_h(const float* dy, const void* x, int dtype, const float* mean, const float* sd,
+                                               const float* invstd, const float* mask, int batch, int c, int hw, void* dx,
+                                               void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    if (!dy || !x || !mean || !sd || !invstd || !dx || !isw_shape_ok(batch, c, hw) || !half_dtype(dtype)) return DGVCC_ERR_ARG;
+    if (dtype == DGVCC_DTYPE_F16)
+        lw_standardize_bwd_half_kernel<<<batch * c, NORM_THREADS, 0, (cudaStream_t)stream>>>(
+            dy, (const __half*)x, mean, sd, invstd, mask, c, hw, (__half*)dx);
+    else
+        lw_standardize_bwd_half_kernel<<<batch * c, NORM_THREADS, 0, (cudaStream_t)stream>>>(
+            dy, (const __nv_bfloat16*)x, mean, sd, invstd, mask, c, hw, (__nv_bfloat16*)dx);
+    return (int)cudaGetLastError();
 }

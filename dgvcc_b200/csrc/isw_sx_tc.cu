@@ -23,6 +23,13 @@
 // (box j = n / 32 at j * 4 KB, k row kk at kk * 128 B, 32-byte chunk c at chunk c ^ (kk % 4)).  X_lo is exactly 0, so
 // the MMAs on it go away: EXACT runs 1 MMA per k step (S X_hi), the general variant 2 (S_hi X_hi, and S_lo X_hi opening
 // the cross accumulator).  dX is written rounded to nearest in the input's type.
+//
+// Standardise on load (isw_sx_tc_kernel<false, half, STD = true>, dY = S Y of lw_loss's backward): TMA loads the half X
+// tile as above, and the converters compute  y = (x - mean_k) / sd_k  (times mask[n] under a mask) with the IEEE
+// operations of lw_standardize_fwd_kernel, k being the channel, and write hi and lo = RN_tf32(y - trunc_tf32(y)) into the
+// B_hi / B_lo tiles of the fp32 layout.  The MMAs and the fp32 epilogue are those of the fp32 general kernel, so dY is the
+// same bits as dgvcc_isw_sx_tc on the materialised standardised map.  Channels k >= C and columns n >= hw are written as
+// 0, what TMA zero-fills there for the fp32 kernel, without reading statistics or mask.
 #include <type_traits>
 
 #include "tc_common.cuh"
@@ -40,12 +47,13 @@ constexpr int TILE_BYTES = TILE * BLOCK_K * 4;  // 16 KB for either operand
 constexpr int THREADS = 192;
 constexpr int CONVERTER_WARPS = 4;
 constexpr int HTILE_BYTES = TILE * BLOCK_K * 2;  // 8 KB: a half-precision X tile as TMA delivers it
-template <bool EXACT, typename T = float> struct Cfg {
+template <bool EXACT, typename T = float, bool STD = false> struct Cfg {
     static constexpr bool HALF = !std::is_same<T, float>::value;
     static constexpr int STAGES = EXACT ? 2 : 3;
-    // fp32: EXACT: A, B_hi, B_lo; else A_hi, B_hi, A_lo, B_lo.  half: the same without B_lo, then the half X tile (B_H)
+    // fp32: EXACT: A, B_hi, B_lo; else A_hi, B_hi, A_lo, B_lo.  half: the same without B_lo, then the half X tile (B_H).
+    // STD (general only): A_hi, B_hi, A_lo, B_lo, then the half X tile
     static constexpr int B_LO = (EXACT ? 2 : 3) * TILE_BYTES;         // offset of B_lo (half: of B_H) inside a stage
-    static constexpr int B_H = B_LO;
+    static constexpr int B_H = STD ? 4 * TILE_BYTES : B_LO;
     static constexpr int STAGE_BYTES = HALF ? B_H + HTILE_BYTES : (EXACT ? 3 : 4) * TILE_BYTES;
     static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 + 256;
     static constexpr int TMEM_COLS = HALF && EXACT ? 128 : 256;  // main accumulator (+ cross terms)
@@ -58,19 +66,25 @@ int launch(const float* s, const float* x, int batch, int c, int hw, float* dx, 
            void* stream);
 int launch_half(const float* s, const void* x, int dtype, int batch, int c, int hw, void* dx, const float* scale,
                 bool a_is_tf32_exact, void* stream);
+int launch_std(const float* s, const void* x, int dtype, const float* mean, const float* sd, const float* mask, int batch,
+               int c, int hw, float* dy, void* stream);
 
 struct Args {
     int c, hw;
     void* dx;              // float or T
     const float* scale;    // [batch] factor applied in the epilogue, or NULL (= 1)
+    const float* mean;     // STD only: [batch * c] per-plane statistics, and the mask [batch, hw] or NULL
+    const float* sd;
+    const float* mask;
 };
 
-template <bool EXACT, typename T>
+template <bool EXACT, typename T, bool STD = false>
 __global__ void __launch_bounds__(THREADS, EXACT ? 2 : 1)
 isw_sx_tc_kernel(const __grid_constant__ CUtensorMap map_s, const __grid_constant__ CUtensorMap map_x, const Args a) {
-    constexpr bool HALF = Cfg<EXACT, T>::HALF;
-    constexpr int STAGES = Cfg<EXACT, T>::STAGES, STAGE_BYTES = Cfg<EXACT, T>::STAGE_BYTES, B_LO = Cfg<EXACT, T>::B_LO;
-    constexpr int B_H = Cfg<EXACT, T>::B_H, TMEM_COLS = Cfg<EXACT, T>::TMEM_COLS;
+    constexpr bool HALF = Cfg<EXACT, T, STD>::HALF;
+    constexpr int STAGES = Cfg<EXACT, T, STD>::STAGES, STAGE_BYTES = Cfg<EXACT, T, STD>::STAGE_BYTES;
+    constexpr int B_LO = Cfg<EXACT, T, STD>::B_LO;
+    constexpr int B_H = Cfg<EXACT, T, STD>::B_H, TMEM_COLS = Cfg<EXACT, T, STD>::TMEM_COLS;
     extern __shared__ uint8_t smem_raw[];
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     uint8_t* base_ptr = smem_raw + (base - smem_u32(smem_raw));
@@ -141,7 +155,7 @@ isw_sx_tc_kernel(const __grid_constant__ CUtensorMap map_s, const __grid_constan
                     // A (K-major): +32 B inside the swizzle row per k step; B (MN-major): next 8-row k group
                     const uint64_t a_hi = umma_desc_sw128(stage + ks * UMMA_K * 4, 16, 1024);
                     const uint64_t b_hi = umma_desc(stage + TILE_BYTES + ks * 1024, B_BOX_BYTES, 512, 1);
-                    if constexpr (HALF) {  // X_lo == 0
+                    if constexpr (HALF && !STD) {  // X_lo == 0
                         umma_tf32(tmem_d, a_hi, b_hi, IDESC, (kb | ks) != 0);
                         if (!EXACT) {
                             const uint64_t a_lo = umma_desc_sw128(stage + 2 * TILE_BYTES + ks * UMMA_K * 4, 16, 1024);
@@ -169,7 +183,59 @@ isw_sx_tc_kernel(const __grid_constant__ CUtensorMap map_s, const __grid_constan
             const uint32_t ph = (kb / STAGES) & 1;
             mbar_wait(full_bar(s), ph);
             uint8_t* stage = base_ptr + s * STAGE_BYTES;
-            if constexpr (HALF) {
+            if constexpr (STD) {
+                {  // A_lo beside A_hi, as the fp32 general kernel
+                    const float4* hi = reinterpret_cast<const float4*>(stage);
+                    float4* lo = reinterpret_cast<float4*>(stage + 2 * TILE_BYTES);
+#pragma unroll 4
+                    for (int i = ctid; i < TILE_BYTES / 16; i += 128) {
+                        const float4 v = hi[i];
+                        lo[i] = make_float4(tf32_round(v.x - tf32_trunc(v.x)), tf32_round(v.y - tf32_trunc(v.y)),
+                                            tf32_round(v.z - tf32_trunc(v.z)), tf32_round(v.w - tf32_trunc(v.w)));
+                    }
+                }
+                // standardise X: this thread's four n values are the same in every k block (n4 = ctid % 32), so is their mask
+                const T* src = reinterpret_cast<const T*>(stage + B_H);
+                const int n4 = ctid & 31, n = n0 + 4 * n4;
+                const bool n_ok = n < a.hw;  // hw % 4 == 0: all four inside or all outside
+                float4 m = make_float4(1.f, 1.f, 1.f, 1.f);
+                if (a.mask && n_ok) {
+                    DGVCC_DEV_CHECK((size_t)b * a.hw + n + 3 < (size_t)gridDim.z * a.hw);
+                    const float* mr = a.mask + (size_t)b * a.hw + n;
+                    m = make_float4(mr[0], mr[1], mr[2], mr[3]);
+                }
+#pragma unroll 4
+                for (int i = ctid; i < BLOCK_K * TILE / 4; i += 128) {
+                    const int kk = i >> 5, ch = kb * BLOCK_K + kk;
+                    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+                    if (n_ok && ch < a.c) {
+                        const size_t si = (size_t)b * a.c + ch;
+                        DGVCC_DEV_CHECK(si < (size_t)gridDim.z * a.c);
+                        const float mu = a.mean[si], sd = a.sd[si];
+                        const float4 xv = widen4(src + kk * TILE + 4 * n4);
+                        v.x = __fdiv_rn(__fsub_rn(xv.x, mu), sd);
+                        v.y = __fdiv_rn(__fsub_rn(xv.y, mu), sd);
+                        v.z = __fdiv_rn(__fsub_rn(xv.z, mu), sd);
+                        v.w = __fdiv_rn(__fsub_rn(xv.w, mu), sd);
+                        if (a.mask) {
+                            v.x = __fmul_rn(v.x, m.x);
+                            v.y = __fmul_rn(v.y, m.y);
+                            v.z = __fmul_rn(v.z, m.z);
+                            v.w = __fmul_rn(v.w, m.w);
+                        }
+                    }
+                    uint8_t* dst = stage + TILE_BYTES + (n4 >> 3) * B_BOX_BYTES + kk * 128 + ((((n4 >> 1) & 3) ^ (kk & 3)) << 5) +
+                                   ((n4 & 1) << 4);
+                    *reinterpret_cast<float4*>(dst) = v;
+                    *reinterpret_cast<float4*>(dst + (B_LO - TILE_BYTES)) =
+                        make_float4(tf32_round(v.x - tf32_trunc(v.x)), tf32_round(v.y - tf32_trunc(v.y)),
+                                    tf32_round(v.z - tf32_trunc(v.z)), tf32_round(v.w - tf32_trunc(v.w)));
+                }
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                __syncwarp();
+                if (lane == 0) mbar_arrive(ready_bar(s));
+                continue;
+            } else if constexpr (HALF) {
                 if (!EXACT) {  // A_lo beside A_hi
                     const float4* hi = reinterpret_cast<const float4*>(stage);
                     float4* lo = reinterpret_cast<float4*>(stage + 2 * TILE_BYTES);
@@ -218,7 +284,7 @@ isw_sx_tc_kernel(const __grid_constant__ CUtensorMap map_s, const __grid_constan
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         const int lane_base = 32 * (warp & 3);
         const int row = m0 + lane_base + lane;
-        if constexpr (HALF) {
+        if constexpr (HALF && !STD) {
             T* out = static_cast<T*>(a.dx) + ((size_t)b * a.c + row) * a.hw + n0;
             const float sc = a.scale ? a.scale[b] : 1.f;
 #pragma unroll 1
@@ -334,6 +400,39 @@ static int sx_tc_half(const float* s, const void* x, int batch, int c, int hw, v
     else
         isw_sx_tc_kernel<false, T><<<grid, THREADS, Cfg<false, T>::SMEM_BYTES, (cudaStream_t)stream>>>(map_s, map_x, a);
     return (int)cudaGetLastError();
+}
+
+template <typename T>
+static int sx_tc_std(const float* s, const void* x, const float* mean, const float* sd, const float* mask, int batch, int c,
+                     int hw, float* dy, void* stream) {
+    CUtensorMap map_s, map_x;
+    if (!make_tmap_f32_3d(&map_s, s, (uint64_t)c, (uint64_t)c, (uint64_t)batch, TILE)) return DGVCC_ERR_UNSUPPORTED;
+    if (!make_tmap_3d(&map_x, HalfIn<T>::TMA, 2, x, (uint64_t)hw, (uint64_t)c, (uint64_t)batch, TILE, BLOCK_K,
+                      CU_TENSOR_MAP_SWIZZLE_NONE, 1))
+        return DGVCC_ERR_UNSUPPORTED;
+    static PerDeviceOnce once;
+    if (once.first())
+        DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_sx_tc_kernel<false, T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                  Cfg<false, T, true>::SMEM_BYTES));
+    Args a;
+    a.c = c; a.hw = hw; a.dx = dy; a.scale = nullptr;
+    a.mean = mean; a.sd = sd; a.mask = mask;
+    const dim3 grid(ceil_div(hw, TILE), ceil_div(c, TILE), batch);
+    isw_sx_tc_kernel<false, T, true><<<grid, THREADS, Cfg<false, T, true>::SMEM_BYTES, (cudaStream_t)stream>>>(map_s, map_x, a);
+    return (int)cudaGetLastError();
+}
+
+// dY_b = S_b Y_b in fp32 with Y = (X - mean) / sd (* mask) standardised on load from the half-precision X, Y never
+// materialised: the same bits as dgvcc_isw_sx_tc on Y.  mean, sd [batch * c]; mask [batch, hw] or NULL.  Same shape rule
+// as launch_half, and a 16-byte aligned dY.
+int dgvcc::isw_sx::launch_std(const float* s, const void* x, int dtype, const float* mean, const float* sd, const float* mask,
+                              int batch, int c, int hw, float* dy, void* stream) {
+    if (!s || !x || !mean || !sd || !dy || batch <= 0 || c <= 0 || hw <= 0) return DGVCC_ERR_ARG;
+    if (dtype != DGVCC_DTYPE_F16 && dtype != DGVCC_DTYPE_BF16) return DGVCC_ERR_ARG;
+    if (hw % 8 != 0 || c % 4 != 0 || c < 32 || ((uintptr_t)s & 15u) || ((uintptr_t)x & 15u) || ((uintptr_t)dy & 15u))
+        return DGVCC_ERR_UNSUPPORTED;
+    return dtype == DGVCC_DTYPE_F16 ? sx_tc_std<__half>(s, x, mean, sd, mask, batch, c, hw, dy, stream)
+                                    : sx_tc_std<__nv_bfloat16>(s, x, mean, sd, mask, batch, c, hw, dy, stream);
 }
 
 // dX_b = scale_b * (S_b X_b) for a half-precision X and dX (dtype DGVCC_DTYPE_F16 / _BF16), S in fp32.  TMA needs

@@ -527,6 +527,35 @@ int dgvcc_ortho_loss_backward(const float* x, const float* y, const float* gram_
                               int use_tensor_cores, void* workspace, size_t workspace_bytes, float* grad_x,
                               float* grad_y, void* stream);
 
+/* Half-precision inputs of the auxiliary losses (autocast training; dtype DGVCC_DTYPE_F16 / DGVCC_DTYPE_BF16): every
+ * output is what the fp32 entry points above compute on the input upcast to fp32, bit for bit, gradients rounded to
+ * nearest into the input type.  The Gram and dX = S X run on the tensor cores only: for hw (p) % 8 != 0, c < 32,
+ * c % 4 != 0 or a half-precision pointer that is not 16-byte aligned they return DGVCC_ERR_UNSUPPORTED, and the caller
+ * upcasts.  mean, sd, invstd [batch*c], mask [batch, hw] (or NULL), gram and grad_y stay fp32. */
+/* lw.py:16 and ortho.py:9 on a half map: gram [batch, c, c] = X X^T, as dgvcc_isw_gram. */
+int dgvcc_isw_gram_h(const void* f_map, int dtype, int batch, int c, int hw, void* workspace, size_t workspace_bytes,
+                     float* gram, void* stream);
+/* ortho.py:9-11 backward on half x, y [c, p]; grad_x, grad_y half. */
+int dgvcc_ortho_loss_backward_h(const void* x, const void* y, int dtype, const float* gram_zz, const float* grad_loss,
+                                int c, int p, void* workspace, size_t workspace_bytes, void* grad_x, void* grad_y,
+                                void* stream);
+/* lw.py:11-13: the statistics of dgvcc_lw_standardize_forward only (mean, sd = sqrt(var + eps), invstd = 1 / sd); the
+ * standardised map is never written. */
+int dgvcc_lw_standardize_stats_h(const void* x, int dtype, int batch, int c, int hw, float eps, float* mean, float* sd,
+                                 float* invstd, void* stream);
+/* lw.py:13-16: gram = Y Y^T with Y = (x - mean) / sd (* mask) standardised inside the Gram kernel. */
+int dgvcc_lw_gram_h(const void* x, int dtype, const float* mean, const float* sd, const float* mask, int batch, int c,
+                    int hw, void* workspace, size_t workspace_bytes, float* gram, void* stream);
+/* Backward of lw.py:16-18: grad_y [batch, c, hw] fp32 = (dG + dG^T) Y, Y standardised inside the GEMM, as
+ * dgvcc_lw_loss_backward on Y. */
+int dgvcc_lw_loss_backward_h(const void* x, int dtype, const float* mean, const float* sd, const float* mask,
+                             const float* gram, const float* grad_loss, int batch, int c, int hw, void* workspace,
+                             size_t workspace_bytes, float* grad_y, void* stream);
+/* Backward of lw.py:11-15: dx (half) from dy (fp32); yhat is recomputed from x, mean and sd. */
+int dgvcc_lw_standardize_backward_h(const float* dy, const void* x, int dtype, const float* mean, const float* sd,
+                                    const float* invstd, const float* mask, int batch, int c, int hw, void* dx,
+                                    void* stream);
+
 /* ---------------------------------------------------------------------------
  * Switchable whitening (SURVEY.md 8f rank 4) -- replaces SwitchWhiten2d.forward
  * (models/ISW/switchwhiten.py:84-183) and SyncMeanCov / SyncSwitchWhiten2d.forward
