@@ -190,7 +190,26 @@ def lib():
     return _lib
 
 
-_ERRORS = {-1: "invalid argument", -2: "workspace too small", -3: "unsupported configuration"}
+ERR_UNSUPPORTED = -3  # DGVCC_ERR_UNSUPPORTED: a shape or alignment the kernel does not tile
+_ERRORS = {-1: "invalid argument", -2: "workspace too small", ERR_UNSUPPORTED: "unsupported configuration"}
+
+
+_half_codes = None
+
+
+def half_code(dtype):
+    """DTYPE_F16 / DTYPE_BF16 for torch.float16 / torch.bfloat16, None for any other dtype."""
+    global _half_codes
+    if _half_codes is None:
+        import torch
+        _half_codes = {torch.float16: DTYPE_F16, torch.bfloat16: DTYPE_BF16}
+    return _half_codes.get(dtype)
+
+
+def use_tensor_cores():
+    """DGVCC_ISW_TENSOR_CORES (default 1), read on every call: 0 runs the ISW-family GEMMs on their exact fp32
+    CUDA-core kernels and sends fp16 / bf16 inputs down the upcast route."""
+    return int(os.environ.get("DGVCC_ISW_TENSOR_CORES", "1"))
 
 
 def check(rc, what):

@@ -39,6 +39,7 @@
 // converters write 0 there and read no statistics.  A stage (4 fp32 tiles + 2 half tiles = 80 KB) allows two stages.
 #include <type_traits>
 
+#include "isw_tc.cuh"
 #include "tc_common.cuh"
 #include "../../include/dgvcc_b200.h"
 
@@ -75,10 +76,6 @@ __device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr) { return umma_
 
 // kind::tf32, fp32 accumulate, A and B K-major, M = N = 128.
 constexpr uint32_t IDESC = umma_idesc_tf32(TILE_M, TILE_M, false);
-
-int launch_half(const void* x, int dtype, int batch, int c, int hw, int splits, int k_per_split, float* part, void* stream);
-int launch_std(const void* x, int dtype, const float* mean, const float* sd, const float* mask, int batch, int c, int hw,
-               int splits, int k_per_split, float* part, void* stream);
 
 struct Args {
     int c, hw, batch, splits, k_per_split, tiles_1d, n_tiles;
@@ -415,43 +412,24 @@ isw_gram_tc_kernel(const __grid_constant__ CUtensorMap tmap, const Args a) {
 using namespace dgvcc;
 using namespace dgvcc::isw_tc;
 
-extern "C" int dgvcc_isw_gram_tc_partials(const float* x, int batch, int c, int hw, int splits, int k_per_split,
-                                          float* part, void* stream) {
-    DGVCC_DEVICE_GUARD(stream);
-    if (!x || !part || batch <= 0 || c <= 0 || hw <= 0 || splits <= 0 || k_per_split <= 0) return DGVCC_ERR_ARG;
-    // TMA needs 16-byte global strides and a 16-byte aligned base; rows past C are zero-filled by the
-    // tensor map, so any C works, but tiny channel counts waste the 128-wide tile
-    if (hw % 4 != 0 || c < 32 || k_per_split % BLOCK_K != 0 || ((uintptr_t)x & 15u)) return DGVCC_ERR_UNSUPPORTED;
-
-    const int pair = c <= 64;
-    CUtensorMap tmap;
-    if (!make_tmap_f32_3d(&tmap, x, (uint64_t)hw, (uint64_t)c, (uint64_t)batch, pair ? 64 : TILE_M, CU_TENSOR_MAP_SWIZZLE_128B,
-                          pair ? 2 : 1))
-        return DGVCC_ERR_UNSUPPORTED;
-
-    static PerDeviceOnce once;
-    if (once.first())
-        DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_gram_tc_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                  Cfg<float>::SMEM_BYTES));
-    Args a;
-    a.c = c; a.hw = hw; a.batch = batch; a.splits = splits; a.k_per_split = k_per_split;
-    a.pair = pair;
-    a.tiles_1d = pair ? 1 : ceil_div(c, TILE_M);
-    a.n_tiles = a.tiles_1d * (a.tiles_1d + 1) / 2;
-    a.part = part;
-    const int grid_z = pair ? ceil_div(batch, 2) : batch;
-    isw_gram_tc_kernel<float><<<dim3(a.n_tiles, splits, grid_z), THREADS, Cfg<float>::SMEM_BYTES, (cudaStream_t)stream>>>(tmap, a);
-    return (int)cudaGetLastError();
-}
-
+// fp32 x: the 128B-swizzled tiles the MMAs read.  Half x: its raw 32 k x 128 row tiles, which the converters widen.
 template <typename T, bool STD>
-static int gram_tc_half(const void* x, const float* mean, const float* sd, const float* mask, int batch, int c, int hw,
-                        int splits, int k_per_split, float* part, void* stream) {
+int dgvcc::isw_tc::launch(const T* x, const float* mean, const float* sd, const float* mask, int batch, int c, int hw,
+                          int splits, int k_per_split, float* part, cudaStream_t stream) {
+    constexpr bool HALF = Cfg<T, STD>::HALF;
+    // rows past C are zero-filled by the tensor map, so C needs no multiple of the tile
+    if (!(HALF ? half_tc_tiles(c, hw) : gram_tc_tiles(c, hw)) || k_per_split % BLOCK_K != 0 || !tma_aligned(x))
+        return DGVCC_ERR_UNSUPPORTED;
     const int pair = c <= 64;
     CUtensorMap tmap;
-    if (!make_tmap_3d(&tmap, HalfIn<T>::TMA, 2, x, (uint64_t)hw, (uint64_t)c, (uint64_t)batch, BLOCK_K, pair ? 64 : TILE_M,
-                      CU_TENSOR_MAP_SWIZZLE_NONE, pair ? 2 : 1))
-        return DGVCC_ERR_UNSUPPORTED;
+    bool mapped;
+    if constexpr (HALF)
+        mapped = make_tmap_3d(&tmap, HalfIn<T>::TMA, 2, x, (uint64_t)hw, (uint64_t)c, (uint64_t)batch, BLOCK_K,
+                              pair ? 64 : TILE_M, CU_TENSOR_MAP_SWIZZLE_NONE, pair ? 2 : 1);
+    else
+        mapped = make_tmap_f32_3d(&tmap, x, (uint64_t)hw, (uint64_t)c, (uint64_t)batch, pair ? 64 : TILE_M,
+                                  CU_TENSOR_MAP_SWIZZLE_128B, pair ? 2 : 1);
+    if (!mapped) return DGVCC_ERR_UNSUPPORTED;
     static PerDeviceOnce once;
     if (once.first())
         DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_gram_tc_kernel<T, STD>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -464,33 +442,24 @@ static int gram_tc_half(const void* x, const float* mean, const float* sd, const
     a.part = part;
     a.mean = mean; a.sd = sd; a.mask = mask;
     const int grid_z = pair ? ceil_div(batch, 2) : batch;
-    isw_gram_tc_kernel<T, STD><<<dim3(a.n_tiles, splits, grid_z), THREADS, Cfg<T, STD>::SMEM_BYTES, (cudaStream_t)stream>>>(
-        tmap, a);
+    isw_gram_tc_kernel<T, STD><<<dim3(a.n_tiles, splits, grid_z), THREADS, Cfg<T, STD>::SMEM_BYTES, stream>>>(tmap, a);
     return (int)cudaGetLastError();
 }
 
-// The same partials from a half-precision map (dtype DGVCC_DTYPE_F16 / _BF16).  TMA needs 16-byte global strides
-// (hw % 8 == 0) and a 16-byte aligned base; c % 4 == 0 keeps one shape rule for the Gram and dX = S X (isw_sx_tc.cu).
-int dgvcc::isw_tc::launch_half(const void* x, int dtype, int batch, int c, int hw, int splits, int k_per_split, float* part,
-                               void* stream) {
-    if (!x || !part || batch <= 0 || c <= 0 || hw <= 0 || splits <= 0 || k_per_split <= 0) return DGVCC_ERR_ARG;
-    if (dtype != DGVCC_DTYPE_F16 && dtype != DGVCC_DTYPE_BF16) return DGVCC_ERR_ARG;
-    if (hw % 8 != 0 || c < 32 || c % 4 != 0 || k_per_split % BLOCK_K != 0 || ((uintptr_t)x & 15u)) return DGVCC_ERR_UNSUPPORTED;
-    return dtype == DGVCC_DTYPE_F16
-               ? gram_tc_half<__half, false>(x, nullptr, nullptr, nullptr, batch, c, hw, splits, k_per_split, part, stream)
-               : gram_tc_half<__nv_bfloat16, false>(x, nullptr, nullptr, nullptr, batch, c, hw, splits, k_per_split, part,
-                                                    stream);
-}
+template int dgvcc::isw_tc::launch<float, false>(const float*, const float*, const float*, const float*, int, int, int, int,
+                                                 int, float*, cudaStream_t);
+template int dgvcc::isw_tc::launch<__half, false>(const __half*, const float*, const float*, const float*, int, int, int, int,
+                                                  int, float*, cudaStream_t);
+template int dgvcc::isw_tc::launch<__nv_bfloat16, false>(const __nv_bfloat16*, const float*, const float*, const float*, int,
+                                                         int, int, int, int, float*, cudaStream_t);
+template int dgvcc::isw_tc::launch<__half, true>(const __half*, const float*, const float*, const float*, int, int, int, int,
+                                                 int, float*, cudaStream_t);
+template int dgvcc::isw_tc::launch<__nv_bfloat16, true>(const __nv_bfloat16*, const float*, const float*, const float*, int,
+                                                        int, int, int, int, float*, cudaStream_t);
 
-// The partials of the standardised map  y = (x - mean) / sd  (* mask)  from the half-precision x, y never materialised:
-// the same bits as dgvcc_isw_gram_tc_partials on y.  mean, sd [batch * c]; mask [batch, hw] or NULL.  Same shape rule as
-// launch_half.
-int dgvcc::isw_tc::launch_std(const void* x, int dtype, const float* mean, const float* sd, const float* mask, int batch,
-                              int c, int hw, int splits, int k_per_split, float* part, void* stream) {
-    if (!x || !mean || !sd || !part || batch <= 0 || c <= 0 || hw <= 0 || splits <= 0 || k_per_split <= 0) return DGVCC_ERR_ARG;
-    if (dtype != DGVCC_DTYPE_F16 && dtype != DGVCC_DTYPE_BF16) return DGVCC_ERR_ARG;
-    if (hw % 8 != 0 || c < 32 || c % 4 != 0 || k_per_split % BLOCK_K != 0 || ((uintptr_t)x & 15u)) return DGVCC_ERR_UNSUPPORTED;
-    return dtype == DGVCC_DTYPE_F16
-               ? gram_tc_half<__half, true>(x, mean, sd, mask, batch, c, hw, splits, k_per_split, part, stream)
-               : gram_tc_half<__nv_bfloat16, true>(x, mean, sd, mask, batch, c, hw, splits, k_per_split, part, stream);
+extern "C" int dgvcc_isw_gram_tc_partials(const float* x, int batch, int c, int hw, int splits, int k_per_split,
+                                          float* part, void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    if (!x || !part || batch <= 0 || c <= 0 || hw <= 0 || splits <= 0 || k_per_split <= 0) return DGVCC_ERR_ARG;
+    return launch(x, nullptr, nullptr, nullptr, batch, c, hw, splits, k_per_split, part, (cudaStream_t)stream);
 }

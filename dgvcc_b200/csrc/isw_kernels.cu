@@ -16,6 +16,9 @@
 // Half-precision feature maps (fp16 / bf16, the *_h entry points): the instance norm is templated over the element type
 // and the Gram / dX = S X run the half variants of the tensor-core kernels; every value is the one the fp32 path computes
 // on the upcast map (DESIGN section 5).
+#include <type_traits>
+
+#include "isw_tc.cuh"
 #include "tc_common.cuh"
 #include "../../include/dgvcc_b200.h"
 
@@ -676,27 +679,29 @@ extern "C" int dgvcc_isw_instnorm_forward(const float* x, int planes, int hw, fl
     return instnorm_forward(x, planes, hw, eps, y, mean, invstd, stream);
 }
 
-static bool half_dtype(int dtype) { return dtype == DGVCC_DTYPE_F16 || dtype == DGVCC_DTYPE_BF16; }
+// The fp16 / bf16 dispatch of the *_h entry points: runs the statements `...` with T the element type dtype names, and
+// returns DGVCC_ERR_ARG for any other dtype.  A macro rather than a function template over a generic lambda, so a kernel
+// template launched in the statements is instantiated where it stands and the kernels keep their order in the object.
+#define DGVCC_BY_HALF_DTYPE(dtype, ...)                                                          \
+    do {                                                                                         \
+        if ((dtype) == DGVCC_DTYPE_F16) { using T = __half; __VA_ARGS__ }                        \
+        else if ((dtype) == DGVCC_DTYPE_BF16) { using T = __nv_bfloat16; __VA_ARGS__ }           \
+        else return DGVCC_ERR_ARG;                                                               \
+    } while (0)
 
 extern "C" int dgvcc_isw_instnorm_forward_h(const void* x, int dtype, int planes, int hw, float eps, void* y, float* mean,
                                             float* invstd, void* stream) {
     DGVCC_DEVICE_GUARD(stream);
-    if (!x || !y || !mean || !invstd || planes <= 0 || hw <= 0 || !half_dtype(dtype)) return DGVCC_ERR_ARG;
-    if (dtype == DGVCC_DTYPE_F16)
-        return instnorm_forward((const __half*)x, planes, hw, eps, (__half*)y, mean, invstd, stream);
-    return instnorm_forward((const __nv_bfloat16*)x, planes, hw, eps, (__nv_bfloat16*)y, mean, invstd, stream);
+    if (!x || !y || !mean || !invstd || planes <= 0 || hw <= 0) return DGVCC_ERR_ARG;
+    DGVCC_BY_HALF_DTYPE(dtype, return instnorm_forward((const T*)x, planes, hw, eps, (T*)y, mean, invstd, stream););
 }
 
 extern "C" int dgvcc_isw_instnorm_backward_h(const void* dy, const void* x, const float* mean, const float* invstd, int dtype,
                                              int planes, int hw, void* dx, void* stream) {
     DGVCC_DEVICE_GUARD(stream);
-    if (!dy || !x || !mean || !invstd || !dx || planes <= 0 || hw <= 0 || !half_dtype(dtype)) return DGVCC_ERR_ARG;
-    if (dtype == DGVCC_DTYPE_F16)
-        isw_instnorm_bwd_half_kernel<<<planes, NORM_THREADS, 0, (cudaStream_t)stream>>>(
-            (const __half*)dy, (const __half*)x, mean, invstd, hw, (__half*)dx);
-    else
-        isw_instnorm_bwd_half_kernel<<<planes, NORM_THREADS, 0, (cudaStream_t)stream>>>(
-            (const __nv_bfloat16*)dy, (const __nv_bfloat16*)x, mean, invstd, hw, (__nv_bfloat16*)dx);
+    if (!dy || !x || !mean || !invstd || !dx || planes <= 0 || hw <= 0) return DGVCC_ERR_ARG;
+    DGVCC_BY_HALF_DTYPE(dtype, isw_instnorm_bwd_half_kernel<<<planes, NORM_THREADS, 0, (cudaStream_t)stream>>>(
+                                   (const T*)dy, (const T*)x, mean, invstd, hw, (T*)dx););
     return (int)cudaGetLastError();
 }
 
@@ -777,73 +782,79 @@ IswWs carve(void* ws, int batch, int c, int hw) {
 }
 }  // namespace
 
-// implemented in isw_gram_tc.cu; returns DGVCC_ERR_UNSUPPORTED for shapes it does not tile
-extern "C" int dgvcc_isw_gram_tc_partials(const float* x, int batch, int c, int hw, int splits, int k_per_split,
-                                          float* part, void* stream);
+template <typename T> constexpr bool HALF = !std::is_same<T, float>::value;
 
-namespace dgvcc { namespace isw_tc {
-int launch_half(const void* x, int dtype, int batch, int c, int hw, int splits, int k_per_split, float* part, void* stream);
-int launch_std(const void* x, int dtype, const float* mean, const float* sd, const float* mask, int batch, int c, int hw,
-               int splits, int k_per_split, float* part, void* stream);
-} }
-
-// The one shape rule of the half-precision Gram and dX = S X (isw_gram_tc.cu, isw_sx_tc.cu): TMA needs 16-byte row strides
-// (hw % 8 == 0) and 16-byte aligned bases; c >= 32 and c % 4 == 0 as for the fp32 dX = S X.  Other shapes return
-// DGVCC_ERR_UNSUPPORTED from every *_h Gram / dX entry point, forward and backward alike, and run upcast to fp32.
-static bool half_tc_tiles(const void* x, const void* out, int c, int hw) {
-    return hw % 8 == 0 && c % 4 == 0 && c >= 32 && !(((uintptr_t)x | (uintptr_t)out) & 15u);
-}
-
-// Gram of every sample on the tensor cores where the shape tiles (else exact fp32 on CUDA cores), finished as
-// out = X X^T / denom (+ eps * eye when eye is given).
-static int launch_gram(const float* f_map, const float* eye, float denom, float eps, int batch, int c, int hw,
-                       int use_tensor_cores, const IswWs& w, float* out, cudaStream_t st) {
+// Gram of every sample, finished as out = X X^T / denom (+ eps * eye when eye is given).  The tensor-core partials where
+// the shape tiles; else exact fp32 on CUDA cores for an fp32 map, and DGVCC_ERR_UNSUPPORTED for a half one.  STD: the Gram
+// of lw's standardised map (x - mean) / sd (* mask), computed from the half x.
+template <typename T, bool STD = false>
+static int launch_gram(const T* x, const float* mean, const float* sd, const float* mask, const float* eye, float denom,
+                       float eps, int batch, int c, int hw, int use_tensor_cores, const IswWs& w, float* out, cudaStream_t st) {
     int splits, kps, n_tiles, tile = 64;
-    bool done = false;
+    int rc = DGVCC_ERR_UNSUPPORTED;
     if (use_tensor_cores) {
         gram_plan_tc(batch, c, hw, &splits, &kps, &n_tiles, &tile);
-        const int rc = dgvcc_isw_gram_tc_partials(f_map, batch, c, hw, splits, kps, w.part, (void*)st);
-        if (rc == DGVCC_OK) done = true;
-        else if (rc != DGVCC_ERR_UNSUPPORTED) return rc;
+        rc = isw_tc::launch<T, STD>(x, mean, sd, mask, batch, c, hw, splits, kps, w.part, st);
     }
-    if (!done) {
-        tile = 64;
-        gram_plan_simt(batch, c, hw, &splits, &kps, &n_tiles);
-        isw_gram_simt_kernel<<<dim3(n_tiles, splits, batch), GEMM_THREADS, 0, st>>>(f_map, c, hw, splits, kps, w.part);
-        DGVCC_RETURN_IF_CUDA(cudaGetLastError());
+    if constexpr (!HALF<T>) {
+        if (rc == DGVCC_ERR_UNSUPPORTED) {
+            tile = 64;
+            gram_plan_simt(batch, c, hw, &splits, &kps, &n_tiles);
+            isw_gram_simt_kernel<<<dim3(n_tiles, splits, batch), GEMM_THREADS, 0, st>>>(x, c, hw, splits, kps, w.part);
+            rc = (int)cudaGetLastError();
+        }
     }
+    if (rc != DGVCC_OK) return rc;
     const int yblocks = (tile / 32) * (tile / 32);
     isw_cov_finish_kernel<<<dim3(n_tiles, yblocks, batch), 256, 0, st>>>(w.part, c, denom, splits, tile, eye, eps, out);
     return (int)cudaGetLastError();
 }
 
+// dX = S X on the tensor cores where the shape tiles; else exact fp32 on CUDA cores for an fp32 X, and
+// DGVCC_ERR_UNSUPPORTED for a half one.
+template <typename T>
+static int launch_sx(const float* s, const void* x, int batch, int c, int hw, int use_tensor_cores, void* dx, cudaStream_t st) {
+    int rc = DGVCC_ERR_UNSUPPORTED;
+    if (use_tensor_cores)
+        rc = isw_sx::launch<T>(s, (const T*)x, nullptr, nullptr, nullptr, batch, c, hw, dx, nullptr, false, st);
+    if constexpr (!HALF<T>) {
+        if (rc == DGVCC_ERR_UNSUPPORTED) {
+            isw_sx_simt_kernel<<<dim3(ceil_div(hw, GT), ceil_div(c, GT), batch), GEMM_THREADS, 0, st>>>(s, (const float*)x, c,
+                                                                                                      hw, (float*)dx);
+            rc = (int)cudaGetLastError();
+        }
+    }
+    return rc;
+}
+
+// A half dX = S X has no CUDA-core fallback, so the half backwards refuse a shape the tensor cores do not tile before they
+// compute S (the launcher checks the rule again, S's base included).
+template <typename T> static bool half_untiled(const void* x, const void* dx, int c, int hw) {
+    return HALF<T> && !(half_tc_tiles(c, hw) && tma_aligned(x, dx));
+}
+
+// The fp32 and half (*_h) entry points share one body per pair, templated over the element type T of the map and its
+// gradient.  The half types run on the tensor cores only (use_tensor_cores = 1) and return DGVCC_ERR_UNSUPPORTED where
+// fp32 falls back to the CUDA cores; every value is the one the fp32 path computes on the upcast map (DESIGN section 5).
+template <typename T>
+static int covariance(const void* f_map, const float* eye, int batch, int c, int hw, int use_tensor_cores, void* workspace,
+                      size_t workspace_bytes, float* f_cor, void* stream) {
+    if (!f_map || !eye || !workspace || !f_cor || !isw_shape_ok(batch, c, hw) || hw <= 1) return DGVCC_ERR_ARG;
+    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
+    return launch_gram((const T*)f_map, nullptr, nullptr, nullptr, eye, (float)(hw - 1), 1e-5f, batch, c, hw, use_tensor_cores,
+                       carve(workspace, batch, c, hw), f_cor, (cudaStream_t)stream);
+}
+
 extern "C" int dgvcc_isw_covariance(const float* f_map, const float* eye, int batch, int c, int hw, int use_tensor_cores,
                                     void* workspace, size_t workspace_bytes, float* f_cor, void* stream) {
     DGVCC_DEVICE_GUARD(stream);
-    if (!f_map || !eye || !workspace || !f_cor || !isw_shape_ok(batch, c, hw) || hw <= 1) return DGVCC_ERR_ARG;
-    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
-    const IswWs w = carve(workspace, batch, c, hw);
-    return launch_gram(f_map, eye, (float)(hw - 1), 1e-5f, batch, c, hw, use_tensor_cores, w, f_cor, (cudaStream_t)stream);
+    return covariance<float>(f_map, eye, batch, c, hw, use_tensor_cores, workspace, workspace_bytes, f_cor, stream);
 }
 
-// The half-precision map: the tensor-core Gram only (the caller checked half_tc_tiles), same split plan and finish.
 extern "C" int dgvcc_isw_covariance_h(const void* f_map, int dtype, const float* eye, int batch, int c, int hw,
                                       void* workspace, size_t workspace_bytes, float* f_cor, void* stream) {
     DGVCC_DEVICE_GUARD(stream);
-    if (!f_map || !eye || !workspace || !f_cor || !isw_shape_ok(batch, c, hw) || hw <= 1 || !half_dtype(dtype))
-        return DGVCC_ERR_ARG;
-    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
-    if (!half_tc_tiles(f_map, f_map, c, hw)) return DGVCC_ERR_UNSUPPORTED;
-    const IswWs w = carve(workspace, batch, c, hw);
-    cudaStream_t st = (cudaStream_t)stream;
-    int splits, kps, n_tiles, tile;
-    gram_plan_tc(batch, c, hw, &splits, &kps, &n_tiles, &tile);
-    const int rc = dgvcc::isw_tc::launch_half(f_map, dtype, batch, c, hw, splits, kps, w.part, (void*)st);
-    if (rc != DGVCC_OK) return rc;
-    const int yblocks = (tile / 32) * (tile / 32);
-    isw_cov_finish_kernel<<<dim3(n_tiles, yblocks, batch), 256, 0, st>>>(w.part, c, (float)(hw - 1), splits, tile, eye, 1e-5f,
-                                                                         f_cor);
-    return (int)cudaGetLastError();
+    DGVCC_BY_HALF_DTYPE(dtype, return covariance<T>(f_map, eye, batch, c, hw, 1, workspace, workspace_bytes, f_cor, stream););
 }
 
 extern "C" int dgvcc_isw_loss_forward(const float* f_cor, const float* mask, const float* margin,
@@ -861,33 +872,27 @@ extern "C" int dgvcc_isw_loss_forward(const float* f_cor, const float* mask, con
     return (int)cudaGetLastError();
 }
 
-// implemented in isw_sx_tc.cu; returns DGVCC_ERR_UNSUPPORTED for shapes it does not tile
-namespace dgvcc { namespace isw_sx {
-int launch(const float* s, const float* x, int batch, int c, int hw, float* dx, const float* scale, bool a_is_tf32_exact,
-           void* stream);
-} }
-
-namespace dgvcc { namespace isw_sx {
-int launch_half(const float* s, const void* x, int dtype, int batch, int c, int hw, void* dx, const float* scale,
-                bool a_is_tf32_exact, void* stream);
-int launch_std(const float* s, const void* x, int dtype, const float* mean, const float* sd, const float* mask, int batch,
-               int c, int hw, float* dy, void* stream);
-} }
-
-// the shapes / alignments dgvcc::isw_sx::launch accepts
-static bool sx_tc_tiles(const float* s, const float* x, const float* dx, int c, int hw) {
-    return hw % 4 == 0 && c % 4 == 0 && c >= 32 && !(((uintptr_t)s | (uintptr_t)x | (uintptr_t)dx) & 15u);
-}
-
-// dX = S X on the tensor cores where the shape tiles, else exact fp32 on CUDA cores
-static int launch_sx(const float* s, const float* x, int batch, int c, int hw, int use_tensor_cores, float* dx,
-                     cudaStream_t st) {
-    if (use_tensor_cores) {
-        const int rc = dgvcc::isw_sx::launch(s, x, batch, c, hw, dx, nullptr, false, (void*)st);
-        if (rc != DGVCC_ERR_UNSUPPORTED) return rc;
+template <typename T>
+static int loss_backward(const void* f_map, const float* f_cor, const float* mask, const float* num_remove_cov,
+                         const float* grad_loss, int batch, int c, int hw, int use_tensor_cores, int mask_is_binary,
+                         void* workspace, size_t workspace_bytes, void* grad_f_map, void* stream) {
+    if (!f_map || !f_cor || !mask || !num_remove_cov || !grad_loss || !workspace || !grad_f_map || !isw_shape_ok(batch, c, hw)) return DGVCC_ERR_ARG;
+    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
+    if (half_untiled<T>(f_map, grad_f_map, c, hw)) return DGVCC_ERR_UNSUPPORTED;
+    const IswWs w = carve(workspace, batch, c, hw);
+    cudaStream_t st = (cudaStream_t)stream;
+    const dim3 s_grid(ceil_div(c, 32), ceil_div(c, 32), batch);
+    if (mask_is_binary && (HALF<T> || (use_tensor_cores && sx_tc_tiles(c, hw) && tma_aligned(w.s, f_map, grad_f_map)))) {
+        // factored S = alpha * T: the GEMM runs on T (TF32-exact for a 0/1 mask) and scales in its epilogue
+        isw_loss_grad_kernel<<<s_grid, 256, 0, st>>>(f_cor, mask, w.off, num_remove_cov, grad_loss, c, hw, batch, w.s, w.alpha);
+        DGVCC_RETURN_IF_CUDA(cudaGetLastError());
+        const int rc = isw_sx::launch<T>(w.s, (const T*)f_map, nullptr, nullptr, nullptr, batch, c, hw, grad_f_map, w.alpha,
+                                         true, st);
+        if (HALF<T> || rc != DGVCC_ERR_UNSUPPORTED) return rc;
     }
-    isw_sx_simt_kernel<<<dim3(ceil_div(hw, GT), ceil_div(c, GT), batch), GEMM_THREADS, 0, st>>>(s, x, c, hw, dx);
-    return (int)cudaGetLastError();
+    isw_loss_grad_kernel<<<s_grid, 256, 0, st>>>(f_cor, mask, w.off, num_remove_cov, grad_loss, c, hw, batch, w.s, nullptr);
+    DGVCC_RETURN_IF_CUDA(cudaGetLastError());
+    return launch_sx<T>(w.s, f_map, batch, c, hw, use_tensor_cores, grad_f_map, st);
 }
 
 extern "C" int dgvcc_isw_loss_backward(const float* f_map, const float* f_cor, const float* mask,
@@ -895,35 +900,8 @@ extern "C" int dgvcc_isw_loss_backward(const float* f_map, const float* f_cor, c
                                        int use_tensor_cores, int mask_is_binary, void* workspace,
                                        size_t workspace_bytes, float* grad_f_map, void* stream) {
     DGVCC_DEVICE_GUARD(stream);
-    if (!f_map || !f_cor || !mask || !num_remove_cov || !grad_loss || !workspace || !grad_f_map || !isw_shape_ok(batch, c, hw)) return DGVCC_ERR_ARG;
-    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
-    const IswWs w = carve(workspace, batch, c, hw);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (use_tensor_cores && mask_is_binary && sx_tc_tiles(w.s, f_map, grad_f_map, c, hw)) {
-        // factored S = alpha * T: the GEMM runs on T (TF32-exact for a 0/1 mask) and scales in its epilogue
-        isw_loss_grad_kernel<<<dim3(ceil_div(c, 32), ceil_div(c, 32), batch), 256, 0, st>>>(f_cor, mask, w.off, num_remove_cov, grad_loss,
-                                                                                c, hw, batch, w.s, w.alpha);
-        DGVCC_RETURN_IF_CUDA(cudaGetLastError());
-        const int rc = dgvcc::isw_sx::launch(w.s, f_map, batch, c, hw, grad_f_map, w.alpha, true, (void*)st);
-        if (rc != DGVCC_ERR_UNSUPPORTED) return rc;
-    }
-    isw_loss_grad_kernel<<<dim3(ceil_div(c, 32), ceil_div(c, 32), batch), 256, 0, st>>>(f_cor, mask, w.off, num_remove_cov, grad_loss,
-                                                                            c, hw, batch, w.s, nullptr);
-    DGVCC_RETURN_IF_CUDA(cudaGetLastError());
-    return launch_sx(w.s, f_map, batch, c, hw, use_tensor_cores, grad_f_map, st);
-}
-
-extern "C" int dgvcc_isw_covariance_backward(const float* f_map, const float* grad_f_cor, int batch, int c, int hw,
-                                             int use_tensor_cores, void* workspace, size_t workspace_bytes,
-                                             float* grad_f_map, void* stream) {
-    DGVCC_DEVICE_GUARD(stream);
-    if (!f_map || !grad_f_cor || !workspace || !grad_f_map || !isw_shape_ok(batch, c, hw)) return DGVCC_ERR_ARG;
-    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
-    const IswWs w = carve(workspace, batch, c, hw);
-    cudaStream_t st = (cudaStream_t)stream;
-    isw_cov_grad_kernel<<<dim3(ceil_div(c * c, 256), batch), 256, 0, st>>>(grad_f_cor, c, hw, w.s);
-    DGVCC_RETURN_IF_CUDA(cudaGetLastError());
-    return launch_sx(w.s, f_map, batch, c, hw, use_tensor_cores, grad_f_map, st);
+    return loss_backward<float>(f_map, f_cor, mask, num_remove_cov, grad_loss, batch, c, hw, use_tensor_cores, mask_is_binary,
+                                workspace, workspace_bytes, grad_f_map, stream);
 }
 
 extern "C" int dgvcc_isw_loss_backward_h(const void* f_map, int dtype, const float* f_cor, const float* mask,
@@ -931,34 +909,37 @@ extern "C" int dgvcc_isw_loss_backward_h(const void* f_map, int dtype, const flo
                                          int mask_is_binary, void* workspace, size_t workspace_bytes, void* grad_f_map,
                                          void* stream) {
     DGVCC_DEVICE_GUARD(stream);
-    if (!f_map || !f_cor || !mask || !num_remove_cov || !grad_loss || !workspace || !grad_f_map ||
-        !isw_shape_ok(batch, c, hw) || !half_dtype(dtype))
-        return DGVCC_ERR_ARG;
+    DGVCC_BY_HALF_DTYPE(dtype, return loss_backward<T>(f_map, f_cor, mask, num_remove_cov, grad_loss, batch, c, hw, 1,
+                                                       mask_is_binary, workspace, workspace_bytes, grad_f_map, stream););
+}
+
+template <typename T>
+static int covariance_backward(const void* f_map, const float* grad_f_cor, int batch, int c, int hw, int use_tensor_cores,
+                               void* workspace, size_t workspace_bytes, void* grad_f_map, void* stream) {
+    if (!f_map || !grad_f_cor || !workspace || !grad_f_map || !isw_shape_ok(batch, c, hw)) return DGVCC_ERR_ARG;
     if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
-    if (!half_tc_tiles(f_map, grad_f_map, c, hw)) return DGVCC_ERR_UNSUPPORTED;
+    if (half_untiled<T>(f_map, grad_f_map, c, hw)) return DGVCC_ERR_UNSUPPORTED;
     const IswWs w = carve(workspace, batch, c, hw);
     cudaStream_t st = (cudaStream_t)stream;
-    // binary mask: factored S = alpha * T and the EXACT GEMM, as dgvcc_isw_loss_backward
-    isw_loss_grad_kernel<<<dim3(ceil_div(c, 32), ceil_div(c, 32), batch), 256, 0, st>>>(
-        f_cor, mask, w.off, num_remove_cov, grad_loss, c, hw, batch, w.s, mask_is_binary ? w.alpha : nullptr);
+    isw_cov_grad_kernel<<<dim3(ceil_div(c * c, 256), batch), 256, 0, st>>>(grad_f_cor, c, hw, w.s);
     DGVCC_RETURN_IF_CUDA(cudaGetLastError());
-    return dgvcc::isw_sx::launch_half(w.s, f_map, dtype, batch, c, hw, grad_f_map, mask_is_binary ? w.alpha : nullptr,
-                                      mask_is_binary != 0, (void*)st);
+    return launch_sx<T>(w.s, f_map, batch, c, hw, use_tensor_cores, grad_f_map, st);
+}
+
+extern "C" int dgvcc_isw_covariance_backward(const float* f_map, const float* grad_f_cor, int batch, int c, int hw,
+                                             int use_tensor_cores, void* workspace, size_t workspace_bytes,
+                                             float* grad_f_map, void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    return covariance_backward<float>(f_map, grad_f_cor, batch, c, hw, use_tensor_cores, workspace, workspace_bytes,
+                                      grad_f_map, stream);
 }
 
 extern "C" int dgvcc_isw_covariance_backward_h(const void* f_map, int dtype, const float* grad_f_cor, int batch, int c,
                                                int hw, void* workspace, size_t workspace_bytes, void* grad_f_map,
                                                void* stream) {
     DGVCC_DEVICE_GUARD(stream);
-    if (!f_map || !grad_f_cor || !workspace || !grad_f_map || !isw_shape_ok(batch, c, hw) || !half_dtype(dtype))
-        return DGVCC_ERR_ARG;
-    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
-    if (!half_tc_tiles(f_map, grad_f_map, c, hw)) return DGVCC_ERR_UNSUPPORTED;
-    const IswWs w = carve(workspace, batch, c, hw);
-    cudaStream_t st = (cudaStream_t)stream;
-    isw_cov_grad_kernel<<<dim3(ceil_div(c * c, 256), batch), 256, 0, st>>>(grad_f_cor, c, hw, w.s);
-    DGVCC_RETURN_IF_CUDA(cudaGetLastError());
-    return dgvcc::isw_sx::launch_half(w.s, f_map, dtype, batch, c, hw, grad_f_map, nullptr, false, (void*)st);
+    DGVCC_BY_HALF_DTYPE(dtype, return covariance_backward<T>(f_map, grad_f_cor, batch, c, hw, 1, workspace, workspace_bytes,
+                                                             grad_f_map, stream););
 }
 
 extern "C" int dgvcc_isw_covstat_var(const float* f_cor, const float* reverse_eye, int batch, int c, float* var_out,
@@ -997,13 +978,25 @@ extern "C" int dgvcc_lw_standardize_backward(const float* dy, const float* yhat,
     return (int)cudaGetLastError();
 }
 
+template <typename T>
+static int gram(const void* f_map, int batch, int c, int hw, int use_tensor_cores, void* workspace, size_t workspace_bytes,
+                float* gram, void* stream) {
+    if (!f_map || !workspace || !gram || !isw_shape_ok(batch, c, hw)) return DGVCC_ERR_ARG;
+    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
+    return launch_gram((const T*)f_map, nullptr, nullptr, nullptr, nullptr, 1.0f, 0.f, batch, c, hw, use_tensor_cores,
+                       carve(workspace, batch, c, hw), gram, (cudaStream_t)stream);
+}
+
 extern "C" int dgvcc_isw_gram(const float* f_map, int batch, int c, int hw, int use_tensor_cores, void* workspace,
                               size_t workspace_bytes, float* gram, void* stream) {
     DGVCC_DEVICE_GUARD(stream);
-    if (!f_map || !workspace || !gram || !isw_shape_ok(batch, c, hw)) return DGVCC_ERR_ARG;
-    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
-    const IswWs w = carve(workspace, batch, c, hw);
-    return launch_gram(f_map, nullptr, 1.0f, 0.f, batch, c, hw, use_tensor_cores, w, gram, (cudaStream_t)stream);
+    return ::gram<float>(f_map, batch, c, hw, use_tensor_cores, workspace, workspace_bytes, gram, stream);
+}
+
+extern "C" int dgvcc_isw_gram_h(const void* f_map, int dtype, int batch, int c, int hw, void* workspace,
+                                size_t workspace_bytes, float* gram, void* stream) {
+    DGVCC_DEVICE_GUARD(stream);
+    DGVCC_BY_HALF_DTYPE(dtype, return ::gram<T>(f_map, batch, c, hw, 1, workspace, workspace_bytes, gram, stream););
 }
 
 static int launch_triu_sq(const float* g, int c, int ld, int col0, size_t sample_stride, int batch, float scale,
@@ -1034,7 +1027,7 @@ extern "C" int dgvcc_lw_loss_backward(const float* y, const float* gram, const f
     cudaStream_t st = (cudaStream_t)stream;
     lw_grad_s_kernel<<<dim3(ceil_div(c * c, 256), batch), 256, 0, st>>>(gram, grad_loss, c, w.s);
     DGVCC_RETURN_IF_CUDA(cudaGetLastError());
-    return launch_sx(w.s, y, batch, c, hw, use_tensor_cores, grad_y, st);
+    return launch_sx<float>(w.s, y, batch, c, hw, use_tensor_cores, grad_y, st);
 }
 
 // z = [x; y] stacked [2c, p]; gram_zz [2c, 2c] = z z^T from dgvcc_isw_gram(z, 1, 2c, p, ...).
@@ -1047,124 +1040,87 @@ extern "C" int dgvcc_ortho_loss_forward(const float* gram_zz, int c, int p, void
     return launch_triu_sq(gram_zz, c, 2 * c, c, 0, 1, 1.0f / ((float)c * (float)c), w, loss_out, (cudaStream_t)stream);
 }
 
-extern "C" int dgvcc_ortho_loss_backward(const float* x, const float* y, const float* gram_zz, const float* grad_loss, int c,
-                                         int p, int use_tensor_cores, void* workspace, size_t workspace_bytes,
-                                         float* grad_x, float* grad_y, void* stream) {
-    DGVCC_DEVICE_GUARD(stream);
+// x, y, grad_x, grad_y [c, p] of type T; gram_zz from the Gram of z = [x; y].
+template <typename T>
+static int ortho_loss_backward(const void* x, const void* y, const float* gram_zz, const float* grad_loss, int c, int p,
+                               int use_tensor_cores, void* workspace, size_t workspace_bytes, void* grad_x, void* grad_y,
+                               void* stream) {
     if (!x || !y || !gram_zz || !grad_loss || !workspace || !grad_x || !grad_y || c > 16384 || !isw_shape_ok(1, 2 * c, p)) return DGVCC_ERR_ARG;
     if (workspace_bytes < dgvcc_isw_workspace_bytes(1, 2 * c, p)) return DGVCC_ERR_WORKSPACE;
+    if (half_untiled<T>(x, grad_x, c, p) || half_untiled<T>(y, grad_y, c, p)) return DGVCC_ERR_UNSUPPORTED;
     const IswWs w = carve(workspace, 1, 2 * c, p);  // S region holds (2c)^2 floats: Sx and Sy fit
     cudaStream_t st = (cudaStream_t)stream;
     float* sx = w.s;
     float* sy = w.s + (size_t)c * c;
     ortho_grad_s_kernel<<<ceil_div(c * c, 256), 256, 0, st>>>(gram_zz, grad_loss, c, sx, sy);
     DGVCC_RETURN_IF_CUDA(cudaGetLastError());
-    const int rc = launch_sx(sx, y, 1, c, p, use_tensor_cores, grad_x, st);
+    const int rc = launch_sx<T>(sx, y, 1, c, p, use_tensor_cores, grad_x, st);
     if (rc != DGVCC_OK) return rc;
-    return launch_sx(sy, x, 1, c, p, use_tensor_cores, grad_y, st);
+    return launch_sx<T>(sy, x, 1, c, p, use_tensor_cores, grad_y, st);
 }
 
-// ------------------------------------------------------- auxiliary Gram losses: half-precision entry points
-// Everything below returns what the fp32 entry points above return on the map upcast to fp32 (DESIGN section 5b); the
-// Gram and dX = S X run on the tensor cores only, under the shape rule half_tc_tiles.
-
-// The tensor-core partials (Gram of the half map, or of lw's standardised map) finished as X X^T: no scaling, no eps.
-static int finish_gram(int batch, int c, int tile, int n_tiles, int splits, const IswWs& w, float* gram, cudaStream_t st) {
-    const int yblocks = (tile / 32) * (tile / 32);
-    isw_cov_finish_kernel<<<dim3(n_tiles, yblocks, batch), 256, 0, st>>>(w.part, c, 1.0f, splits, tile, nullptr, 0.f, gram);
-    return (int)cudaGetLastError();
-}
-
-extern "C" int dgvcc_isw_gram_h(const void* f_map, int dtype, int batch, int c, int hw, void* workspace,
-                                size_t workspace_bytes, float* gram, void* stream) {
+extern "C" int dgvcc_ortho_loss_backward(const float* x, const float* y, const float* gram_zz, const float* grad_loss, int c,
+                                         int p, int use_tensor_cores, void* workspace, size_t workspace_bytes,
+                                         float* grad_x, float* grad_y, void* stream) {
     DGVCC_DEVICE_GUARD(stream);
-    if (!f_map || !workspace || !gram || !isw_shape_ok(batch, c, hw) || !half_dtype(dtype)) return DGVCC_ERR_ARG;
-    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
-    if (!half_tc_tiles(f_map, f_map, c, hw)) return DGVCC_ERR_UNSUPPORTED;
-    const IswWs w = carve(workspace, batch, c, hw);
-    cudaStream_t st = (cudaStream_t)stream;
-    int splits, kps, n_tiles, tile;
-    gram_plan_tc(batch, c, hw, &splits, &kps, &n_tiles, &tile);
-    const int rc = dgvcc::isw_tc::launch_half(f_map, dtype, batch, c, hw, splits, kps, w.part, (void*)st);
-    if (rc != DGVCC_OK) return rc;
-    return finish_gram(batch, c, tile, n_tiles, splits, w, gram, st);
+    return ortho_loss_backward<float>(x, y, gram_zz, grad_loss, c, p, use_tensor_cores, workspace, workspace_bytes, grad_x,
+                                      grad_y, stream);
 }
 
-// x, y, grad_x, grad_y [c, p] half; gram_zz from dgvcc_isw_gram_h on z = [x; y].
 extern "C" int dgvcc_ortho_loss_backward_h(const void* x, const void* y, int dtype, const float* gram_zz,
                                            const float* grad_loss, int c, int p, void* workspace, size_t workspace_bytes,
                                            void* grad_x, void* grad_y, void* stream) {
     DGVCC_DEVICE_GUARD(stream);
-    if (!x || !y || !gram_zz || !grad_loss || !workspace || !grad_x || !grad_y || c > 16384 || !isw_shape_ok(1, 2 * c, p) ||
-        !half_dtype(dtype))
-        return DGVCC_ERR_ARG;
-    if (workspace_bytes < dgvcc_isw_workspace_bytes(1, 2 * c, p)) return DGVCC_ERR_WORKSPACE;
-    if (!half_tc_tiles(x, grad_x, c, p) || !half_tc_tiles(y, grad_y, c, p)) return DGVCC_ERR_UNSUPPORTED;
-    const IswWs w = carve(workspace, 1, 2 * c, p);
-    cudaStream_t st = (cudaStream_t)stream;
-    float* sx = w.s;
-    float* sy = w.s + (size_t)c * c;
-    ortho_grad_s_kernel<<<ceil_div(c * c, 256), 256, 0, st>>>(gram_zz, grad_loss, c, sx, sy);
-    DGVCC_RETURN_IF_CUDA(cudaGetLastError());
-    const int rc = dgvcc::isw_sx::launch_half(sx, y, dtype, 1, c, p, grad_x, nullptr, false, (void*)st);
-    if (rc != DGVCC_OK) return rc;
-    return dgvcc::isw_sx::launch_half(sy, x, dtype, 1, c, p, grad_y, nullptr, false, (void*)st);
+    DGVCC_BY_HALF_DTYPE(dtype, return ortho_loss_backward<T>(x, y, gram_zz, grad_loss, c, p, 1, workspace, workspace_bytes,
+                                                             grad_x, grad_y, stream););
 }
+
+// ------------------------------------------------------- auxiliary Gram losses: half-precision entry points
+// lw_loss on a half map, the standardised map never materialised: the values of the fp32 entry points above on the map
+// upcast to fp32 (DESIGN section 5b); the Gram and dY = S Y run on the tensor cores only, under half_tc_tiles.
 
 extern "C" int dgvcc_lw_standardize_stats_h(const void* x, int dtype, int batch, int c, int hw, float eps, float* mean,
                                             float* sd, float* invstd, void* stream) {
     DGVCC_DEVICE_GUARD(stream);
-    if (!x || !mean || !sd || !invstd || !isw_shape_ok(batch, c, hw) || !half_dtype(dtype)) return DGVCC_ERR_ARG;
-    if (dtype == DGVCC_DTYPE_F16)
-        lw_standardize_fwd_kernel<__half, true><<<batch * c, NORM_THREADS, 0, (cudaStream_t)stream>>>(
-            (const __half*)x, nullptr, c, hw, eps, nullptr, nullptr, invstd, mean, sd);
-    else
-        lw_standardize_fwd_kernel<__nv_bfloat16, true><<<batch * c, NORM_THREADS, 0, (cudaStream_t)stream>>>(
-            (const __nv_bfloat16*)x, nullptr, c, hw, eps, nullptr, nullptr, invstd, mean, sd);
+    if (!x || !mean || !sd || !invstd || !isw_shape_ok(batch, c, hw)) return DGVCC_ERR_ARG;
+    DGVCC_BY_HALF_DTYPE(dtype, lw_standardize_fwd_kernel<T, true><<<batch * c, NORM_THREADS, 0, (cudaStream_t)stream>>>(
+                                   (const T*)x, nullptr, c, hw, eps, nullptr, nullptr, invstd, mean, sd););
     return (int)cudaGetLastError();
 }
 
 extern "C" int dgvcc_lw_gram_h(const void* x, int dtype, const float* mean, const float* sd, const float* mask, int batch,
                                int c, int hw, void* workspace, size_t workspace_bytes, float* gram, void* stream) {
     DGVCC_DEVICE_GUARD(stream);
-    if (!x || !mean || !sd || !workspace || !gram || !isw_shape_ok(batch, c, hw) || !half_dtype(dtype)) return DGVCC_ERR_ARG;
-    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
-    if (!half_tc_tiles(x, x, c, hw)) return DGVCC_ERR_UNSUPPORTED;
-    const IswWs w = carve(workspace, batch, c, hw);
-    cudaStream_t st = (cudaStream_t)stream;
-    int splits, kps, n_tiles, tile;
-    gram_plan_tc(batch, c, hw, &splits, &kps, &n_tiles, &tile);
-    const int rc = dgvcc::isw_tc::launch_std(x, dtype, mean, sd, mask, batch, c, hw, splits, kps, w.part, (void*)st);
-    if (rc != DGVCC_OK) return rc;
-    return finish_gram(batch, c, tile, n_tiles, splits, w, gram, st);
+    if (!x || !mean || !sd || !workspace || !gram || !isw_shape_ok(batch, c, hw)) return DGVCC_ERR_ARG;
+    DGVCC_BY_HALF_DTYPE(dtype, {
+        if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
+        return launch_gram<T, true>((const T*)x, mean, sd, mask, nullptr, 1.0f, 0.f, batch, c, hw, 1,
+                                    carve(workspace, batch, c, hw), gram, (cudaStream_t)stream);
+    });
 }
 
 extern "C" int dgvcc_lw_loss_backward_h(const void* x, int dtype, const float* mean, const float* sd, const float* mask,
                                         const float* gram, const float* grad_loss, int batch, int c, int hw, void* workspace,
                                         size_t workspace_bytes, float* grad_y, void* stream) {
     DGVCC_DEVICE_GUARD(stream);
-    if (!x || !mean || !sd || !gram || !grad_loss || !workspace || !grad_y || !isw_shape_ok(batch, c, hw) ||
-        !half_dtype(dtype))
-        return DGVCC_ERR_ARG;
-    if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
-    if (!half_tc_tiles(x, grad_y, c, hw)) return DGVCC_ERR_UNSUPPORTED;
-    const IswWs w = carve(workspace, batch, c, hw);
-    cudaStream_t st = (cudaStream_t)stream;
-    lw_grad_s_kernel<<<dim3(ceil_div(c * c, 256), batch), 256, 0, st>>>(gram, grad_loss, c, w.s);
-    DGVCC_RETURN_IF_CUDA(cudaGetLastError());
-    return dgvcc::isw_sx::launch_std(w.s, x, dtype, mean, sd, mask, batch, c, hw, grad_y, (void*)st);
+    if (!x || !mean || !sd || !gram || !grad_loss || !workspace || !grad_y || !isw_shape_ok(batch, c, hw)) return DGVCC_ERR_ARG;
+    DGVCC_BY_HALF_DTYPE(dtype, {
+        if (workspace_bytes < dgvcc_isw_workspace_bytes(batch, c, hw)) return DGVCC_ERR_WORKSPACE;
+        if (half_untiled<T>(x, grad_y, c, hw)) return DGVCC_ERR_UNSUPPORTED;
+        const IswWs w = carve(workspace, batch, c, hw);
+        cudaStream_t st = (cudaStream_t)stream;
+        lw_grad_s_kernel<<<dim3(ceil_div(c * c, 256), batch), 256, 0, st>>>(gram, grad_loss, c, w.s);
+        DGVCC_RETURN_IF_CUDA(cudaGetLastError());
+        return isw_sx::launch<T, true>(w.s, (const T*)x, mean, sd, mask, batch, c, hw, grad_y, nullptr, false, st);
+    });
 }
 
 extern "C" int dgvcc_lw_standardize_backward_h(const float* dy, const void* x, int dtype, const float* mean, const float* sd,
                                                const float* invstd, const float* mask, int batch, int c, int hw, void* dx,
                                                void* stream) {
     DGVCC_DEVICE_GUARD(stream);
-    if (!dy || !x || !mean || !sd || !invstd || !dx || !isw_shape_ok(batch, c, hw) || !half_dtype(dtype)) return DGVCC_ERR_ARG;
-    if (dtype == DGVCC_DTYPE_F16)
-        lw_standardize_bwd_half_kernel<<<batch * c, NORM_THREADS, 0, (cudaStream_t)stream>>>(
-            dy, (const __half*)x, mean, sd, invstd, mask, c, hw, (__half*)dx);
-    else
-        lw_standardize_bwd_half_kernel<<<batch * c, NORM_THREADS, 0, (cudaStream_t)stream>>>(
-            dy, (const __nv_bfloat16*)x, mean, sd, invstd, mask, c, hw, (__nv_bfloat16*)dx);
+    if (!dy || !x || !mean || !sd || !invstd || !dx || !isw_shape_ok(batch, c, hw)) return DGVCC_ERR_ARG;
+    DGVCC_BY_HALF_DTYPE(dtype, lw_standardize_bwd_half_kernel<<<batch * c, NORM_THREADS, 0, (cudaStream_t)stream>>>(
+                                   dy, (const T*)x, mean, sd, invstd, mask, c, hw, (T*)dx););
     return (int)cudaGetLastError();
 }

@@ -32,6 +32,7 @@
 // 0, what TMA zero-fills there for the fp32 kernel, without reading statistics or mask.
 #include <type_traits>
 
+#include "isw_tc.cuh"
 #include "tc_common.cuh"
 #include "../../include/dgvcc_b200.h"
 
@@ -61,13 +62,6 @@ template <bool EXACT, typename T = float, bool STD = false> struct Cfg {
 constexpr int B_BOX_BYTES = 32 * BLOCK_K * 4;   // one 32(n) x 32(k) box = 4 KB
 
 constexpr uint32_t IDESC = umma_idesc_tf32(TILE, TILE, /*b_mn_major=*/true);
-
-int launch(const float* s, const float* x, int batch, int c, int hw, float* dx, const float* scale, bool a_is_tf32_exact,
-           void* stream);
-int launch_half(const float* s, const void* x, int dtype, int batch, int c, int hw, void* dx, const float* scale,
-                bool a_is_tf32_exact, void* stream);
-int launch_std(const float* s, const void* x, int dtype, const float* mean, const float* sd, const float* mask, int batch,
-               int c, int hw, float* dy, void* stream);
 
 struct Args {
     int c, hw;
@@ -348,106 +342,58 @@ isw_sx_tc_kernel(const __grid_constant__ CUtensorMap map_s, const __grid_constan
 using namespace dgvcc;
 using namespace dgvcc::isw_sx;
 
-// dX_b = scale_b * (S_b X_b); a_is_tf32_exact selects the EXACT variant.  Returns DGVCC_ERR_UNSUPPORTED for shapes
-// TMA cannot tile.
-int dgvcc::isw_sx::launch(const float* s, const float* x, int batch, int c, int hw, float* dx, const float* scale,
-                          bool a_is_tf32_exact, void* stream) {
-    if (!s || !x || !dx || batch <= 0 || c <= 0 || hw <= 0) return DGVCC_ERR_ARG;
-    // TMA: 16-byte global strides and bases; tiny channel counts waste the 128-wide tile
-    if (hw % 4 != 0 || c % 4 != 0 || c < 32 || ((uintptr_t)s & 15u) || ((uintptr_t)x & 15u) || ((uintptr_t)dx & 15u))
-        return DGVCC_ERR_UNSUPPORTED;
+// fp32 X: four 32(n) x 32(k) boxes per k block in the SWIZZLE_128B_BASE32B layout.  Half X: one raw 32(k) x 128(n) box,
+// which the converters widen.
+template <typename T, bool STD>
+int dgvcc::isw_sx::launch(const float* s, const T* x, const float* mean, const float* sd, const float* mask, int batch, int c,
+                          int hw, void* dx, const float* scale, bool exact, cudaStream_t stream) {
+    constexpr bool HALF = Cfg<false, T, STD>::HALF;
+    if (!(HALF ? half_tc_tiles(c, hw) : sx_tc_tiles(c, hw)) || !tma_aligned(s, x, dx)) return DGVCC_ERR_UNSUPPORTED;
     CUtensorMap map_s, map_x;
     if (!make_tmap_f32_3d(&map_s, s, (uint64_t)c, (uint64_t)c, (uint64_t)batch, TILE)) return DGVCC_ERR_UNSUPPORTED;
-    if (!make_tmap_f32_3d(&map_x, x, (uint64_t)hw, (uint64_t)c, (uint64_t)batch, BLOCK_K, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B))
-        return DGVCC_ERR_UNSUPPORTED;
+    bool mapped;
+    if constexpr (HALF)
+        mapped = make_tmap_3d(&map_x, HalfIn<T>::TMA, 2, x, (uint64_t)hw, (uint64_t)c, (uint64_t)batch, TILE, BLOCK_K,
+                              CU_TENSOR_MAP_SWIZZLE_NONE, 1);
+    else
+        mapped = make_tmap_f32_3d(&map_x, x, (uint64_t)hw, (uint64_t)c, (uint64_t)batch, BLOCK_K,
+                                  CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
+    if (!mapped) return DGVCC_ERR_UNSUPPORTED;
     static PerDeviceOnce once;
     if (once.first()) {
-        DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_sx_tc_kernel<false, float>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                  Cfg<false>::SMEM_BYTES));
-        DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_sx_tc_kernel<true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                  Cfg<true>::SMEM_BYTES));
+        DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_sx_tc_kernel<false, T, STD>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                  Cfg<false, T, STD>::SMEM_BYTES));
+        if constexpr (!STD)  // STD has no EXACT variant
+            DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_sx_tc_kernel<true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                      Cfg<true, T>::SMEM_BYTES));
     }
     Args a;
     a.c = c; a.hw = hw; a.dx = dx; a.scale = scale;
-    const dim3 grid(ceil_div(hw, TILE), ceil_div(c, TILE), batch);
-    if (a_is_tf32_exact)
-        isw_sx_tc_kernel<true, float><<<grid, THREADS, Cfg<true>::SMEM_BYTES, (cudaStream_t)stream>>>(map_s, map_x, a);
-    else
-        isw_sx_tc_kernel<false, float><<<grid, THREADS, Cfg<false>::SMEM_BYTES, (cudaStream_t)stream>>>(map_s, map_x, a);
-    return (int)cudaGetLastError();
-}
-
-template <typename T>
-static int sx_tc_half(const float* s, const void* x, int batch, int c, int hw, void* dx, const float* scale, bool exact,
-                      void* stream) {
-    CUtensorMap map_s, map_x;
-    if (!make_tmap_f32_3d(&map_s, s, (uint64_t)c, (uint64_t)c, (uint64_t)batch, TILE)) return DGVCC_ERR_UNSUPPORTED;
-    if (!make_tmap_3d(&map_x, HalfIn<T>::TMA, 2, x, (uint64_t)hw, (uint64_t)c, (uint64_t)batch, TILE, BLOCK_K,
-                      CU_TENSOR_MAP_SWIZZLE_NONE, 1))
-        return DGVCC_ERR_UNSUPPORTED;
-    static PerDeviceOnce once;
-    if (once.first()) {
-        DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_sx_tc_kernel<false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                  Cfg<false, T>::SMEM_BYTES));
-        DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_sx_tc_kernel<true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                  Cfg<true, T>::SMEM_BYTES));
-    }
-    Args a;
-    a.c = c; a.hw = hw; a.dx = dx; a.scale = scale;
-    const dim3 grid(ceil_div(hw, TILE), ceil_div(c, TILE), batch);
-    if (exact)
-        isw_sx_tc_kernel<true, T><<<grid, THREADS, Cfg<true, T>::SMEM_BYTES, (cudaStream_t)stream>>>(map_s, map_x, a);
-    else
-        isw_sx_tc_kernel<false, T><<<grid, THREADS, Cfg<false, T>::SMEM_BYTES, (cudaStream_t)stream>>>(map_s, map_x, a);
-    return (int)cudaGetLastError();
-}
-
-template <typename T>
-static int sx_tc_std(const float* s, const void* x, const float* mean, const float* sd, const float* mask, int batch, int c,
-                     int hw, float* dy, void* stream) {
-    CUtensorMap map_s, map_x;
-    if (!make_tmap_f32_3d(&map_s, s, (uint64_t)c, (uint64_t)c, (uint64_t)batch, TILE)) return DGVCC_ERR_UNSUPPORTED;
-    if (!make_tmap_3d(&map_x, HalfIn<T>::TMA, 2, x, (uint64_t)hw, (uint64_t)c, (uint64_t)batch, TILE, BLOCK_K,
-                      CU_TENSOR_MAP_SWIZZLE_NONE, 1))
-        return DGVCC_ERR_UNSUPPORTED;
-    static PerDeviceOnce once;
-    if (once.first())
-        DGVCC_RETURN_IF_CUDA(cudaFuncSetAttribute(isw_sx_tc_kernel<false, T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                  Cfg<false, T, true>::SMEM_BYTES));
-    Args a;
-    a.c = c; a.hw = hw; a.dx = dy; a.scale = nullptr;
     a.mean = mean; a.sd = sd; a.mask = mask;
     const dim3 grid(ceil_div(hw, TILE), ceil_div(c, TILE), batch);
-    isw_sx_tc_kernel<false, T, true><<<grid, THREADS, Cfg<false, T, true>::SMEM_BYTES, (cudaStream_t)stream>>>(map_s, map_x, a);
+    if constexpr (!STD) {
+        if (exact) {
+            isw_sx_tc_kernel<true, T><<<grid, THREADS, Cfg<true, T>::SMEM_BYTES, stream>>>(map_s, map_x, a);
+            return (int)cudaGetLastError();
+        }
+    }
+    isw_sx_tc_kernel<false, T, STD><<<grid, THREADS, Cfg<false, T, STD>::SMEM_BYTES, stream>>>(map_s, map_x, a);
     return (int)cudaGetLastError();
 }
 
-// dY_b = S_b Y_b in fp32 with Y = (X - mean) / sd (* mask) standardised on load from the half-precision X, Y never
-// materialised: the same bits as dgvcc_isw_sx_tc on Y.  mean, sd [batch * c]; mask [batch, hw] or NULL.  Same shape rule
-// as launch_half, and a 16-byte aligned dY.
-int dgvcc::isw_sx::launch_std(const float* s, const void* x, int dtype, const float* mean, const float* sd, const float* mask,
-                              int batch, int c, int hw, float* dy, void* stream) {
-    if (!s || !x || !mean || !sd || !dy || batch <= 0 || c <= 0 || hw <= 0) return DGVCC_ERR_ARG;
-    if (dtype != DGVCC_DTYPE_F16 && dtype != DGVCC_DTYPE_BF16) return DGVCC_ERR_ARG;
-    if (hw % 8 != 0 || c % 4 != 0 || c < 32 || ((uintptr_t)s & 15u) || ((uintptr_t)x & 15u) || ((uintptr_t)dy & 15u))
-        return DGVCC_ERR_UNSUPPORTED;
-    return dtype == DGVCC_DTYPE_F16 ? sx_tc_std<__half>(s, x, mean, sd, mask, batch, c, hw, dy, stream)
-                                    : sx_tc_std<__nv_bfloat16>(s, x, mean, sd, mask, batch, c, hw, dy, stream);
-}
-
-// dX_b = scale_b * (S_b X_b) for a half-precision X and dX (dtype DGVCC_DTYPE_F16 / _BF16), S in fp32.  TMA needs
-// hw % 8 == 0 (16-byte row strides of X) and 16-byte aligned bases.
-int dgvcc::isw_sx::launch_half(const float* s, const void* x, int dtype, int batch, int c, int hw, void* dx,
-                               const float* scale, bool a_is_tf32_exact, void* stream) {
-    if (!s || !x || !dx || batch <= 0 || c <= 0 || hw <= 0) return DGVCC_ERR_ARG;
-    if (dtype != DGVCC_DTYPE_F16 && dtype != DGVCC_DTYPE_BF16) return DGVCC_ERR_ARG;
-    if (hw % 8 != 0 || c % 4 != 0 || c < 32 || ((uintptr_t)s & 15u) || ((uintptr_t)x & 15u) || ((uintptr_t)dx & 15u))
-        return DGVCC_ERR_UNSUPPORTED;
-    return dtype == DGVCC_DTYPE_F16 ? sx_tc_half<__half>(s, x, batch, c, hw, dx, scale, a_is_tf32_exact, stream)
-                                    : sx_tc_half<__nv_bfloat16>(s, x, batch, c, hw, dx, scale, a_is_tf32_exact, stream);
-}
+template int dgvcc::isw_sx::launch<float, false>(const float*, const float*, const float*, const float*, const float*, int, int,
+                                                 int, void*, const float*, bool, cudaStream_t);
+template int dgvcc::isw_sx::launch<__half, true>(const float*, const __half*, const float*, const float*, const float*, int, int,
+                                                 int, void*, const float*, bool, cudaStream_t);
+template int dgvcc::isw_sx::launch<__nv_bfloat16, true>(const float*, const __nv_bfloat16*, const float*, const float*,
+                                                        const float*, int, int, int, void*, const float*, bool, cudaStream_t);
+template int dgvcc::isw_sx::launch<__half, false>(const float*, const __half*, const float*, const float*, const float*, int,
+                                                  int, int, void*, const float*, bool, cudaStream_t);
+template int dgvcc::isw_sx::launch<__nv_bfloat16, false>(const float*, const __nv_bfloat16*, const float*, const float*,
+                                                         const float*, int, int, int, void*, const float*, bool, cudaStream_t);
 
 extern "C" int dgvcc_isw_sx_tc(const float* s, const float* x, int batch, int c, int hw, float* dx, void* stream) {
     DGVCC_DEVICE_GUARD(stream);
-    return dgvcc::isw_sx::launch(s, x, batch, c, hw, dx, nullptr, false, stream);
+    if (!s || !x || !dx || batch <= 0 || c <= 0 || hw <= 0) return DGVCC_ERR_ARG;
+    return launch(s, x, nullptr, nullptr, nullptr, batch, c, hw, dx, nullptr, false, (cudaStream_t)stream);
 }

@@ -13,19 +13,9 @@ load it, and the standardisation backward recomputes it from x.  Loss and gradie
 the Gram and the workspace.  Shapes the half tensor-core kernels do not tile (HW % 8 != 0, C < 32, C % 4 != 0, a
 misaligned view) and ``DGVCC_ISW_TENSOR_CORES=0`` take the upcast route; the forward's choice holds for its backward.
 """
-import os
-
 import torch
 
 from .. import _native
-
-
-def _use_tc():
-    return int(os.environ.get("DGVCC_ISW_TENSOR_CORES", "1"))
-
-
-_HALF = {torch.float16: _native.DTYPE_F16, torch.bfloat16: _native.DTYPE_BF16}
-_UNSUPPORTED = -3  # DGVCC_ERR_UNSUPPORTED
 
 
 def _forward_half(ctx, x, m, dt):
@@ -45,7 +35,7 @@ def _forward_half(ctx, x, m, dt):
     gram = torch.empty((n, c, c), dtype=torch.float32, device=dev)
     rc = lib.dgvcc_lw_gram_h(_native.ptr(xh), dt, _native.ptr(mean), _native.ptr(sd), _native.ptr(m), n, c, hw,
                              _native.ptr(ws), nbytes, _native.ptr(gram), stream)
-    if rc == _UNSUPPORTED:
+    if rc == _native.ERR_UNSUPPORTED:
         return None
     _native.check(rc, "dgvcc_lw_gram_h")
     loss = torch.empty((1,), dtype=torch.float32, device=dev)
@@ -91,8 +81,8 @@ class _LwLoss(torch.autograd.Function):
         if mask is not None:
             m = mask.detach().to(device=dev, dtype=torch.float32).reshape(n, hw).contiguous()
         ctx.half = None
-        dt = _HALF.get(x.dtype)
-        if dt is not None and _use_tc():
+        dt = _native.half_code(x.dtype)
+        if dt is not None and _native.use_tensor_cores():
             loss = _forward_half(ctx, x, m, dt)
             if loss is not None:
                 return loss
@@ -107,8 +97,8 @@ class _LwLoss(torch.autograd.Function):
         nbytes = lib.dgvcc_isw_workspace_bytes(n, c, hw)
         ws = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
         gram = torch.empty((n, c, c), dtype=torch.float32, device=dev)
-        _native.check(lib.dgvcc_isw_gram(_native.ptr(y), n, c, hw, _use_tc(), _native.ptr(ws), nbytes, _native.ptr(gram),
-                                         stream), "dgvcc_isw_gram")
+        _native.check(lib.dgvcc_isw_gram(_native.ptr(y), n, c, hw, _native.use_tensor_cores(), _native.ptr(ws), nbytes,
+                                         _native.ptr(gram), stream), "dgvcc_isw_gram")
         loss = torch.empty((1,), dtype=torch.float32, device=dev)
         _native.check(lib.dgvcc_lw_loss_forward(_native.ptr(gram), n, c, hw, _native.ptr(ws), nbytes, _native.ptr(loss),
                                                 stream), "dgvcc_lw_loss_forward")
@@ -129,8 +119,9 @@ class _LwLoss(torch.autograd.Function):
         stream = _native.stream_ptr(dev)
         g = grad_loss.detach().to(device=dev, dtype=torch.float32).reshape(1).contiguous()
         dy = torch.empty_like(yhat)
-        _native.check(lib.dgvcc_lw_loss_backward(_native.ptr(y), _native.ptr(gram), _native.ptr(g), n, c, hw, _use_tc(),
-                                                 _native.ptr(ws), nbytes, _native.ptr(dy), stream),
+        _native.check(lib.dgvcc_lw_loss_backward(_native.ptr(y), _native.ptr(gram), _native.ptr(g), n, c, hw,
+                                                 _native.use_tensor_cores(), _native.ptr(ws), nbytes, _native.ptr(dy),
+                                                 stream),
                       "dgvcc_lw_loss_backward")
         dx = torch.empty_like(yhat)
         _native.check(lib.dgvcc_lw_standardize_backward(_native.ptr(dy), _native.ptr(yhat), _native.ptr(invstd),

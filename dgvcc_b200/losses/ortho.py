@@ -11,19 +11,9 @@ route on the upcast inputs bit for bit (gradients rounded to the input dtype).  
 not tile (P % 8 != 0, C < 32, C % 4 != 0) and ``DGVCC_ISW_TENSOR_CORES=0`` take the upcast route; the forward's choice
 holds for its backward.
 """
-import os
-
 import torch
 
 from .. import _native
-
-
-def _use_tc():
-    return int(os.environ.get("DGVCC_ISW_TENSOR_CORES", "1"))
-
-
-_HALF = {torch.float16: _native.DTYPE_F16, torch.bfloat16: _native.DTYPE_BF16}
-_UNSUPPORTED = -3  # DGVCC_ERR_UNSUPPORTED
 
 
 class _OrthoLoss(torch.autograd.Function):
@@ -41,19 +31,21 @@ class _OrthoLoss(torch.autograd.Function):
         ws = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
         gram = torch.empty((2 * c, 2 * c), dtype=torch.float32, device=dev)
         # the Gram tiles [x; y] (2C rows); the two dX GEMMs need C >= 32 and C % 4 == 0 themselves
-        ctx.half = _HALF.get(x.dtype) if x.dtype == y.dtype and c >= 32 and c % 4 == 0 and _use_tc() else None
+        ctx.half = None
+        if x.dtype == y.dtype and c >= 32 and c % 4 == 0 and _native.use_tensor_cores():
+            ctx.half = _native.half_code(x.dtype)
         if ctx.half is not None:
             z = torch.cat([x.detach(), y.detach()], dim=0).contiguous()  # [2C, P] in the input dtype
             rc = lib.dgvcc_isw_gram_h(_native.ptr(z), ctx.half, 1, 2 * c, p, _native.ptr(ws), nbytes, _native.ptr(gram),
                                       stream)
-            if rc == _UNSUPPORTED:
+            if rc == _native.ERR_UNSUPPORTED:
                 ctx.half = None
             else:
                 _native.check(rc, "dgvcc_isw_gram_h")
         if ctx.half is None:
             z = torch.cat([x.detach().to(torch.float32), y.detach().to(torch.float32)], dim=0).contiguous()  # [2C, P]
-            _native.check(lib.dgvcc_isw_gram(_native.ptr(z), 1, 2 * c, p, _use_tc(), _native.ptr(ws), nbytes,
-                                             _native.ptr(gram), stream), "dgvcc_isw_gram")
+            _native.check(lib.dgvcc_isw_gram(_native.ptr(z), 1, 2 * c, p, _native.use_tensor_cores(), _native.ptr(ws),
+                                             nbytes, _native.ptr(gram), stream), "dgvcc_isw_gram")
         loss = torch.empty((1,), dtype=torch.float32, device=dev)
         _native.check(lib.dgvcc_ortho_loss_forward(_native.ptr(gram), c, p, _native.ptr(ws), nbytes, _native.ptr(loss), stream),
                       "dgvcc_ortho_loss_forward")
@@ -77,8 +69,9 @@ class _OrthoLoss(torch.autograd.Function):
         gx = torch.empty((c, p), dtype=torch.float32, device=dev)
         gy = torch.empty((c, p), dtype=torch.float32, device=dev)
         _native.check(_native.lib().dgvcc_ortho_loss_backward(
-            _native.ptr(z[:c]), _native.ptr(z[c:]), _native.ptr(gram), _native.ptr(g), c, p, _use_tc(), _native.ptr(ws),
-            nbytes, _native.ptr(gx), _native.ptr(gy), _native.stream_ptr(dev)), "dgvcc_ortho_loss_backward")
+            _native.ptr(z[:c]), _native.ptr(z[c:]), _native.ptr(gram), _native.ptr(g), c, p, _native.use_tensor_cores(),
+            _native.ptr(ws), nbytes, _native.ptr(gx), _native.ptr(gy), _native.stream_ptr(dev)),
+            "dgvcc_ortho_loss_backward")
         return gx.to(xdt), gy.to(ydt)
 
 

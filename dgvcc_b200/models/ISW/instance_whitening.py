@@ -18,8 +18,6 @@ results are those of the fp32 path on the upcast map, bit for bit: y and the gra
 ``f_cor`` and the loss are fp32.  Shapes the half tensor-core kernels do not tile (HW % 8 != 0, C < 32, C % 4 != 0,
 a misaligned view) and ``DGVCC_ISW_TENSOR_CORES=0`` take the upcast route; the forward's choice holds for its backward.
 """
-import os
-
 import weakref
 
 import torch
@@ -28,38 +26,12 @@ import torch.nn as nn
 from ... import _native
 
 
-def _use_tc():
-    return int(os.environ.get("DGVCC_ISW_TENSOR_CORES", "1"))
-
-
 def _f32c(t, dev=None):
     """``t`` as a detached contiguous fp32 tensor (on ``dev``); no copy, and one call only, when it already is one."""
     if t.dtype is torch.float32 and t.is_contiguous() and (dev is None or t.device == dev):
         return t.detach()
     return t.detach().to(device=dev if dev is not None else t.device, dtype=torch.float32).contiguous()
 
-
-_HALF = {torch.float16: _native.DTYPE_F16, torch.bfloat16: _native.DTYPE_BF16}
-
-
-def _half3d(f_map):
-    """(dtype code, contiguous half [B,C,HW] view) when ``f_map`` is fp16 / bf16 and the tensor cores are on, else
-    (None, None): the caller then takes the fp32 route of ``_as3d``."""
-    dt = _HALF.get(f_map.dtype)
-    if dt is None or not _use_tc():
-        return None, None
-    _native.require_cuda(f_map, "instance_whitening")
-    b, c, h, w = f_map.shape
-    return dt, f_map.detach().contiguous().view(b, c, h * w)
-
-
-def _as3d(f_map):
-    _native.require_cuda(f_map, "instance_whitening")
-    b, c, h, w = f_map.shape
-    return _f32c(f_map).view(b, c, h * w), b, c, h * w
-
-
-_UNSUPPORTED = -3  # DGVCC_ERR_UNSUPPORTED
 
 _ws_bytes = {}
 
@@ -91,7 +63,7 @@ class _InstanceNorm(torch.autograd.Function):
     def forward(ctx, x, eps):
         _native.require_cuda(x, "InstanceWhitening")
         b, c, h, w = x.shape
-        ctx.half = _HALF.get(x.dtype)
+        ctx.half = _native.half_code(x.dtype)
         if ctx.half is not None:  # y = RN(fp32 y) in the input dtype; the backward recomputes fp32 y from x
             xc = x.detach().contiguous()
             y = torch.empty_like(xc)
@@ -147,32 +119,38 @@ class InstanceWhitening(nn.Module):
         return x, w
 
 
+def _covariance(f_map, eye):
+    """(f_cor [B,C,C] fp32, x, half dtype code or None, workspace, its bytes, stream).  x is the [B,C,HW] map the
+    covariance was computed from, which the backward needs: the half map itself when the half kernels take it, else the
+    fp32 upcast (other dtypes, a shape the half tensor-core kernels do not tile, DGVCC_ISW_TENSOR_CORES=0)."""
+    _native.require_cuda(f_map, "instance_whitening")
+    b, c, h, w = f_map.shape
+    hw = h * w
+    half = _native.half_code(f_map.dtype)
+    half = half if half is not None and _native.use_tensor_cores() else None
+    x = f_map.detach().contiguous().view(b, c, hw) if half is not None else _f32c(f_map).view(b, c, hw)
+    dev = x.device
+    lib = _native.lib()
+    ws, n = _workspace(b, c, hw, dev)
+    f_cor = torch.empty((b, c, c), dtype=torch.float32, device=dev)
+    eye32 = _f32c(eye, dev)
+    stream = _native.stream_ptr(dev)
+    if half is not None:
+        rc = lib.dgvcc_isw_covariance_h(_native.ptr(x), half, _native.ptr(eye32), b, c, hw, _native.ptr(ws), n,
+                                        _native.ptr(f_cor), stream)
+        if rc != _native.ERR_UNSUPPORTED:
+            _native.check(rc, "dgvcc_isw_covariance_h")
+            return f_cor, x, half, ws, n, stream
+        half, x = None, _f32c(f_map).view(b, c, hw)  # upcast, as for every other dtype
+    _native.check(lib.dgvcc_isw_covariance(_native.ptr(x), _native.ptr(eye32), b, c, hw, _native.use_tensor_cores(),
+                                           _native.ptr(ws), n, _native.ptr(f_cor), stream), "dgvcc_isw_covariance")
+    return f_cor, x, half, ws, n, stream
+
+
 class _Covariance(torch.autograd.Function):
     @staticmethod
     def forward(ctx, f_map, eye):
-        ctx.half, x = _half3d(f_map)
-        if ctx.half is not None:
-            b, c, hw = x.shape
-            dev = x.device
-            ws, n = _workspace(b, c, hw, dev)
-            f_cor = torch.empty((b, c, c), dtype=torch.float32, device=dev)
-            rc = _native.lib().dgvcc_isw_covariance_h(_native.ptr(x), ctx.half, _native.ptr(_f32c(eye, dev)), b, c, hw,
-                                                      _native.ptr(ws), n, _native.ptr(f_cor), _native.stream_ptr(dev))
-            if rc == _UNSUPPORTED:
-                ctx.half = None
-            else:
-                _native.check(rc, "dgvcc_isw_covariance_h")
-                ctx.save_for_backward(x)
-                ctx.meta = (f_map.shape, f_map.dtype)
-                return f_cor
-        x, b, c, hw = _as3d(f_map)
-        dev = x.device
-        ws, n = _workspace(b, c, hw, dev)
-        f_cor = torch.empty((b, c, c), dtype=torch.float32, device=dev)
-        eye32 = _f32c(eye, dev)
-        _native.check(_native.lib().dgvcc_isw_covariance(
-            _native.ptr(x), _native.ptr(eye32), b, c, hw, _use_tc(), _native.ptr(ws), n, _native.ptr(f_cor),
-            _native.stream_ptr(dev)), "dgvcc_isw_covariance")
+        f_cor, x, ctx.half, _, _, _ = _covariance(f_map, eye)
         ctx.save_for_backward(x)
         ctx.meta = (f_map.shape, f_map.dtype)
         return f_cor
@@ -191,7 +169,7 @@ class _Covariance(torch.autograd.Function):
                 _native.stream_ptr(dev)), "dgvcc_isw_covariance_backward_h")
             return dx.view(ctx.meta[0]), None
         _native.check(_native.lib().dgvcc_isw_covariance_backward(
-            _native.ptr(x), _native.ptr(g), b, c, hw, _use_tc(), _native.ptr(ws), n, _native.ptr(dx),
+            _native.ptr(x), _native.ptr(g), b, c, hw, _native.use_tensor_cores(), _native.ptr(ws), n, _native.ptr(dx),
             _native.stream_ptr(dev)), "dgvcc_isw_covariance_backward")
         shape, dtype = ctx.meta
         return dx.view(shape).to(dtype), None
@@ -215,32 +193,14 @@ def _mask_is_binary(mask):
 class _WhiteningLoss(torch.autograd.Function):
     @staticmethod
     def forward(ctx, f_map, eye, mask_matrix, margin, num_remove_cov):
-        ctx.half, x = _half3d(f_map)
-        if ctx.half is None:
-            x, b, c, hw = _as3d(f_map)
-        else:
-            b, c, hw = x.shape
+        f_cor, x, ctx.half, ws, n, stream = _covariance(f_map, eye)
+        b, c, hw = x.shape
         dev = x.device
         lib = _native.lib()
-        ws, n = _workspace(b, c, hw, dev)
-        f_cor = torch.empty((b, c, c), dtype=torch.float32, device=dev)
-        eye32 = _f32c(eye, dev)
         mask = _f32c(mask_matrix, dev)
         if mask.shape != (c, c):
             raise ValueError(f"mask_matrix must be [{c},{c}], got {tuple(mask.shape)}")
         mg, nr = _scalar(margin, dev), _scalar(num_remove_cov, dev)
-        stream = _native.stream_ptr(dev)
-        if ctx.half is not None:
-            rc = lib.dgvcc_isw_covariance_h(_native.ptr(x), ctx.half, _native.ptr(eye32), b, c, hw, _native.ptr(ws), n,
-                                            _native.ptr(f_cor), stream)
-            if rc == _UNSUPPORTED:  # a shape the half tensor-core kernels do not tile: upcast, as for every other dtype
-                ctx.half = None
-                x = _as3d(f_map)[0]
-            else:
-                _native.check(rc, "dgvcc_isw_covariance_h")
-        if ctx.half is None:
-            _native.check(lib.dgvcc_isw_covariance(_native.ptr(x), _native.ptr(eye32), b, c, hw, _use_tc(), _native.ptr(ws),
-                                                   n, _native.ptr(f_cor), stream), "dgvcc_isw_covariance")
         loss = torch.empty((1,), dtype=torch.float32, device=dev)
         _native.check(lib.dgvcc_isw_loss_forward(_native.ptr(f_cor), _native.ptr(mask), _native.ptr(mg), _native.ptr(nr),
                                                  b, c, hw, _native.ptr(ws), n, _native.ptr(loss), stream),
@@ -263,8 +223,9 @@ class _WhiteningLoss(torch.autograd.Function):
                 int(binary), _native.ptr(ws), n, _native.ptr(dx), _native.stream_ptr(dev)), "dgvcc_isw_loss_backward_h")
             return dx.view(shape), None, None, None, None
         _native.check(_native.lib().dgvcc_isw_loss_backward(
-            _native.ptr(x), _native.ptr(f_cor), _native.ptr(mask), _native.ptr(nr), _native.ptr(g), b, c, hw, _use_tc(),
-            int(binary), _native.ptr(ws), n, _native.ptr(dx), _native.stream_ptr(dev)), "dgvcc_isw_loss_backward")
+            _native.ptr(x), _native.ptr(f_cor), _native.ptr(mask), _native.ptr(nr), _native.ptr(g), b, c, hw,
+            _native.use_tensor_cores(), int(binary), _native.ptr(ws), n, _native.ptr(dx), _native.stream_ptr(dev)),
+            "dgvcc_isw_loss_backward")
         return dx.view(shape).to(dtype), None, None, None, None
 
 

@@ -83,12 +83,12 @@ def loss_vector(c, f_cor, mask):
 
 
 def sx_tc_tiles(c, hw, *tensors):
-    """sx_tc_tiles (isw_kernels.cu): dX = S X on the tensor cores."""
+    """sx_tc_tiles and tma_aligned (isw_tc.cuh): dX = S X on the tensor cores."""
     return hw % 4 == 0 and c % 4 == 0 and c >= 32 and all(t.data_ptr() % 16 == 0 for t in tensors)
 
 
 def half_tc_tiles(c, hw, *tensors):
-    """half_tc_tiles (isw_kernels.cu): the native fp16 / bf16 route."""
+    """half_tc_tiles and tma_aligned (isw_tc.cuh): the native fp16 / bf16 route."""
     return hw % 8 == 0 and c % 4 == 0 and c >= 32 and all(t.data_ptr() % 16 == 0 for t in tensors)
 
 
