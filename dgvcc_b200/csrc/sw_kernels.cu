@@ -4,7 +4,8 @@
 // (models/ISW/sync_switchwhiten.py:9-56,135-223).  The evaluation order is the one oracle/switchwhiten_oracle.py:
 // ``decomposed`` spells out:
 //
-//   forward   moments pass     one read of x: shifted sums and upper-triangular products per (sample, group)
+//   forward   moments pass     one read of x: sums and upper-triangular products per (sample, group), shifted by a
+//                              sample mean of the plane
 //             instance stats   mean_in, cov_in (fp64)
 //             batch mean/cov   from the per-sample statistics (the caller exchanges them between ranks)
 //             whiten matrices  softmax mix, T Newton iterations on cp x cp matrices in fp64, A = diag(weight) wm
@@ -126,7 +127,39 @@ __device__ __forceinline__ void warp_transpose_sum(const float (&acc)[NV], float
     }
 }
 
-// grid (splits, n * groups).  part[(ng * splits + split) * NV + k]: k < CP the shifted sums, then the upper triangle.
+// Floats per (sample, group, split) in the forward partials: the shifted sums, the upper triangle of the shifted
+// products, then the shift itself.
+template <int CP>
+__host__ __device__ constexpr int fwd_part_floats() { return CP + CP * (CP + 1) / 2 + CP; }
+
+// The shift the forward moments are centred on: the mean of up to 128 pixels of the plane, summed in a fixed order so
+// that every CTA of a plane computes the same bits.  Centring on a sample mean rather than on one pixel keeps the
+// shifted sums small when some pixels sit far from the plane mean (zero-padded corners of conv features):
+// S2 / hw - delta delta^T then cancels no digits.  The sample is 16 runs of 8 consecutive pixels starting at
+// (c hw) / 16, c = 0 .. 15 (every pixel when hw <= 128): a warp's load touches 4 to 8 sectors where 32 scattered
+// pixels touched 32, which measured 15 % of the moments kernel's time at the benchmark shapes.
+template <int CP>
+__device__ __forceinline__ void sample_shift(const float* base, int hw, float (&shift)[CP], float (*sred)[CP]) {
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int p = hw > MOM_THREADS ? (int)(((long long)(tid >> 3) * hw) / 16) + (tid & 7) : tid;
+    float v[CP], tot[1];
+#pragma unroll
+    for (int j = 0; j < CP; ++j) v[j] = p < hw ? __ldg(base + (size_t)j * hw + p) : 0.f;
+    warp_transpose_sum<CP>(v, tot);
+    if (lane < CP) sred[warp][lane] = tot[0];
+    __syncthreads();
+    const float inv = 1.f / (float)(hw < MOM_THREADS ? hw : MOM_THREADS);   // 2^-7 but on planes under 128 pixels
+#pragma unroll
+    for (int j = 0; j < CP; ++j) {
+        float s = 0.f;
+#pragma unroll
+        for (int w = 0; w < MOM_THREADS / 32; ++w) s += sred[w][j];
+        shift[j] = s * inv;
+    }
+}
+
+// grid (splits, n * groups).  part[(ng * splits + split) * fwd_part_floats<CP>() + k]: k < CP the shifted sums, then
+// the upper triangle, then the CP shifts (the same in every split of a plane).
 template <int CP>
 __global__ void __launch_bounds__(MOM_THREADS, 2)
 sw_moments_kernel(const float* __restrict__ x, int hw, int chunk, float* __restrict__ part) {
@@ -134,11 +167,10 @@ sw_moments_kernel(const float* __restrict__ x, int hw, int chunk, float* __restr
     extern __shared__ float ring_raw[];
     float (*ring)[CP][MOM_THREADS] = reinterpret_cast<float (*)[CP][MOM_THREADS]>(ring_raw);
     __shared__ float red[MOM_THREADS / 32][NV];
+    __shared__ float sred[MOM_THREADS / 32][CP];
     const float* base = x + (size_t)blockIdx.y * CP * hw;
     const int tid = threadIdx.x;
     float shift[CP], acc[NV];
-#pragma unroll
-    for (int j = 0; j < CP; ++j) shift[j] = __ldg(base + (size_t)j * hw);
 #pragma unroll
     for (int k = 0; k < NV; ++k) acc[k] = 0.f;
     const int p0 = blockIdx.x * chunk, p1 = min(hw, p0 + chunk);
@@ -152,6 +184,7 @@ sw_moments_kernel(const float* __restrict__ x, int hw, int chunk, float* __restr
         cp_async_commit();
     };
     for (int it = 0; it < FWD_STAGES - 1; ++it) issue(it);
+    sample_shift<CP>(base, hw, shift, sred);   // after the ring's first copies: their latencies overlap
     for (int it = 0; it < iters; ++it) {
         issue(it + FWD_STAGES - 1);       // its slot was read (into registers) one iteration ago
         cp_async_wait<FWD_STAGES - 1>();
@@ -174,36 +207,41 @@ sw_moments_kernel(const float* __restrict__ x, int hw, int chunk, float* __restr
     for (int g = 0; g < (NV + 31) / 32; ++g)
         if (g * 32 + lane < NV) red[warp][g * 32 + lane] = tot[g];
     __syncthreads();
-    float* out = part + ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * NV;
+    float* out = part + ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * fwd_part_floats<CP>();
     for (int k = tid; k < NV; k += MOM_THREADS) {
         float s = 0.f;
 #pragma unroll
         for (int w = 0; w < MOM_THREADS / 32; ++w) s += red[w][k];
         out[k] = s;
     }
+    if (tid < CP) {
+#pragma unroll
+        for (int j = 0; j < CP; ++j)
+            if (j == tid) out[NV + j] = shift[j];   // static register index: no local-memory copy of shift
+    }
 }
 
 // grid n * groups, 256 threads.
 template <int CP>
 __global__ void __launch_bounds__(MAT_THREADS)
-sw_instance_stats_kernel(const float* __restrict__ x, const float* __restrict__ part, int splits, int hw,
-                         double* __restrict__ mean_in, double* __restrict__ cov_in) {
-    constexpr int NV = CP + CP * (CP + 1) / 2;
+sw_instance_stats_kernel(const float* __restrict__ part, int splits, int hw, double* __restrict__ mean_in,
+                         double* __restrict__ cov_in) {
+    constexpr int NV = CP + CP * (CP + 1) / 2, NP = fwd_part_floats<CP>();
     __shared__ double delta[CP];
     const int ng = blockIdx.x, t = threadIdx.x;
-    const float* mine = part + (size_t)ng * splits * NV;
+    const float* mine = part + (size_t)ng * splits * NP;
     if (t < CP) {
         double s = 0.0;
-        for (int q = 0; q < splits; ++q) s += (double)mine[(size_t)q * NV + t];
+        for (int q = 0; q < splits; ++q) s += (double)mine[(size_t)q * NP + t];
         delta[t] = s / hw;
-        mean_in[(size_t)ng * CP + t] = (double)x[((size_t)ng * CP + t) * hw] + s / hw;
+        mean_in[(size_t)ng * CP + t] = (double)mine[NV + t] + s / hw;
     }
     __syncthreads();
     if (t < CP * CP) {
         const int i = t / CP, j = t % CP;
         const int k = CP + tri_index(CP, min(i, j), max(i, j));
         double s = 0.0;
-        for (int q = 0; q < splits; ++q) s += (double)mine[(size_t)q * NV + k];
+        for (int q = 0; q < splits; ++q) s += (double)mine[(size_t)q * NP + k];
         cov_in[(size_t)ng * CP * CP + t] = s / hw - delta[i] * delta[j];
     }
 }
@@ -496,7 +534,7 @@ __host__ inline int bwd_z(int cp) { return cp / (cp < BWD_ROWS ? cp : BWD_ROWS);
 
 __host__ inline BwdLayout layout(int n, int channels, int hw, int cp) {
     const size_t ng = (size_t)n * (channels / cp), mat = (size_t)cp * cp;
-    const size_t fwd_part = ng * plan_split((int)ng, hw, 1).splits * (cp + cp * (cp + 1) / 2) * sizeof(float);
+    const size_t fwd_part = ng * plan_split((int)ng, hw, 1).splits * (cp + cp * (cp + 1) / 2 + cp) * sizeof(float);
     const size_t bwd_part = ng * plan_split((int)ng, hw, bwd_z(cp)).splits * cp * (cp + 1) * sizeof(float);
     BwdLayout l;
     size_t o = 0;
@@ -820,7 +858,7 @@ extern "C" int dgvcc_sw_instance_stats(const float* x, int n, int channels, int 
     float* part = (float*)((char*)workspace + l.part);
 #define CALL(CP)                                                                                             \
     DGVCC_RETURN_IF_CUDA(launch_moments<CP>(x, ng, hw, sp, part, st));                                       \
-    sw_instance_stats_kernel<CP><<<ng, MAT_THREADS, 0, st>>>(x, part, sp.splits, hw, mean_in, cov_in)
+    sw_instance_stats_kernel<CP><<<ng, MAT_THREADS, 0, st>>>(part, sp.splits, hw, mean_in, cov_in)
     SW_DISPATCH(num_pergroup, CALL);
 #undef CALL
     DGVCC_RETURN_IF_CUDA(cudaGetLastError());

@@ -7,10 +7,10 @@ byte-identical copies live under models/SW/ops/) -- SURVEY.md section 8f, rank 4
 * ``forward``: the reference's op sequence in torch (any dtype), gradients by autograd, the batch statistics through a
   custom Function with SyncMeanCov's hand-written backward when a process group is given.  Pinned by
   tests/golden/sw_cases.npz, produced by the unmodified files loaded by path (tests/golden/make_golden.py: make_sw).
-* ``decomposed``: the same mathematics in the order the CUDA kernels evaluate it (shifted one-pass moments, batch
-  covariance from the per-sample ones, closed-form adjoint of the Newton iteration, the two affine passes), numpy
-  fp64, no autograd.  tests/test_oracle_sw.py checks it against ``forward``; it is the specification the kernels in
-  dgvcc_b200/csrc/sw_kernels.cu are compared with.
+* ``decomposed``: the same mathematics in the order the CUDA kernels evaluate it (one-pass moments shifted by a
+  sample mean of each plane, batch covariance from the per-sample ones, closed-form adjoint of the Newton iteration,
+  the two affine passes), numpy fp64, no autograd.  tests/test_oracle_sw.py checks it against ``forward``; it is the
+  specification the kernels in dgvcc_b200/csrc/sw_kernels.cu are compared with.
 """
 import numpy as np
 import torch
@@ -177,10 +177,22 @@ def newton_backward(g_wm, cov, saved):
     return g_cov + (-g_r * r * r) * np.eye(c)
 
 
+def sample_shift(xg):
+    """The per-channel centre of the forward moments pass: the mean of up to 128 pixels of the plane (16 runs of 8
+    consecutive pixels starting at (c hw) // 16, or every pixel when hw <= 128), rounded to fp32.  The kernel sums the sample in
+    fp32 and may land an ulp away; any centre gives the same statistics up to rounding, so only the choice of pixels is
+    specification."""
+    hw = xg.shape[-1]
+    idx = ((np.arange(16)[:, None] * hw) // 16 + np.arange(8)).ravel() if hw > 128 else np.arange(hw)
+    return xg[..., idx].mean(-1).astype(np.float32).astype(np.float64)
+
+
 def decomposed(x, gy, sw_mean_weight, sw_var_weight, weight, bias, running_mean, running_cov, *, num_pergroup=16,
-               sw_type=2, T=5, eps=1e-5, training=True, all_reduce=None, world_size=1):
+               sw_type=2, T=5, eps=1e-5, training=True, all_reduce=None, world_size=1, stages=None):
     """Forward and backward in the kernels' order.  ``all_reduce(array)`` sums a numpy array over ranks in place (the
-    four exchanges of SyncMeanCov); ``running_*`` are only read (eval mode).  Returns (y, grads, (mean_bn, cov_bn))."""
+    four exchanges of SyncMeanCov); ``running_*`` are only read (eval mode).  Returns (y, grads, (mean_bn, cov_bn)).
+    A dict passed as ``stages`` receives the intermediates the C entry points return: mean_in [n, g, c],
+    cov_in [n, g, c, c], a_fwd [n, g, c, c], g_mean_bn [g, c] and g_cov_bn [g, c, c] (before any exchange)."""
     x = np.asarray(x, np.float64)
     gy = np.asarray(gy, np.float64)
     n, ch, h, w = x.shape
@@ -189,8 +201,8 @@ def decomposed(x, gy, sw_mean_weight, sw_var_weight, weight, bias, running_mean,
     gyg = gy.reshape(n, g, c, hw)
     reduce_ = all_reduce if all_reduce is not None else (lambda a: a)
 
-    # --- moments pass: one read of x, shifted by each channel's first pixel --------------------------------------
-    shift = xg[..., :1]
+    # --- moments pass: one read of x, shifted by a sample mean of each channel -----------------------------------
+    shift = sample_shift(xg)[..., None]
     s1 = (xg - shift).sum(-1)
     s2 = np.einsum("ngip,ngjp->ngij", xg - shift, xg - shift)
     delta = s1 / hw
@@ -287,6 +299,8 @@ def decomposed(x, gy, sw_mean_weight, sw_var_weight, weight, bias, running_mean,
     g_mw = mw * (gm - (mw * gm).sum())
     g_vw = None if gv is None else vw * (gv - (vw * gv).sum())
 
+    if stages is not None:
+        stages.update(mean_in=mean_in, cov_in=cov_in, a_fwd=a_fwd, g_mean_bn=g_mean_bn.copy(), g_cov_bn=g_cov_bn.copy())
     if training:
         reduce_(g_mean_bn)
         reduce_(g_cov_bn)
